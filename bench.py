@@ -4,9 +4,11 @@
   python bench.py --gpus N --steps K --warmup W            our arm (libacx kernels on B200)
   python bench.py --impl reference --gpus N ...             the reference's CPU path (oracle port) on host cores
   torchrun ... bench.py --gpus N ...                        N > 1: one rank per GPU, clips sharded by clip
+  python bench.py ... --dump-outputs DIR                    also save the last timed step's outputs as DIR/<name>.npy
 
 One step = one forward of BASELINE.json configs[1] (batch 64 synthetic clips, ConvNeXt-Tiny random init) per GPU
 (weak scaling) followed, for N > 1, by the NCCL all-gather of the logits.  Prints ONE JSON line (rank 0).
+Weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -17,6 +19,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -332,7 +335,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[0]/[2]/[3]/[4] and eager-GPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -381,11 +390,19 @@ def main():
     mark0 = clocks.mark()
     e0.record()
     for i in range(args.steps):
-        step(i)
+        out = step(i)
     e1.record()
     fence()
     mark1 = clocks.mark()
     launches = eng.launches - launches0
+    if args.dump_outputs and rank == 0:
+        # written now: the passes below reuse `gathered`.  64 clips x (logits, probs, scene) is under 0.5 MB.
+        dumped = {k: v.float().cpu().numpy() for k, v in out.items()}
+        if world > 1:
+            dumped["logits_all_ranks"] = gathered.float().cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     # ---- same K steps again with a CUDA-event pair around every launch of the dominant kernel (individual launches:
     #      events cannot bracket a node inside a replayed graph); used only for roofline.achieved ------------------
     eng.start_timing(only=top)
@@ -410,7 +427,7 @@ def main():
     pipe = acx.HostPipeline(model, want=("logits",))
     pipe.run([host[i % 3] for i in range(3)])                  # warm-up
     fence()
-    n_e2e = max(6, args.steps)
+    n_e2e = args.steps
     t0 = time.perf_counter()
     res = pipe.run([host[i % 3] for i in range(n_e2e)])
     if world > 1:
