@@ -49,6 +49,17 @@ SIGNATURES = {
     "acx_head": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp],
     "acx_nhwc_to_nchw_f32": [_vp, _vp, _i, _i, _i, _i, _i, _vp],
     "acx_resample_fit": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp],
+    # ragged batches: the entry point above plus the device array of per-clip bounds (and, for the prep kernels, the
+    # input row pitch), just before the stream
+    "acx_wave_prep_ragged": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
+    "acx_frame_fold_ragged": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
+    "acx_stem_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp],
+    "acx_stem_gp_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "acx_dwconv_tc_ragged": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp],
+    "acx_dwconv_tc_gp_ragged": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp],
+    "acx_dwconv_ln_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
+    "acx_head_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
+    "acx_nhwc_to_nchw_f32_ragged": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
 }
 
 

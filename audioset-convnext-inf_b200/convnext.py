@@ -20,7 +20,7 @@ import torch
 import torch.nn as nn
 
 from . import _native
-from .engine import DEPTHS, DIMS, Engine
+from .engine import DEPTHS, DIMS, Engine, out_time_dims
 from .frontend_consts import slaney_mel_filterbank, windowed_dft
 
 HF_PYTORCH_WEIGHTS_NAME = "model.safetensors"
@@ -210,12 +210,23 @@ class ConvNeXt(nn.Module):
         eng, x = self._prep(x, mixup_lambda)
         return eng.run(x, want=("frame",))["frame"]
 
-    def forward_all(self, x):
-        """One pass for everything (the reference demo runs three, demo_convnext.py:73-104)."""
+    def forward_all(self, x, lengths=None):
+        """One pass for everything (the reference demo runs three, demo_convnext.py:73-104).
+
+        lengths: None, or one length per clip (a host sequence or CPU tensor of B ints, each in [7360, x.shape[1]]) for a
+        RAGGED batch: clip b is x[b, :lengths[b]], and samples past it are never read.  Every output of clip b then equals
+        forward_all(x[b:b + 1, :lengths[b]]) bit for bit; "frame_embeddings" is (B, 768, T', 7) with T' the canvas's frame
+        count and zeros past each clip's own count, which "frame_lengths" ((B,) int64) gives.  A clip's result depends on
+        its exact length (reflect padding at its end, frame count), so this is NOT what the reference computes for a
+        zero-padded batch such as AudioCaps' BasicCollate output: forward(x_padded) still gives that."""
         eng, x = self._prep(x, None)
-        out = eng.run(x, want=("logits", "scene", "frame"))
-        return {"clipwise_output": out["probs"], "clipwise_logits": out["logits"],
-                "scene_embeddings": out["scene"], "frame_embeddings": out["frame"]}
+        out = eng.run(x, want=("logits", "scene", "frame"), lengths=lengths)
+        res = {"clipwise_output": out["probs"], "clipwise_logits": out["logits"],
+               "scene_embeddings": out["scene"], "frame_embeddings": out["frame"]}
+        if lengths is not None:
+            h3 = [out_time_dims(int(n))[1][3] for n in lengths]
+            res["frame_lengths"] = torch.tensor(h3, dtype=torch.int64).to(x.device)
+        return res
 
     def forward_logmel(self, x):
         """Normalised log-mel (B, T, 224): the tensor the reference has after bn0 (CX:298-306)."""

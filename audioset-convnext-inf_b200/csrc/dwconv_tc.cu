@@ -75,11 +75,13 @@ __device__ __forceinline__ void tmem_ld_32x32b_x8(uint32_t taddr, uint32_t (&r)[
 // request and the staging / write-out phases ran at ~5 useful B/clk/SM (24 k + 8 k of a unit's 54 k cycles, in-kernel
 // clock trace; TMA gathers the same pieces at 14 B/clk/SM, tools/ubench/tma_gather.cu).  In the planar layout a unit's
 // image rows are contiguous: fragment loads are full 128-byte lines and the results leave as 512-byte runs.
-template <int W, bool GP>
+// RAG = ragged batch: clip n has valid[n] rows (clamped to [0, H]); the rows past it are staged as the conv's zero padding,
+// so its first valid[n] output rows equal a run at that height (the rows past it are computed but carry no meaning).
+template <int W, bool GP, bool RAG = false>
 __global__ void __launch_bounds__(THREADS, 2)
     dwconv_tc_kernel(const bf16* __restrict__ x, const bf16* __restrict__ taps /*[49][C]*/,
                      const float* __restrict__ bias, bf16* __restrict__ v, int n_clips, int H, int C,
-                     long long* __restrict__ trace) {
+                     long long* __restrict__ trace, const int32_t* __restrict__ valid) {
   constexpr int NHALF = W > 32 ? 2 : 1;
   constexpr int HW = NHALF == 2 ? 28 : W;       // output pixels per half row
   constexpr int WB = (W + 7) / 8;               // 8-pixel blocks per image row
@@ -161,6 +163,7 @@ __global__ void __launch_bounds__(THREADS, 2)
       constexpr int kPix = GP ? 8 : 0;            // element stride between pixels: 8 (planar) or C (NHWC)
       const int px = lane >> 2;                           // pixel of the fragment this lane loads
       const int sj = lane & 7, smi = lane >> 3;           // stored row (channel) / matrix this lane addresses
+      const int hv = RAG ? min(max(__ldg(valid + n), 0), H) : H;      // RAG only
 #pragma unroll 1
       for (int rd = 0; rd < ROUNDS; ++rd) {
         uint32_t q[4][4];
@@ -172,7 +175,7 @@ __global__ void __launch_bounds__(THREADS, 2)
             const int m = 4 * gi + mi;
             const int r = m / WB, wb = m - r * WB;
             const int h = h0 - 3 + r, w = wb * 8 + px;
-            const bool ok = m < NM && h >= 0 && h < H && w < W;
+            const bool ok = m < NM && (RAG ? (unsigned)h < (unsigned)hv : (h >= 0 && h < H)) && w < W;
             q[u][mi] = ok ? ldg_nc_u32(xin + ((size_t)h * W + w) * (GP ? kPix : C)) : 0u;
           }
         }
@@ -356,10 +359,12 @@ constexpr int NLOAD = 7;                       // loader warps
 static_assert(OFF_A % 1024 == 0 && A_BUF % 512 == 0, "swizzle atoms");
 static_assert(SMEM_BYTES <= 227 * 1024, "smem budget");
 
-template <int W>
+// RAG: as in dwconv_tc_kernel; a paired item (W = 14) bounds each of its two clips by its own valid[] entry.
+template <int W, bool RAG = false>
 __global__ void __launch_bounds__(THREADS, 1)
     dwconv_tc3_kernel(const bf16* __restrict__ x, const bf16* __restrict__ taps /*[49][C]*/, const float* __restrict__ bias,
-                      bf16* __restrict__ v, int n_clips, int H, int C, long long* __restrict__ trace) {
+                      bf16* __restrict__ v, int n_clips, int H, int C, long long* __restrict__ trace,
+                      const int32_t* __restrict__ valid) {
   constexpr int NHALF = W > 32 ? 2 : 1;
   constexpr int HW = NHALF == 2 ? 28 : W;
   // W = 14: an item takes the rows of TWO clips side by side in one 32-column K window -- clip A in columns 0..13, three
@@ -486,6 +491,8 @@ __global__ void __launch_bounds__(THREADS, 1)
       V3_ACC(tr_wait);
       const bf16* xin = xg + ((size_t)n * H * W + kw0) * 8;
       const bool b_ok = PAIR && n + 1 < n_clips;        // the pair's second clip exists
+      const int hv_a = RAG ? min(max(__ldg(valid + n), 0), H) : H;
+      const int hv_b = RAG && b_ok ? min(max(__ldg(valid + n + 1), 0), H) : H;
       const uint32_t abuf = s_base + OFF_A + buf * A_BUF;
       constexpr int RPR = (AR + NLOAD - 1) / NLOAD;     // rows per warp: all requested at once
 #pragma unroll 1
@@ -494,7 +501,7 @@ __global__ void __launch_bounds__(THREADS, 1)
 #pragma unroll
         for (int u = 0; u < RPR; ++u) {
           const int r = r0 + NLOAD * u, h = h0 - 3 + r;
-          const bool row_ok = r < AR && h >= 0 && h < H;
+          const bool row_ok = r < AR && h >= 0 && h < hv_a;
 #pragma unroll
           for (int mi = 0; mi < 4; ++mi) {
             const int col = kw0 + mi * 8 + px;
@@ -502,7 +509,12 @@ __global__ void __launch_bounds__(THREADS, 1)
               const int ca = mi * 8 + px;               // A column: 0..13 clip A, 17..30 clip B
               const bool in_a = ca < 14, in_b = ca >= 17 && ca < 31 && b_ok;
               const size_t off = in_a ? ((size_t)h * W + ca) : ((size_t)(H + h) * W + ca - 17);
-              q[u][mi] = (row_ok && (in_a || in_b)) ? ldg_nc_u32(xin + off * 8) : 0u;
+              if (RAG) {                                // row_ok bounds clip A only
+                const bool rb = r < AR && h >= 0 && h < hv_b;
+                q[u][mi] = ((in_a && row_ok) || (in_b && rb)) ? ldg_nc_u32(xin + off * 8) : 0u;
+              } else {
+                q[u][mi] = (row_ok && (in_a || in_b)) ? ldg_nc_u32(xin + off * 8) : 0u;
+              }
             } else {
               q[u][mi] = (mi < NMI && row_ok && col < W) ? ldg_nc_u32(xin + ((size_t)h * W + mi * 8 + px) * 8) : 0u;
             }
@@ -622,9 +634,10 @@ __global__ void __launch_bounds__(THREADS, 1)
   }
 }
 
-template <int W>
-static int launch(const void* x, const void* taps, const float* bias, void* v, int B, int H, int C, cudaStream_t st) {
-  auto kern = dwconv_tc3_kernel<W>;
+template <int W, bool RAG>
+static int launch(const void* x, const void* taps, const float* bias, void* v, int B, int H, int C, const int32_t* valid,
+                  cudaStream_t st) {
+  auto kern = dwconv_tc3_kernel<W, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM_BYTES);
   const int G = C / CG;
   const long long work = (long long)G * (W == 14 ? (B + 1) / 2 : B) * ceil_div(H, TR) * (W > 32 ? 2 : 1);
@@ -635,14 +648,15 @@ static int launch(const void* x, const void* taps, const float* bias, void* v, i
   if (getenv("ACX_DWTC_TRACE")) trace = reinterpret_cast<long long*>(strtoull(getenv("ACX_DWTC_TRACE"), nullptr, 0));
 #endif
   ACX_CUDA(launch_pdl(kern, dim3(grid), dim3(THREADS), SMEM_BYTES, st, 1, PDL_DWTC, reinterpret_cast<const bf16*>(x),
-                      reinterpret_cast<const bf16*>(taps), bias, reinterpret_cast<bf16*>(v), B, H, C, trace));
+                      reinterpret_cast<const bf16*>(taps), bias, reinterpret_cast<bf16*>(v), B, H, C, trace, valid));
   return ACX_OK;
 }
 }  // namespace v3
 
-template <int W, bool GP>
-static int launch(const void* x, const void* taps, const float* bias, void* v, int B, int H, int C, cudaStream_t st) {
-  auto kern = dwconv_tc_kernel<W, GP>;
+template <int W, bool GP, bool RAG>
+static int launch(const void* x, const void* taps, const float* bias, void* v, int B, int H, int C, const int32_t* valid,
+                  cudaStream_t st) {
+  auto kern = dwconv_tc_kernel<W, GP, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM_BYTES);
   const int units = B * ceil_div(H, TR) * (C / CG);
   const int grid = units < 2 * sm_count() ? units : 2 * sm_count();
@@ -652,7 +666,7 @@ static int launch(const void* x, const void* taps, const float* bias, void* v, i
   if (getenv("ACX_DWTC_TRACE")) trace = reinterpret_cast<long long*>(strtoull(getenv("ACX_DWTC_TRACE"), nullptr, 0));
 #endif
   kern<<<grid, THREADS, SMEM_BYTES, st>>>(reinterpret_cast<const bf16*>(x), reinterpret_cast<const bf16*>(taps), bias,
-                                          reinterpret_cast<bf16*>(v), B, H, C, trace);
+                                          reinterpret_cast<bf16*>(v), B, H, C, trace, valid);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }
@@ -738,8 +752,9 @@ static int launch_ln(const void* in, const float* ln_w, const float* ln_b, void*
 
 using namespace acx;
 
-extern "C" int acx_dwconv_tc(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
-                             void* stream) {
+template <bool RAG>
+static int dwconv_tc_impl(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                          const int32_t* valid, void* stream) {
   ACX_CHECK(x && w && bias && v, ACX_ERR_ARG, "dwconv_tc: null pointer");
   ACX_CHECK(B > 0 && H > 0, ACX_ERR_ARG, "dwconv_tc: B and H must be positive");
   ACX_CHECK(C % 8 == 0 && C > 0, ACX_ERR_ARG, "dwconv_tc: C must be a positive multiple of 8 (got %d)", C);
@@ -748,19 +763,31 @@ extern "C" int acx_dwconv_tc(const void* x, const void* w, const float* bias, vo
             "dwconv_tc: x and v must be 16-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   switch (W) {
-    case 56: return dwtc::launch<56, false>(x, w, bias, v, B, H, C, st);
-    case 28: return dwtc::launch<28, false>(x, w, bias, v, B, H, C, st);
-    case 14: return dwtc::launch<14, false>(x, w, bias, v, B, H, C, st);
-    case 7: return dwtc::launch<7, false>(x, w, bias, v, B, H, C, st);
+    case 56: return dwtc::launch<56, false, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 28: return dwtc::launch<28, false, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 14: return dwtc::launch<14, false, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 7: return dwtc::launch<7, false, RAG>(x, w, bias, v, B, H, C, valid, st);
     default:
       set_error("dwconv_tc: W=%d not supported (the ConvNeXt stages are 56 / 28 / 14 / 7 wide)", W);
       return ACX_ERR_UNSUPPORTED;
   }
 }
 
+extern "C" int acx_dwconv_tc(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                             void* stream) {
+  return dwconv_tc_impl<false>(x, w, bias, v, B, H, W, C, nullptr, stream);
+}
+
+extern "C" int acx_dwconv_tc_ragged(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                                    const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "dwconv_tc_ragged: null valid-length array");
+  return dwconv_tc_impl<true>(x, w, bias, v, B, H, W, C, valid, stream);
+}
+
 // Same on group-planar activations: x, v = [C/8][B*H*W][8] bf16.
-extern "C" int acx_dwconv_tc_gp(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
-                                void* stream) {
+template <bool RAG>
+static int dwconv_tc_gp_impl(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                             const int32_t* valid, void* stream) {
   ACX_CHECK(x && w && bias && v, ACX_ERR_ARG, "dwconv_tc_gp: null pointer");
   ACX_CHECK(B > 0 && H > 0, ACX_ERR_ARG, "dwconv_tc_gp: B and H must be positive");
   ACX_CHECK(C % 8 == 0 && C > 0, ACX_ERR_ARG, "dwconv_tc_gp: C must be a positive multiple of 8 (got %d)", C);
@@ -770,13 +797,28 @@ extern "C" int acx_dwconv_tc_gp(const void* x, const void* w, const float* bias,
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   static const bool use_v1 = getenv("ACX_DWTC_V1") != nullptr;      // the two-CTA-per-SM kernel, kept for A/B timing
   switch (W) {
-    case 56: return use_v1 ? dwtc::launch<56, true>(x, w, bias, v, B, H, C, st) : dwtc::v3::launch<56>(x, w, bias, v, B, H, C, st);
-    case 28: return use_v1 ? dwtc::launch<28, true>(x, w, bias, v, B, H, C, st) : dwtc::v3::launch<28>(x, w, bias, v, B, H, C, st);
-    case 14: return dwtc::v3::launch<14>(x, w, bias, v, B, H, C, st);
+    case 56:
+      return use_v1 ? dwtc::launch<56, true, RAG>(x, w, bias, v, B, H, C, valid, st)
+                    : dwtc::v3::launch<56, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 28:
+      return use_v1 ? dwtc::launch<28, true, RAG>(x, w, bias, v, B, H, C, valid, st)
+                    : dwtc::v3::launch<28, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 14: return dwtc::v3::launch<14, RAG>(x, w, bias, v, B, H, C, valid, st);
     default:
       set_error("dwconv_tc_gp: W=%d not supported (stages 0 - 2: 56 / 28 / 14)", W);
       return ACX_ERR_UNSUPPORTED;
   }
+}
+
+extern "C" int acx_dwconv_tc_gp(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                                void* stream) {
+  return dwconv_tc_gp_impl<false>(x, w, bias, v, B, H, W, C, nullptr, stream);
+}
+
+extern "C" int acx_dwconv_tc_gp_ragged(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                                       const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "dwconv_tc_gp_ragged: null valid-length array");
+  return dwconv_tc_gp_impl<true>(x, w, bias, v, B, H, W, C, valid, stream);
 }
 
 // ---- (M, C) row-major <-> group-planar [C/8][M][8] ----------------------------------------------------------------------

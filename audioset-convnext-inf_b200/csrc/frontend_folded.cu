@@ -304,9 +304,12 @@ __global__ void __launch_bounds__(ff::THREADS, 1)
 __device__ __forceinline__ float ff_sample(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ff_sample(const int16_t* p) { return __fdiv_rn((float)__ldg(p), 32767.0f); }   // utils/utilities.py:226
 
-template <typename TIn>
+// RAG: row b is a clip of valid[b] samples (clamped to [n_fft/2 + 1, L]) at row pitch ld_wave, reflected at its own end and
+// zero past the reflected range; samples past valid[b] are never read.
+template <typename TIn, bool RAG = false>
 __global__ void __launch_bounds__(256) frame_fold_kernel(const TIn* __restrict__ wave, __half* __restrict__ fhi, __half* __restrict__ flo,
-                                                         int L, int T, int n_fft, int hop) {
+                                                         int L, int T, int n_fft, int hop, int ld_wave,
+                                                         const int32_t* __restrict__ valid) {
   // thread = (frame t, four consecutive fold indices j0 .. j0 + 3): 8-byte stores of E and O, hi and lo
   const int b = blockIdx.y;
   const int half_n = n_fft >> 1;
@@ -314,9 +317,11 @@ __global__ void __launch_bounds__(256) frame_fold_kernel(const TIn* __restrict__
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (long long)T * per_frame) return;
   const int t = (int)(idx / per_frame), j0 = (int)(idx - (long long)t * per_frame) * 4;
-  const TIn* w = wave + (size_t)b * L;
+  const TIn* w = wave + (size_t)b * (RAG ? ld_wave : L);
+  if (RAG) L = min(max(__ldg(valid + b), half_n + 1), L);
   const int s = t * hop - half_n;              // un-padded sample index of frame position 0 (center = True)
   auto x = [&](int m) {
+    if (RAG && m >= L + half_n) return 0.f;    // past the padded clip: only frames >= the clip's own frame count get here
     if (m < 0) m = -m;                         // reflect (edge sample not repeated), as F.pad(mode="reflect")
     if (m >= L) m = 2 * (L - 1) - m;
     return ff_sample(w + m);
@@ -357,8 +362,10 @@ __global__ void __launch_bounds__(256) frame_fold_kernel(const TIn* __restrict__
 
 using namespace acx;
 
-static int frame_fold_impl(const void* wave, int pcm16, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
+static int frame_fold_impl(const void* wave, int pcm16, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop,
+                           int ld_wave, const int32_t* valid, void* stream) {
   ACX_CHECK(wave && f_hi && f_lo, ACX_ERR_ARG, "frame_fold: null pointer");
+  ACX_CHECK(ld_wave >= L, ACX_ERR_ARG, "frame_fold: row pitch %d < L=%d", ld_wave, L);
   ACX_CHECK(n_fft == 1024 && hop == 320, ACX_ERR_UNSUPPORTED, "frame_fold: built for n_fft=1024, hop=320 (reference convnext.py:161-174)");
   ACX_CHECK(B > 0 && B <= 65535 && L > n_fft / 2 && T == L / hop + 1, ACX_ERR_ARG,
             "frame_fold: bad sizes B=%d L=%d T=%d (reflect padding needs L > n_fft/2, T = L / hop + 1)", B, L, T);
@@ -368,19 +375,27 @@ static int frame_fold_impl(const void* wave, int pcm16, void* f_hi, void* f_lo, 
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (pcm16)
     frame_fold_kernel<int16_t><<<grid, 256, 0, st>>>(reinterpret_cast<const int16_t*>(wave), reinterpret_cast<__half*>(f_hi),
-                                                     reinterpret_cast<__half*>(f_lo), L, T, n_fft, hop);
+                                                     reinterpret_cast<__half*>(f_lo), L, T, n_fft, hop, L, nullptr);
+  else if (valid)
+    frame_fold_kernel<float, true><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(wave), reinterpret_cast<__half*>(f_hi),
+                                                         reinterpret_cast<__half*>(f_lo), L, T, n_fft, hop, ld_wave, valid);
   else
     frame_fold_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(wave), reinterpret_cast<__half*>(f_hi),
-                                                   reinterpret_cast<__half*>(f_lo), L, T, n_fft, hop);
+                                                   reinterpret_cast<__half*>(f_lo), L, T, n_fft, hop, L, nullptr);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }
 
 extern "C" int acx_frame_fold(const float* wave, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
-  return frame_fold_impl(wave, 0, f_hi, f_lo, B, L, T, n_fft, hop, stream);
+  return frame_fold_impl(wave, 0, f_hi, f_lo, B, L, T, n_fft, hop, L, nullptr, stream);
+}
+extern "C" int acx_frame_fold_ragged(const float* wave, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, int ld_wave,
+                                     const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "frame_fold_ragged: null valid-length array");
+  return frame_fold_impl(wave, 0, f_hi, f_lo, B, L, T, n_fft, hop, ld_wave, valid, stream);
 }
 extern "C" int acx_frame_fold_pcm16(const int16_t* pcm, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
-  return frame_fold_impl(pcm, 1, f_hi, f_lo, B, L, T, n_fft, hop, stream);
+  return frame_fold_impl(pcm, 1, f_hi, f_lo, B, L, T, n_fft, hop, L, nullptr, stream);
 }
 
 extern "C" int acx_frontend_folded(const void* f_hi, const void* f_lo, const void* w_hi, const void* w_lo, const void* mel_hi,

@@ -7,6 +7,8 @@
 //   head             mel-mean, time max+mean, LayerNorm, fc, sigmoid   (CX:279-285, CX:321-325)
 //   nhwc_to_nchw     frame-embedding layout                            (CX:399-402)
 // "CX" = reference src/audioset_convnext_inf/pytorch/convnext.py.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace acx {
@@ -19,13 +21,16 @@ namespace acx {
 __device__ __forceinline__ float load_sample(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float load_sample(const int16_t* p) { return __fdiv_rn((float)__ldg(p), 32767.0f); }
 
-template <bool kSplit, typename TIn>
+// RAG: row b is a clip of valid[b] samples (clamped to [pad + 1, L]) at row pitch ld_wave; it is reflected at its own end
+// and zero past it, exactly like a run at that length.  Samples past valid[b] are never read.
+template <bool kSplit, typename TIn, bool RAG = false>
 __global__ void wave_prep_kernel(const TIn* __restrict__ wave, void* __restrict__ hi_, void* __restrict__ lo_,
-                                 int L, int pad, int ld_pad) {
+                                 int L, int pad, int ld_pad, int ld_wave, const int32_t* __restrict__ valid) {
   // 4 consecutive output samples per thread (ld_pad % 8 == 0): 8-byte bf16 / 16-byte fp32 stores
   const int b = blockIdx.y;
   const int j0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (j0 >= ld_pad) return;
+  if (RAG) L = min(max(__ldg(valid + b), pad + 1), L);
   float v[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -35,7 +40,7 @@ __global__ void wave_prep_kernel(const TIn* __restrict__ wave, void* __restrict_
       int s = j - pad;
       if (s < 0) s = -s;                       // reflect (edge sample not repeated)
       if (s >= L) s = 2 * (L - 1) - s;
-      v[i] = load_sample(wave + (size_t)b * L + s);
+      v[i] = load_sample(wave + (size_t)b * (RAG ? ld_wave : L) + s);
     }
   }
   const size_t o = (size_t)b * ld_pad + j0;
@@ -94,11 +99,12 @@ __global__ void power_mel_log_kernel(const float* __restrict__ spec, int ld_spec
 //  * LayerNorm statistics need no cross-thread traffic at all;
 //  * the warp's 32 x 96 outputs (contiguous in HBM) are transposed through padded smem and stored coalesced.
 // =============================================================================================
-template <typename T>
+// RAG: clip b has valid[b] frames (clamped to [0, Tn]); later rows are read as the conv's zero padding.
+template <typename T, bool RAG = false>
 __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ logmel, const float* __restrict__ w,
                                                    const float* __restrict__ bias, const float* __restrict__ ln_w,
                                                    const float* __restrict__ ln_b, T* __restrict__ out, int B,
-                                                   int Tn, int n_mels, int H0, int W0) {
+                                                   int Tn, int n_mels, int H0, int W0, const int32_t* __restrict__ valid) {
   constexpr int CO = 96;
   constexpr int ROW_BYTES = CO * (int)sizeof(T);       // 192 (bf16) / 384 (fp32)
   constexpr int ROW_PITCH = ROW_BYTES + 16;            // +16 B: conflict-free 16-byte row writes
@@ -123,11 +129,12 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ log
     const int ox = (int)(pp % W0);
     const int oy = (int)((pp / W0) % H0);
     const int b = (int)(pp / ((long long)W0 * H0));
+    const int Tb = RAG ? min(max(__ldg(valid + b), 0), Tn) : Tn;
 #pragma unroll
     for (int ky = 0; ky < 4; ++ky) {
       const int t = oy * 4 - 4 + ky;
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (ok && t >= 0 && t < Tn) v = __ldg(reinterpret_cast<const float4*>(logmel + ((size_t)b * Tn + t) * n_mels + ox * 4));
+      if (ok && t >= 0 && t < Tb) v = __ldg(reinterpret_cast<const float4*>(logmel + ((size_t)b * Tn + t) * n_mels + ox * 4));
       xin[ky * 4 + 0] = v.x;
       xin[ky * 4 + 1] = v.y;
       xin[ky * 4 + 2] = v.z;
@@ -230,11 +237,12 @@ __device__ __forceinline__ int slot_of_lane(int lane) {
 // resident blocks the register budget is capped for: 5 x 96, 2 x 192 or 1 x 384 threads (15 / 12 / 12 warps per SM)
 constexpr int dw_min_blocks(int threads) { return threads <= 96 ? 5 : (threads <= 192 ? 2 : 1); }
 
-template <typename T, int C, int S, int PF>
+// RAG: clip b has valid[b] rows (clamped to [0, H]); rows past it are read as the conv's zero padding and not written.
+template <typename T, int C, int S, int PF, bool RAG = false>
 __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
     dwconv_ln_kernel(const T* __restrict__ x, const T* __restrict__ w, const float* __restrict__ bias,
                      const float* __restrict__ ln_w, const float* __restrict__ ln_b, T* __restrict__ y, int H,
-                     int W, int groups_per_block) {
+                     int W, int groups_per_block, const int32_t* __restrict__ valid) {
   using P = Pair<T>;
   using PT = typename P::type;
   constexpr int R = DW_R;
@@ -280,6 +288,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
   static_assert((R + 6) % PF == 0, "prefetch ring must divide the row count");
   pdl_trigger();       // programmatic dependent launch (common.cuh); x is the previous kernel's output
   pdl_wait();
+  const int Hv = RAG ? min(max(__ldg(valid + b), 0), H) : H;      // block-uniform
   PT nxt[PF][13];
 #pragma unroll
   for (int k = 0; k < PF; ++k) load_row((int)blockIdx.y * groups_per_block * R - 3 + k, nxt[k]);
@@ -311,7 +320,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
 
   for (int grp_i = 0; grp_i < groups_per_block; ++grp_i) {
   const int h0 = (blockIdx.y * groups_per_block + grp_i) * R;
-  if (h0 >= H) break;   // block-uniform
+  if (h0 >= Hv) break;   // block-uniform
 
   float2 acc[R][7];
 #pragma unroll
@@ -329,7 +338,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
     if (i + PF < R + 6) load_row(h0 - 3 + i + PF, nxt[i % PF]);
     else if (grp_i + 1 < groups_per_block) load_row(h0 + R - 3 + (i + PF - (R + 6)), nxt[i % PF]);
     const int ih = h0 - 3 + i;
-    if (ih >= 0 && ih < H) {                                    // zero padding contributes nothing (block-uniform)
+    if (ih >= 0 && ih < Hv) {                                   // zero padding contributes nothing (block-uniform)
 #pragma unroll
       for (int r = 0; r < R; ++r) {
         const int ky = i - r;                                   // compile-time after unrolling
@@ -383,7 +392,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
 #pragma unroll
     for (int r = 0; r < R; ++r) {
       const int h = h0 + r;
-      if (h >= H) break;
+      if (h >= Hv) break;
       PT* orow = yp + ((size_t)h * W + w0) * TPS;
 #pragma unroll
       for (int p = 0; p < 7; ++p) {
@@ -425,7 +434,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
 #pragma unroll
     for (int r = 0; r < R; ++r) {
       const int h = h0 + r;
-      if (h >= H) break;
+      if (h >= Hv) break;
       PT* orow = yp + ((size_t)h * W + w0) * TPS;
 #pragma unroll
       for (int p = 0; p < 7; ++p) {
@@ -552,9 +561,10 @@ __global__ void __launch_bounds__(256, 3)
 //   ln_fc:  grid (B, 8):    LayerNorm(C) (recomputed per block, 768 values) -> scene; 1/8 of the fc rows -> logits,
 //           sigmoid -> probs
 // =============================================================================================
-template <typename T>
+// RAG: clip b pools over its first valid[b] rows (clamped to [1, H]).
+template <typename T, bool RAG = false>
 __global__ void __launch_bounds__(256)
-    head_pool_kernel(const T* __restrict__ x, float* __restrict__ pooled, int H, int W, int C) {
+    head_pool_kernel(const T* __restrict__ x, float* __restrict__ pooled, int H, int W, int C, const int32_t* __restrict__ valid) {
   using P = Pair<T>;
   using PT = typename P::type;
   __shared__ float2 smax[8][32], ssum[8][32];
@@ -564,9 +574,10 @@ __global__ void __launch_bounds__(256)
   const int b = blockIdx.y;
   const int cp = blockIdx.x * 32 + lane;                 // channel pair
   const PT* xb = reinterpret_cast<const PT*>(x) + (size_t)b * H * W * (C / 2) + cp;
+  const int Hv = RAG ? min(max(__ldg(valid + b), 1), H) : H;
   float2 mx = make_float2(-INFINITY, -INFINITY), sm = make_float2(0.f, 0.f);
   const float inv_w = 1.0f / W;
-  for (int h = warp; h < H; h += 8) {
+  for (int h = warp; h < Hv; h += 8) {
     float2 s = make_float2(0.f, 0.f);
     for (int wv = 0; wv < W; ++wv) {
       const float2 f = P::unpack(__ldg(xb + ((size_t)h * W + wv) * (C / 2)));
@@ -591,7 +602,7 @@ __global__ void __launch_bounds__(256)
       sm.x += ssum[i][lane].x;
       sm.y += ssum[i][lane].y;
     }
-    *reinterpret_cast<float2*>(pooled + (size_t)b * C + 2 * cp) = make_float2(mx.x + sm.x / H, mx.y + sm.y / H);  // CX:282
+    *reinterpret_cast<float2*>(pooled + (size_t)b * C + 2 * cp) = make_float2(mx.x + sm.x / Hv, mx.y + sm.y / Hv);  // CX:282
   }
 }
 
@@ -672,8 +683,10 @@ __global__ void __launch_bounds__(256)
 // =============================================================================================
 // NHWC (act dtype) -> NCHW fp32
 // =============================================================================================
-template <typename T>
-__global__ void nhwc_to_nchw_kernel(const T* __restrict__ x, float* __restrict__ out, int HW, int C) {
+// RAG: rows of clip b at or past valid[b] (clamped to [0, H]) are written as zeros and not read.
+template <typename T, bool RAG = false>
+__global__ void nhwc_to_nchw_kernel(const T* __restrict__ x, float* __restrict__ out, int HW, int C, int W,
+                                    const int32_t* __restrict__ valid) {
   __shared__ float tile[32][33];
   pdl_trigger();       // programmatic dependent launch (common.cuh)
   pdl_wait();
@@ -681,9 +694,10 @@ __global__ void nhwc_to_nchw_kernel(const T* __restrict__ x, float* __restrict__
   const int p0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   const T* xb = x + (size_t)b * HW * C;
   float* ob = out + (size_t)b * HW * C;
+  const int pv = RAG ? min(max(__ldg(valid + b), 0), HW / W) * W : HW;      // valid pixels of this clip
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
     const int p = p0 + i, c = c0 + threadIdx.x;
-    if (p < HW && c < C) tile[i][threadIdx.x] = to_float(xb[(size_t)p * C + c]);
+    if (p < HW && c < C) tile[i][threadIdx.x] = p < pv ? to_float(xb[(size_t)p * C + c]) : 0.f;
   }
   __syncthreads();
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -718,14 +732,14 @@ __global__ void __launch_bounds__(256)
 }
 
 // ---- launch helpers ---------------------------------------------------------------------------
-template <typename T, int C, int S, int PF = 2>
+template <typename T, int C, int S, int PF = 2, bool RAG = false>
 static int launch_dwconv(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
-                         void* y, int B, int H, int W, cudaStream_t st) {
+                         void* y, int B, int H, int W, const int32_t* valid, cudaStream_t st) {
   const int strips = W / 7;
   ACX_CHECK(strips % S == 0, ACX_ERR_ARG, "dwconv_ln: W/7=%d not a multiple of strips-per-block %d", strips, S);
   constexpr int NV = sizeof(T) == 4 ? 32 : 64;
   constexpr int SMEM = (2 * 49 * (C / 2) + S * (C / 32) * NV + S * NV) * (int)sizeof(float);
-  auto kern = dwconv_ln_kernel<T, C, S, PF>;
+  auto kern = dwconv_ln_kernel<T, C, S, PF, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM);
   const int row_groups = ceil_div(H, DW_R);
   // Row groups per block.  With the first input rows requested ahead of the tap fill (and the next group's rows
@@ -737,20 +751,20 @@ static int launch_dwconv(const void* x, const void* w, const float* bias, const 
   if (gpb_env > 0) gpb = gpb_env < row_groups ? gpb_env : row_groups;
   dim3 grid(strips / S, ceil_div(row_groups, gpb), B);
   ACX_CUDA(launch_pdl(kern, grid, dim3(S * C / 2), SMEM, st, 1, PDL_SMALL, reinterpret_cast<const T*>(x), reinterpret_cast<const T*>(w), bias,
-                      ln_w, ln_b, reinterpret_cast<T*>(y), H, W, gpb));
+                      ln_w, ln_b, reinterpret_cast<T*>(y), H, W, gpb, valid));
   return ACX_OK;
 }
 
-template <typename T>
+template <typename T, bool RAG>
 static int dispatch_dwconv(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
-                           void* y, int B, int H, int W, int C, cudaStream_t st) {
+                           void* y, int B, int H, int W, int C, const int32_t* valid, cudaStream_t st) {
   const int strips = W / 7;
   // A/B switches (development only): ACX_DW_PF=1 -> one-row prefetch, ACX_DW_NARROW=1 -> half-width blocks
   static const bool pf1 = [] { const char* e = getenv("ACX_DW_PF"); return e && e[0] == '1'; }();
   static const bool narrow = [] { const char* e = getenv("ACX_DW_NARROW"); return e && e[0] == '1'; }();
 #define ACX_DW_LAUNCH(CC, SS) \
-  (pf1 ? launch_dwconv<T, CC, SS, 1>(x, w, bias, ln_w, ln_b, y, B, H, W, st) \
-       : launch_dwconv<T, CC, SS, 2>(x, w, bias, ln_w, ln_b, y, B, H, W, st))
+  (pf1 ? launch_dwconv<T, CC, SS, 1, RAG>(x, w, bias, ln_w, ln_b, y, B, H, W, valid, st) \
+       : launch_dwconv<T, CC, SS, 2, RAG>(x, w, bias, ln_w, ln_b, y, B, H, W, valid, st))
   switch (C) {
     case 96:
       if (strips % 4 == 0 && !narrow) return ACX_DW_LAUNCH(96, 4);
@@ -775,26 +789,31 @@ static int dispatch_dwconv(const void* x, const void* w, const float* bias, cons
 
 namespace acx {
 int launch_stem_umma(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b,
-                     void* out, int B, int T, int n_mels, int gp, cudaStream_t st);   // stem_umma.cu
+                     void* out, int B, int T, int n_mels, int gp, const int32_t* valid, cudaStream_t st);   // stem_umma.cu
 }
 using namespace acx;
 
 template <typename TIn>
 static int wave_prep_launch(const TIn* wave, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
-                            void* stream) {
+                            int ld_wave, const int32_t* valid, void* stream) {
   ACX_CHECK(wave && hi && B > 0 && L > 0, ACX_ERR_ARG, "wave_prep: null pointer or empty batch");
+  ACX_CHECK(ld_wave >= L, ACX_ERR_ARG, "wave_prep: row pitch %d < L=%d", ld_wave, L);
   ACX_CHECK(L > n_fft / 2, ACX_ERR_ARG, "wave_prep: reflect padding needs L > n_fft/2 (L=%d)", L);
   ACX_CHECK(ld_pad >= L + n_fft && ld_pad % 8 == 0, ACX_ERR_ARG, "wave_prep: ld_pad=%d must be >= L+n_fft and %%8==0",
             ld_pad);
   ACX_CHECK(B <= 65535, ACX_ERR_ARG, "wave_prep: batch %d exceeds gridDim.y", B);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   dim3 grid(ceil_div(ld_pad, 1024), B);
-  if (act_dtype == ACX_BF16) {
-    ACX_CHECK(lo != nullptr, ACX_ERR_ARG, "wave_prep: lo buffer required for bf16 split");
-    wave_prep_kernel<true, TIn><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad);
-  } else {
-    wave_prep_kernel<false, TIn><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad);
-  }
+  ACX_CHECK(act_dtype != ACX_BF16 || lo != nullptr, ACX_ERR_ARG, "wave_prep: lo buffer required for bf16 split");
+  constexpr bool kRagged = std::is_same<TIn, float>::value;     // ragged batches are fp32 waveforms only
+  if (kRagged && valid && act_dtype == ACX_BF16)
+    wave_prep_kernel<true, TIn, kRagged><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, valid);
+  else if (kRagged && valid)
+    wave_prep_kernel<false, TIn, kRagged><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, valid);
+  else if (act_dtype == ACX_BF16)
+    wave_prep_kernel<true, TIn><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, nullptr);
+  else
+    wave_prep_kernel<false, TIn><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, nullptr);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }
@@ -803,12 +822,18 @@ extern "C" {
 
 int acx_wave_prep(const float* wave, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
                   void* stream) {
-  return wave_prep_launch<float>(wave, hi, lo, B, L, n_fft, ld_pad, act_dtype, stream);
+  return wave_prep_launch<float>(wave, hi, lo, B, L, n_fft, ld_pad, act_dtype, L, nullptr, stream);
+}
+
+int acx_wave_prep_ragged(const float* wave, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
+                         int ld_wave, const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "wave_prep_ragged: null valid-length array");
+  return wave_prep_launch<float>(wave, hi, lo, B, L, n_fft, ld_pad, act_dtype, ld_wave, valid, stream);
 }
 
 int acx_wave_prep_pcm16(const int16_t* pcm, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
                         void* stream) {
-  return wave_prep_launch<int16_t>(pcm, hi, lo, B, L, n_fft, ld_pad, act_dtype, stream);
+  return wave_prep_launch<int16_t>(pcm, hi, lo, B, L, n_fft, ld_pad, act_dtype, L, nullptr, stream);
 }
 
 int acx_power_mel_log(const float* spec, int ld_spec, int n_bins, const float* melT, const int32_t* mel_lo,
@@ -822,8 +847,8 @@ int acx_power_mel_log(const float* spec, int ld_spec, int n_bins, const float* m
   return ACX_OK;
 }
 
-int acx_stem(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b, void* out,
-             int B, int T, int n_mels, int act_dtype, void* stream) {
+static int stem_impl(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b, void* out,
+                     int B, int T, int n_mels, int act_dtype, const int32_t* valid, void* stream) {
   ACX_CHECK(logmel && w && bias && ln_w && ln_b && out, ACX_ERR_ARG, "stem: null pointer");
   ACX_CHECK(n_mels % 4 == 0 && B > 0 && T > 0, ACX_ERR_ARG, "stem: n_mels must be a multiple of 4");
   const int H0 = (T + 4) / 4 + 1, W0 = n_mels / 4;
@@ -833,29 +858,55 @@ int acx_stem(const float* logmel, const float* w, const float* bias, const float
   // bf16 mode: tensor-core stem (stem_umma.cu); ACX_STEM=simt selects the CUDA-core kernel for A/B timing
   static const bool stem_simt = [] { const char* e = getenv("ACX_STEM"); return e && e[0] == 's'; }();
   if (act_dtype == ACX_BF16 && !stem_simt)
-    return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 0, st);
+    return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 0, valid, st);
   if (act_dtype == ACX_BF16) {
     const int smem = 19 * 96 * 4 + 4 * 32 * (96 * 2 + 16);
-    stem_kernel<bf16><<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<bf16*>(out), B, T,
-                                                 n_mels, H0, W0);
+    auto kern = valid ? stem_kernel<bf16, true> : stem_kernel<bf16>;
+    kern<<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<bf16*>(out), B, T, n_mels, H0, W0, valid);
   } else {
     const int smem = 19 * 96 * 4 + 4 * 32 * (96 * 4 + 16);
-    ACX_SET_MAX_SMEM(stem_kernel<float>, smem);
-    stem_kernel<float><<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<float*>(out), B, T,
-                                                  n_mels, H0, W0);
+    auto kern = valid ? stem_kernel<float, true> : stem_kernel<float>;
+    if (valid) ACX_SET_MAX_SMEM((stem_kernel<float, true>), smem);
+    else ACX_SET_MAX_SMEM(stem_kernel<float>, smem);
+    kern<<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<float*>(out), B, T, n_mels, H0, W0, valid);
   }
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }
 
-int acx_dwconv_ln(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b, void* y, int B,
-                  int H, int W, int C, int act_dtype, void* stream) {
+int acx_stem(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b, void* out,
+             int B, int T, int n_mels, int act_dtype, void* stream) {
+  return stem_impl(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, act_dtype, nullptr, stream);
+}
+
+int acx_stem_ragged(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b, void* out,
+                    int B, int T, int n_mels, int act_dtype, const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "stem_ragged: null valid-length array");
+  return stem_impl(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, act_dtype, valid, stream);
+}
+
+static int dwconv_ln_impl(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b, void* y,
+                          int B, int H, int W, int C, int act_dtype, const int32_t* valid, void* stream) {
   ACX_CHECK(x && w && bias && ln_w && ln_b && y, ACX_ERR_ARG, "dwconv_ln: null pointer");
   ACX_CHECK(B > 0 && H > 0 && W > 0 && W % 7 == 0, ACX_ERR_ARG, "dwconv_ln: W=%d must be a positive multiple of 7", W);
   ACX_CHECK(B <= 65535, ACX_ERR_ARG, "dwconv_ln: batch %d exceeds gridDim.z", B);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  return act_dtype == ACX_BF16 ? dispatch_dwconv<bf16>(x, w, bias, ln_w, ln_b, y, B, H, W, C, st)
-                               : dispatch_dwconv<float>(x, w, bias, ln_w, ln_b, y, B, H, W, C, st);
+  if (valid)
+    return act_dtype == ACX_BF16 ? dispatch_dwconv<bf16, true>(x, w, bias, ln_w, ln_b, y, B, H, W, C, valid, st)
+                                 : dispatch_dwconv<float, true>(x, w, bias, ln_w, ln_b, y, B, H, W, C, valid, st);
+  return act_dtype == ACX_BF16 ? dispatch_dwconv<bf16, false>(x, w, bias, ln_w, ln_b, y, B, H, W, C, nullptr, st)
+                               : dispatch_dwconv<float, false>(x, w, bias, ln_w, ln_b, y, B, H, W, C, nullptr, st);
+}
+
+int acx_dwconv_ln(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b, void* y, int B,
+                  int H, int W, int C, int act_dtype, void* stream) {
+  return dwconv_ln_impl(x, w, bias, ln_w, ln_b, y, B, H, W, C, act_dtype, nullptr, stream);
+}
+
+int acx_dwconv_ln_ragged(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b, void* y,
+                         int B, int H, int W, int C, int act_dtype, const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "dwconv_ln_ragged: null valid-length array");
+  return dwconv_ln_impl(x, w, bias, ln_w, ln_b, y, B, H, W, C, act_dtype, valid, stream);
 }
 
 // bf16 tensor-core stem writing the group-planar layout [12][Mp][8] directly (Mp = B * H0 * 56 rounded up to 128)
@@ -863,7 +914,15 @@ int acx_stem_gp(const float* logmel, const float* w, const float* bias, const fl
                 int B, int T, int n_mels, void* stream) {
   ACX_CHECK(logmel && w && bias && ln_w && ln_b && out, ACX_ERR_ARG, "stem_gp: null pointer");
   ACX_CHECK(n_mels % 4 == 0 && B > 0 && T > 0, ACX_ERR_ARG, "stem_gp: n_mels must be a multiple of 4");
-  return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 1, reinterpret_cast<cudaStream_t>(stream));
+  return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 1, nullptr, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int acx_stem_gp_ragged(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b, void* out,
+                       int B, int T, int n_mels, const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "stem_gp_ragged: null valid-length array");
+  ACX_CHECK(logmel && w && bias && ln_w && ln_b && out, ACX_ERR_ARG, "stem_gp: null pointer");
+  ACX_CHECK(n_mels % 4 == 0 && B > 0 && T > 0, ACX_ERR_ARG, "stem_gp: n_mels must be a multiple of 4");
+  return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 1, valid, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int acx_ln_patchify(const void* x, const float* ln_w, const float* ln_b, void* a, int B, int H, int W, int C,
@@ -904,34 +963,63 @@ int acx_ln_patchify_gp(const void* x, const float* ln_w, const float* ln_b, void
   return ACX_OK;
 }
 
-int acx_head(const void* x, const float* ln_w, const float* ln_b, const float* fc_w, const float* fc_b, float* pooled,
-             float* scene, float* logits, float* probs, int B, int H, int W, int C, int n_cls, int act_dtype,
-             void* stream) {
+static int head_impl(const void* x, const float* ln_w, const float* ln_b, const float* fc_w, const float* fc_b, float* pooled,
+                     float* scene, float* logits, float* probs, int B, int H, int W, int C, int n_cls, int act_dtype,
+                     const int32_t* valid, void* stream) {
   ACX_CHECK(x && ln_w && ln_b && scene && pooled, ACX_ERR_ARG, "head: null pointer");
   ACX_CHECK(n_cls == 0 || (fc_w && fc_b && logits && probs), ACX_ERR_ARG, "head: fc pointers required when n_cls>0");
   ACX_CHECK(C % 64 == 0 && C <= 1024 && B > 0 && B <= 65535 && H > 0 && W > 0, ACX_ERR_ARG, "head: unsupported shape");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   dim3 pgrid(C / 64, B);
   if (act_dtype == ACX_BF16)
-    ACX_CUDA(launch_pdl(head_pool_kernel<bf16>, pgrid, dim3(256), 0, st, 1, PDL_SMALL, reinterpret_cast<const bf16*>(x), pooled, H, W, C));
+    ACX_CUDA(launch_pdl(valid ? head_pool_kernel<bf16, true> : head_pool_kernel<bf16>, pgrid, dim3(256), 0, st, 1, PDL_SMALL,
+                        reinterpret_cast<const bf16*>(x), pooled, H, W, C, valid));
   else
-    ACX_CUDA(launch_pdl(head_pool_kernel<float>, pgrid, dim3(256), 0, st, 1, PDL_SMALL, reinterpret_cast<const float*>(x), pooled, H, W, C));
+    ACX_CUDA(launch_pdl(valid ? head_pool_kernel<float, true> : head_pool_kernel<float>, pgrid, dim3(256), 0, st, 1, PDL_SMALL,
+                        reinterpret_cast<const float*>(x), pooled, H, W, C, valid));
   dim3 fgrid(B, n_cls > 0 ? 8 : 1);
   ACX_CUDA(launch_pdl(head_ln_fc_kernel, fgrid, dim3(256), C * sizeof(float), st, 1, PDL_SMALL, pooled, ln_w, ln_b, fc_w, fc_b, scene, logits,
                       probs, C, n_cls));
   return ACX_OK;
 }
 
-int acx_nhwc_to_nchw_f32(const void* x, float* out, int B, int H, int W, int C, int act_dtype, void* stream) {
+int acx_head(const void* x, const float* ln_w, const float* ln_b, const float* fc_w, const float* fc_b, float* pooled,
+             float* scene, float* logits, float* probs, int B, int H, int W, int C, int n_cls, int act_dtype,
+             void* stream) {
+  return head_impl(x, ln_w, ln_b, fc_w, fc_b, pooled, scene, logits, probs, B, H, W, C, n_cls, act_dtype, nullptr, stream);
+}
+
+int acx_head_ragged(const void* x, const float* ln_w, const float* ln_b, const float* fc_w, const float* fc_b, float* pooled,
+                    float* scene, float* logits, float* probs, int B, int H, int W, int C, int n_cls, int act_dtype,
+                    const int32_t* valid, void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "head_ragged: null valid-length array");
+  return head_impl(x, ln_w, ln_b, fc_w, fc_b, pooled, scene, logits, probs, B, H, W, C, n_cls, act_dtype, valid, stream);
+}
+
+static int nhwc_to_nchw_impl(const void* x, float* out, int B, int H, int W, int C, int act_dtype, const int32_t* valid,
+                             void* stream) {
   ACX_CHECK(x && out && B > 0 && B <= 65535, ACX_ERR_ARG, "nhwc_to_nchw: bad arguments");
+  ACX_CHECK(!valid || (H > 0 && W > 0), ACX_ERR_ARG, "nhwc_to_nchw: H=%d W=%d must be positive", H, W);
   const int HW = H * W;
   dim3 grid(ceil_div(HW, 32), ceil_div(C, 32), B), block(32, 8);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (act_dtype == ACX_BF16)
-    ACX_CUDA(launch_pdl(nhwc_to_nchw_kernel<bf16>, grid, block, 0, st, 1, PDL_SMALL, reinterpret_cast<const bf16*>(x), out, HW, C));
+    ACX_CUDA(launch_pdl(valid ? nhwc_to_nchw_kernel<bf16, true> : nhwc_to_nchw_kernel<bf16>, grid, block, 0, st, 1, PDL_SMALL,
+                        reinterpret_cast<const bf16*>(x), out, HW, C, W, valid));
   else
-    ACX_CUDA(launch_pdl(nhwc_to_nchw_kernel<float>, grid, block, 0, st, 1, PDL_SMALL, reinterpret_cast<const float*>(x), out, HW, C));
+    ACX_CUDA(launch_pdl(valid ? nhwc_to_nchw_kernel<float, true> : nhwc_to_nchw_kernel<float>, grid, block, 0, st, 1, PDL_SMALL,
+                        reinterpret_cast<const float*>(x), out, HW, C, W, valid));
   return ACX_OK;
+}
+
+int acx_nhwc_to_nchw_f32(const void* x, float* out, int B, int H, int W, int C, int act_dtype, void* stream) {
+  return nhwc_to_nchw_impl(x, out, B, H, W, C, act_dtype, nullptr, stream);
+}
+
+int acx_nhwc_to_nchw_f32_ragged(const void* x, float* out, int B, int H, int W, int C, int act_dtype, const int32_t* valid,
+                                void* stream) {
+  ACX_CHECK(valid, ACX_ERR_ARG, "nhwc_to_nchw_ragged: null valid-length array");
+  return nhwc_to_nchw_impl(x, out, B, H, W, C, act_dtype, valid, stream);
 }
 
 int acx_resample_fit(const float* x, int ld_in, const float* taps, float* out, int ld_out, int B, int L_in, int orig,

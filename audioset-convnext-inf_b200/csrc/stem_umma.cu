@@ -42,10 +42,12 @@ __device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi, uin
   lo = (uint32_t)__bfloat16_as_ushort(al) | ((uint32_t)__bfloat16_as_ushort(bl) << 16);
 }
 
+// RAG: clip b has valid[b] frames (clamped to [0, Tn]); later rows are read as the conv's zero padding.
+template <bool RAG = false>
 __global__ void __launch_bounds__(128, 4)
     stem_umma_kernel(const float* __restrict__ logmel, const float* __restrict__ w, const float* __restrict__ bias,
                      const float* __restrict__ ln_w, const float* __restrict__ ln_b, bf16* __restrict__ out, int Tn,
-                     int n_mels, int H0, int W0, long long total, int gp) {
+                     int n_mels, int H0, int W0, long long total, int gp, const int32_t* __restrict__ valid) {
   using Cfg = StemCfg;
   constexpr int CO = Cfg::CO;
   extern __shared__ uint8_t smem_raw[];
@@ -102,11 +104,12 @@ __global__ void __launch_bounds__(128, 4)
     const int ox = (int)(pp % W0);
     const int oy = (int)((pp / W0) % H0);
     const long long b = pp / ((long long)W0 * H0);
+    const int Tb = RAG ? min(max(__ldg(valid + b), 0), Tn) : Tn;
 #pragma unroll
     for (int ky = 0; ky < 4; ++ky) {
       const int t = oy * 4 - 4 + ky;                           // 4 rows of zero padding in time (pad = (4, 0))
       v[ky] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (ok && t >= 0 && t < Tn) v[ky] = __ldg(reinterpret_cast<const float4*>(logmel + ((size_t)b * Tn + t) * n_mels + ox * 4));
+      if (ok && t >= 0 && t < Tb) v[ky] = __ldg(reinterpret_cast<const float4*>(logmel + ((size_t)b * Tn + t) * n_mels + ox * 4));
     }
   };
 
@@ -211,19 +214,21 @@ __global__ void __launch_bounds__(128, 4)
 }
 
 int launch_stem_umma(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b,
-                     void* out, int B, int T, int n_mels, int gp, cudaStream_t st) {
+                     void* out, int B, int T, int n_mels, int gp, const int32_t* valid, cudaStream_t st) {
   using Cfg = StemCfg;
   const int H0 = (T + 4) / 4 + 1, W0 = n_mels / 4;
   const long long total = (long long)B * H0 * W0;
-  ACX_SET_MAX_SMEM(stem_umma_kernel, Cfg::SMEM_BYTES);
+  auto kern = valid ? stem_umma_kernel<true> : stem_umma_kernel<false>;
+  if (valid) ACX_SET_MAX_SMEM(stem_umma_kernel<true>, Cfg::SMEM_BYTES);
+  else ACX_SET_MAX_SMEM(stem_umma_kernel<false>, Cfg::SMEM_BYTES);
   int dev = 0, sms = 0;
   ACX_CUDA(cudaGetDevice(&dev));
   ACX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const long long tiles = (total + Cfg::BM - 1) / Cfg::BM;
   const long long want = 4LL * sms;                              // 4 resident CTAs per SM (4 x 128 TMEM columns)
   const int grid = (int)(tiles < want ? tiles : want);
-  ACX_CUDA(launch_pdl(stem_umma_kernel, dim3(grid), dim3(128), Cfg::SMEM_BYTES, st, 1, PDL_SMALL, logmel, w, bias, ln_w, ln_b,
-                      reinterpret_cast<bf16*>(out), T, n_mels, H0, W0, total, gp));
+  ACX_CUDA(launch_pdl(kern, dim3(grid), dim3(128), Cfg::SMEM_BYTES, st, 1, PDL_SMALL, logmel, w, bias, ln_w, ln_b,
+                      reinterpret_cast<bf16*>(out), T, n_mels, H0, W0, total, gp, valid));
   return ACX_OK;
 }
 

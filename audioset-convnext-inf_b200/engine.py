@@ -202,6 +202,36 @@ def out_time_dims(L):
     return T, hs
 
 
+MIN_RAGGED_LEN = 7360      # shortest clip with h3 >= 1 (it also reflects: L > N_FFT / 2)
+
+
+def check_lengths(lengths, B, L):
+    """Per-clip lengths of a ragged batch -> list of B ints in [MIN_RAGGED_LEN, L]; ValueError otherwise."""
+    if isinstance(lengths, torch.Tensor):
+        if lengths.device.type != "cpu":
+            raise ValueError("lengths must be a host sequence or a CPU tensor")
+        lengths = lengths.tolist()
+    try:
+        ls = [int(n) for n in lengths]
+    except (TypeError, ValueError) as e:
+        raise ValueError(f"lengths must be a sequence of integers: {e}") from e
+    if len(ls) != B:
+        raise ValueError(f"lengths has {len(ls)} entries for a batch of {B} clips")
+    bad = [n for n in ls if not MIN_RAGGED_LEN <= n <= L]
+    if bad:
+        raise ValueError(f"every length must lie in [{MIN_RAGGED_LEN}, {L}] (the canvas), got {bad[:4]}")
+    return ls
+
+
+def ragged_table(lengths):
+    """(6, n) int32 table of a ragged chunk: per clip L, T, h0, h1, h2, h3 (the bound each kernel family reads)."""
+    rows = []
+    for n in lengths:
+        T, hs = out_time_dims(n)
+        rows.append([n, T] + hs)
+    return torch.tensor(rows, dtype=torch.int32).t().contiguous()
+
+
 class Engine:
     def __init__(self, state_dict, device, precision="bf16", chunk=None, frontend=None, mlp=None):
         self.lib = N.load()
@@ -288,6 +318,7 @@ class Engine:
         ws["logits"] = torch.empty(n, N_CLASSES, device=dev, dtype=torch.float32)
         ws["probs"] = torch.empty(n, N_CLASSES, device=dev, dtype=torch.float32)
         ws["frame"] = torch.empty(n, DIMS[3], hs[3], 7, device=dev, dtype=torch.float32)
+        ws["valid"] = torch.empty(6 * n, device=dev, dtype=torch.int32)     # ragged batches: ragged_table of the chunk
         ws["graphs"] = {}         # (n, trunk, head, frame) -> (CUDAGraph, launches per replay); dies with the buffers
         ws["uses"] = {}
         while len(self._ws) >= max(1, self.max_workspaces):
@@ -306,6 +337,13 @@ class Engine:
         N.call(name, *args)
         e1.record()
         self._prof.append((tag, e0, e1))
+
+    def _call_v(self, tag, name, valid, *args):
+        """`name`, or with a per-clip bound (device pointer `valid`) its _ragged twin, which takes it before the stream."""
+        if valid:
+            self._call(tag, name + "_ragged", *args[:-1], valid, args[-1])
+        else:
+            self._call(tag, name, *args)
 
     def profile(self, wave, want=("logits",)):
         """Run once with a CUDA-event pair around every kernel launch (serialised on the current
@@ -375,19 +413,24 @@ class Engine:
         return "hbm", 0.0
 
     # ---- stages (each is one libacx call) ----------------------------------------------------------
-    def _wave_prep(self, wave, ws, n, L, st):
-        """Reads the caller's tensor -> stays outside any captured graph."""
+    def _wave_prep(self, wave, ws, n, L, st, rv=None):
+        """Reads the caller's tensor -> stays outside any captured graph.  rv: the ragged chunk's bound pointers or None."""
         ld_pad = ws["ld_pad"]
         fn = "acx_wave_prep_pcm16" if wave.dtype == torch.int16 else "acx_wave_prep"
         if self.frontend == "folded":
             fn = "acx_frame_fold_pcm16" if wave.dtype == torch.int16 else "acx_frame_fold"
-            self._call("frame_fold", fn, wave.data_ptr(), ws["f_hi"].data_ptr(), ws["f_lo"].data_ptr(), n, L, ws["T"], N_FFT, HOP, st)
+            args = (wave.data_ptr(), ws["f_hi"].data_ptr(), ws["f_lo"].data_ptr(), n, L, ws["T"], N_FFT, HOP)
+            tag = "frame_fold"
         elif self.frontend == "fused":
-            self._call("wave_prep", fn, wave.data_ptr(), ws["wav_hi"].data_ptr(), ws["wav_lo"].data_ptr(),
-                       n, L, N_FFT, ld_pad, N.ACX_BF16, st)
+            args = (wave.data_ptr(), ws["wav_hi"].data_ptr(), ws["wav_lo"].data_ptr(), n, L, N_FFT, ld_pad, N.ACX_BF16)
+            tag = "wave_prep"
         else:
-            self._call("wave_prep", fn, wave.data_ptr(), ws["wav_pad"].data_ptr(), 0, n, L, N_FFT, ld_pad,
-                       N.ACX_F32, st)
+            args = (wave.data_ptr(), ws["wav_pad"].data_ptr(), 0, n, L, N_FFT, ld_pad, N.ACX_F32)
+            tag = "wave_prep"
+        if rv:
+            self._call(tag, fn + "_ragged", *args, L, rv[0], st)       # rows of the (n, L) chunk are L samples apart
+        else:
+            self._call(tag, fn, *args, st)
 
     def _frontend(self, ws, n, L, st):
         w = self.w
@@ -414,22 +457,24 @@ class Engine:
         else:
             self._call(tag, "acx_gemm_f32", a, M * K, M, K, wt, out, Nn, M, Nn, K, epi, bias, gamma, resid, st)
 
-    def _trunk(self, ws, n, st):
+    def _trunk(self, ws, n, st, rv=None):
         w = self.w
         x, y, hid = ws["x"].data_ptr(), ws["y"].data_ptr(), ws["hid"].data_ptr()
         xgp = ws["xg"].data_ptr() if "xg" in ws else 0      # planar residual stream; trades places with y at a fused downsample
         fused0 = self.mlp == "fused" and self.dwconv == "tc" and 0 in self.dwconv_tc_stages and self.gp
         stem_gp = fused0 and os.environ.get("ACX_STEM", "") != "simt"     # the stem writes stage 0's planar layout itself
+        rT = rv[1] if rv else 0
         if stem_gp:
-            self._call("stem", "acx_stem_gp", ws["logmel"].data_ptr(), w.stem_w.data_ptr(), w.stem_b.data_ptr(),
-                       w.stem_ln_w.data_ptr(), w.stem_ln_b.data_ptr(), xgp, n, ws["T"], N_MELS, st)
+            self._call_v("stem", "acx_stem_gp", rT, ws["logmel"].data_ptr(), w.stem_w.data_ptr(), w.stem_b.data_ptr(),
+                         w.stem_ln_w.data_ptr(), w.stem_ln_b.data_ptr(), xgp, n, ws["T"], N_MELS, st)
         else:
-            self._call("stem", "acx_stem", ws["logmel"].data_ptr(), w.stem_w.data_ptr(), w.stem_b.data_ptr(),
-                       w.stem_ln_w.data_ptr(), w.stem_ln_b.data_ptr(), x, n, ws["T"], N_MELS, self.adt, st)
+            self._call_v("stem", "acx_stem", rT, ws["logmel"].data_ptr(), w.stem_w.data_ptr(), w.stem_b.data_ptr(),
+                         w.stem_ln_w.data_ptr(), w.stem_ln_b.data_ptr(), x, n, ws["T"], N_MELS, self.adt, st)
         Wd = 56
         entered_gp = False          # the previous downsample GEMM already wrote this stage's planar input
         for s in range(4):
             C, H = DIMS[s], ws["hs"][s]
+            rh = rv[2 + s] if rv else 0         # ragged: each clip's own height at this stage
             M = n * H * Wd
             fused_mlp = self.mlp == "fused" and C in (96, 192)
             tc = self.dwconv == "tc" and s in self.dwconv_tc_stages
@@ -441,7 +486,7 @@ class Engine:
                     self._call(f"to_gp_c{C}", "acx_gp_transpose", x, xg, M, C, 1, st)
                 stats = ws["stats"].data_ptr()
                 for blk in w.blocks[s]:
-                    self._call(f"dwconv_tc_c{C}", "acx_dwconv_tc_gp", xg, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), vg, n, H, Wd, C, st)
+                    self._call_v(f"dwconv_tc_c{C}", "acx_dwconv_tc_gp", rh, xg, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), vg, n, H, Wd, C, st)
                     self._call(f"row_stats_c{C}", "acx_gp_row_stats", vg, stats, M, C, st)
                     self._call(f"pw1_gelu_k{C}_n{4 * C}", "acx_gemm_bf16_pw1_gp", vg, blk["w1f"].data_ptr(), hid, M, 4 * C, C,
                                blk["b1f"].data_ptr(), stats, blk["s1"].data_ptr(), st)
@@ -454,7 +499,7 @@ class Engine:
                     self._call(f"to_gp_c{C}", "acx_gp_transpose", x, xg, M, C, 1, st)
             for blk in (() if gp2 else w.blocks[s]):
                 if gp:
-                    self._call(f"dwconv_tc_c{C}", "acx_dwconv_tc_gp", xg, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), vg, n, H, Wd, C, st)
+                    self._call_v(f"dwconv_tc_c{C}", "acx_dwconv_tc_gp", rh, xg, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), vg, n, H, Wd, C, st)
                     # the LayerNorm runs inside the MLP kernel: folded into pwconv1 as a rank-1 epilogue correction
                     # ("fused", default) or applied to the operand tile in shared memory (ACX_LN=smem)
                     if self.ln_mode == "smem":
@@ -468,13 +513,13 @@ class Engine:
                     continue
                 ln_fused = False
                 if tc:
-                    self._call(f"dwconv_tc_c{C}", "acx_dwconv_tc", x, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), y, n, H, Wd, C, st)
+                    self._call_v(f"dwconv_tc_c{C}", "acx_dwconv_tc", rh, x, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), y, n, H, Wd, C, st)
                     ln_fused = fused_mlp and self.ln_mode == "fused"
                     if not ln_fused:
                         self._call(f"ln_rows_c{C}", "acx_layernorm_rows", y, blk["ln_w"].data_ptr(), blk["ln_b"].data_ptr(), y, M, C, st)
                 else:
-                    self._call(f"dwconv_ln_c{C}", "acx_dwconv_ln", x, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(), blk["ln_w"].data_ptr(),
-                               blk["ln_b"].data_ptr(), y, n, H, Wd, C, self.adt, st)
+                    self._call_v(f"dwconv_ln_c{C}", "acx_dwconv_ln", rh, x, blk["dw_w"].data_ptr(), blk["dw_b"].data_ptr(),
+                                 blk["ln_w"].data_ptr(), blk["ln_b"].data_ptr(), y, n, H, Wd, C, self.adt, st)
                 if ln_fused:
                     self._call(f"mlp_fused_c{C}", "acx_mlp_fused_ln", y, x, blk["ln_w"].data_ptr(), blk["ln_b"].data_ptr(),
                                blk["w1"].data_ptr(), blk["b1"].data_ptr(), blk["w2"].data_ptr(), blk["b2"].data_ptr(),
@@ -512,47 +557,69 @@ class Engine:
                 else:
                     self._gemm(y, d["w"].data_ptr(), x, Mo, 2 * C, 4 * C, N.EPI_BIAS, d["b"].data_ptr(), 0, 0, st)
 
-    def _body(self, ws, n, L, st, trunk, need_head, need_frame):
-        """Everything after wave_prep for one chunk; writes only into the workspace (graph-capturable)."""
+    @staticmethod
+    def _ragged_ptrs(ws, n, ragged):
+        """Device pointers of the six rows of the chunk's (6, n) bound table in ws["valid"], or None."""
+        if not ragged:
+            return None
+        base = ws["valid"].data_ptr()
+        return [base + 4 * k * n for k in range(6)]
+
+    def _body(self, ws, n, L, st, trunk, need_head, need_frame, ragged=False):
+        """Everything after wave_prep for one chunk; writes only into the workspace (graph-capturable).  ragged: the
+        kernels read each clip's bounds from ws["valid"] (data, so one graph serves every length mix)."""
+        rv = self._ragged_ptrs(ws, n, ragged)
         self._frontend(ws, n, L, st)
         if not trunk:
             return
-        self._trunk(ws, n, st)
+        self._trunk(ws, n, st, rv)
         x = ws["x"].data_ptr()
         h3 = ws["hs"][3]
+        rh3 = rv[5] if rv else 0
         if need_head:
             w = self.w
-            self._call("head", "acx_head", x, w.norm_w.data_ptr(), w.norm_b.data_ptr(), w.fc_w.data_ptr(),
-                       w.fc_b.data_ptr(), ws["pooled"].data_ptr(), ws["scene"].data_ptr(), ws["logits"].data_ptr(),
-                       ws["probs"].data_ptr(), n, h3, 7, DIMS[3], N_CLASSES, self.adt, st)
+            self._call_v("head", "acx_head", rh3, x, w.norm_w.data_ptr(), w.norm_b.data_ptr(), w.fc_w.data_ptr(),
+                         w.fc_b.data_ptr(), ws["pooled"].data_ptr(), ws["scene"].data_ptr(), ws["logits"].data_ptr(),
+                         ws["probs"].data_ptr(), n, h3, 7, DIMS[3], N_CLASSES, self.adt, st)
         if need_frame:
-            self._call("frame_nchw", "acx_nhwc_to_nchw_f32", x, ws["frame"].data_ptr(), n, h3, 7, DIMS[3], self.adt, st)
+            self._call_v("frame_nchw", "acx_nhwc_to_nchw_f32", rh3, x, ws["frame"].data_ptr(), n, h3, 7, DIMS[3], self.adt, st)
 
-    def _capture(self, ws, n, L, trunk, need_head, need_frame):
+    def _capture(self, ws, n, L, trunk, need_head, need_frame, ragged=False):
         """Capture the chunk's ~65 launches into one CUDA graph (fixed workspace pointers, tensor maps baked
         into the kernel parameters); one eager pass first so per-kernel attributes are already set."""
         st = torch.cuda.current_stream(self.device).cuda_stream
         before = self.launches
-        self._body(ws, n, L, st, trunk, need_head, need_frame)
+        self._body(ws, n, L, st, trunk, need_head, need_frame, ragged)
         per_replay = self.launches - before
         torch.cuda.synchronize(self.device)
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
             cst = torch.cuda.current_stream(self.device).cuda_stream
-            self._body(ws, n, L, cst, trunk, need_head, need_frame)
+            self._body(ws, n, L, cst, trunk, need_head, need_frame, ragged)
         self.launches = before                     # the eager pass is replaced by the first replay; capture launches nothing
         return g, per_replay
 
     # ---- public -----------------------------------------------------------------------------------
-    def run(self, wave, want=("logits",)):
+    def run(self, wave, want=("logits",), lengths=None):
         """wave: (B, L) float32 CUDA tensor (or int16 PCM, converted x / 32767. on the fly).  want: subset of {"logits", "scene", "frame", "logmel"}.
-        Returns dict of fp32 tensors: probs/logits (B,527), scene (B,768), frame (B,768,T',7)."""
+        Returns dict of fp32 tensors: probs/logits (B,527), scene (B,768), frame (B,768,T',7).
+
+        lengths (B ints on the host, each in [MIN_RAGGED_LEN, L]): a ragged batch.  Clip b is wave[b, :lengths[b]] and its
+        results equal a run of that clip alone; samples past it are never read, and frame rows past its own h3 are zero.
+        Checked here, before any launch.  fp32 waveforms only; "logmel" is not available (its tail rows are not masked)."""
         assert wave.is_cuda and wave.dim() == 2 and wave.is_contiguous()
         assert wave.dtype in (torch.float32, torch.int16), "waveform must be float32 or int16 PCM"
         B, L = wave.shape
         T, hs = out_time_dims(L)
         if hs[3] < 1:
             raise ValueError(f"clip of {L} samples is too short for the 4-stage trunk")
+        ragged = lengths is not None
+        if ragged:
+            lengths = check_lengths(lengths, B, L)
+            if "logmel" in want:
+                raise ValueError("a ragged batch has no log-mel output (its rows past each clip's end are not masked)")
+            if wave.dtype != torch.float32:
+                raise ValueError("a ragged batch takes a float32 waveform")
         dev = self.device
         out = {}
         need_head = "logits" in want or "scene" in want
@@ -570,9 +637,15 @@ class Engine:
             for b0 in range(0, B, self.chunk):
                 n = min(self.chunk, B - b0)
                 ws = self._workspace(min(self.chunk, B), L)
-                self._wave_prep(wave[b0:b0 + n], ws, n, L, st)
+                rv = None
+                if ragged:
+                    # a fresh pinned host tensor per chunk: the caching host allocator keeps it until the copy has run
+                    tab = ragged_table(lengths[b0:b0 + n]).pin_memory()
+                    ws["valid"][:6 * n].view(6, n).copy_(tab, non_blocking=True)
+                    rv = self._ragged_ptrs(ws, n, True)
+                self._wave_prep(wave[b0:b0 + n], ws, n, L, st, rv)
                 trunk = need_head or "frame" in want
-                key = (n, L, trunk, need_head, "frame" in want)
+                key = (n, L, trunk, need_head, "frame" in want, ragged)
                 g = ws["graphs"].get(key) if (self.use_graph and self._prof is None) else None
                 if g is None and self.use_graph and self._prof is None:
                     ws["uses"][key] = ws["uses"].get(key, 0) + 1

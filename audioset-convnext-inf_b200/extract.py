@@ -1,13 +1,16 @@
 """Counterpart of the reference's per-file extraction loop (pytorch/extract_embeddings.py:64-92: one forward per wav,
 whatever its length) for a LIST of variable-length clips (SURVEY §8 row f3).
 
-The model's result for a clip depends on its exact length (reflect padding, frame count), so clips are never padded
-to a common length: they are bucketed by EXACT length, every bucket runs as batched forwards, and the outputs are
-returned in the caller's order -- identical to looping clip by clip, at batch throughput."""
+The model's result for a clip depends on its exact length (reflect padding, frame count), so clips are never simply
+zero-padded to a common length.  They run as RAGGED batches instead (ConvNeXt.forward_all(x, lengths=...)): clips of
+similar length share a canvas, and every kernel bounds each clip by its own length.  The outputs are returned in the
+caller's order -- identical to looping clip by clip, at batch throughput."""
 import collections
 
 import numpy as np
 import torch
+
+CANVAS_STEP = 32000        # canvases are whole seconds: few distinct workspace shapes (and CUDA graphs) per clip list
 
 
 def length_buckets(lengths, max_batch):
@@ -22,17 +25,34 @@ def length_buckets(lengths, max_batch):
     return out
 
 
+def ragged_batches(lengths, max_batch, step=CANVAS_STEP):
+    """[(canvas, [indices...])...]: indices sorted by length (ties in input order), cut into runs of at most max_batch;
+    each run's canvas is its longest length rounded up to a multiple of `step`."""
+    order = sorted(range(len(lengths)), key=lambda i: (int(lengths[i]), i))
+    out = []
+    for s in range(0, len(order), max_batch):
+        idx = order[s:s + max_batch]
+        longest = max(int(lengths[i]) for i in idx)
+        out.append(((longest + step - 1) // step * step, idx))
+    return out
+
+
 def extract_clipwise(model, waveforms, max_batch=64, want=("clipwise_logits",)):
     """waveforms: sequence of 1-D float arrays / tensors at 32 kHz (any lengths).  Returns {name: list of per-clip
-    tensors on the host, in input order} for the names in `want` (keys of ConvNeXt.forward_all)."""
+    tensors on the host, in input order} for the names in `want` (keys of ConvNeXt.forward_all); a clip's
+    "frame_embeddings" cover its own frames only, like a forward of that clip alone."""
     dev = next(model.parameters()).device
+    lengths = [len(w) for w in waveforms]
     res = {k: [None] * len(waveforms) for k in want}
-    for n, idx in length_buckets([len(w) for w in waveforms], max_batch):
-        batch = torch.stack([torch.as_tensor(np.asarray(waveforms[i]), dtype=torch.float32) for i in idx]).to(dev)
+    for canvas, idx in ragged_batches(lengths, max_batch):
+        batch = torch.zeros(len(idx), canvas, dtype=torch.float32)
+        for j, i in enumerate(idx):
+            batch[j, :lengths[i]] = torch.as_tensor(np.asarray(waveforms[i]), dtype=torch.float32)
         with torch.no_grad():
-            out = model.forward_all(batch)
+            out = model.forward_all(batch.to(dev), lengths=[lengths[i] for i in idx])
+        frames = out["frame_lengths"].tolist()
         for k in want:
-            host = out[k].float().cpu()
+            host = out[k].cpu() if k == "frame_lengths" else out[k].float().cpu()
             for j, i in enumerate(idx):
-                res[k][i] = host[j]
+                res[k][i] = host[j, :, :frames[j]] if k == "frame_embeddings" else host[j]
     return res

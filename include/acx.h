@@ -201,6 +201,40 @@ ACX_API int acx_head(const void* x, const float* ln_w, const float* ln_b, const 
 /* x (B,H,W,C) act_dtype -> out (B,C,H,W) fp32: the layout forward_frame_embeddings returns (CX:399-402). */
 ACX_API int acx_nhwc_to_nchw_f32(const void* x, float* out, int B, int H, int W, int C, int act_dtype, void* stream);
 
+/* ---- ragged batches: clips of different lengths in one launch sequence -------------------------------------------------
+ * Clip b sits in row b of a canvas sized for the longest clip; every size argument is the CANVAS size.  `valid` (device,
+ * B int32 entries) gives each clip's own extent in the unit the kernel bounds:
+ *   acx_wave_prep_ragged, acx_frame_fold_ragged   samples L_b (the input rows are ld_wave apart, ld_wave >= L)
+ *   acx_stem_ragged, acx_stem_gp_ragged           frames  T_b = L_b / hop + 1
+ *   acx_dwconv_*_ragged                           rows    h_b of the stage (h0_b = (T_b + 4) / 4 + 1, h(s+1)_b = h(s)_b / 2)
+ *   acx_head_ragged, acx_nhwc_to_nchw_f32_ragged  rows    h3_b of the last stage
+ * A clip's rows past its extent are never read: the prep kernels reflect at L_b and write zeros past L_b + n_fft, the
+ * convolutions read those rows as their own zero padding, the head pools over h3_b rows, and the frame transpose writes
+ * zeros there.  Rows below the extent therefore equal a run of the clip alone at its own length, bit for bit; rows past
+ * it hold values without meaning.  The kernels clamp each entry to the canvas (and to what their indexing needs: > n_fft/2
+ * samples for the prep kernels, >= 1 row for the head), so no value can make them access memory outside their buffers;
+ * whether the values are right (L_b > n_fft/2, h3_b >= 1, entries consistent with each other) is for the caller to check.
+ * A null `valid` returns ACX_ERR_ARG. */
+ACX_API int acx_wave_prep_ragged(const float* wave, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
+                                 int ld_wave, const int32_t* valid, void* stream);
+ACX_API int acx_frame_fold_ragged(const float* wave, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop,
+                                  int ld_wave, const int32_t* valid, void* stream);
+ACX_API int acx_stem_ragged(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b,
+                            void* out, int B, int T, int n_mels, int act_dtype, const int32_t* valid, void* stream);
+ACX_API int acx_stem_gp_ragged(const float* logmel, const float* w, const float* bias, const float* ln_w, const float* ln_b,
+                               void* out, int B, int T, int n_mels, const int32_t* valid, void* stream);
+ACX_API int acx_dwconv_tc_ragged(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                                 const int32_t* valid, void* stream);
+ACX_API int acx_dwconv_tc_gp_ragged(const void* x, const void* w, const float* bias, void* v, int B, int H, int W, int C,
+                                    const int32_t* valid, void* stream);
+ACX_API int acx_dwconv_ln_ragged(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
+                                 void* y, int B, int H, int W, int C, int act_dtype, const int32_t* valid, void* stream);
+ACX_API int acx_head_ragged(const void* x, const float* ln_w, const float* ln_b, const float* fc_w, const float* fc_b,
+                            float* pooled, float* scene, float* logits, float* probs, int B, int H, int W, int C, int n_cls,
+                            int act_dtype, const int32_t* valid, void* stream);
+ACX_API int acx_nhwc_to_nchw_f32_ragged(const void* x, float* out, int B, int H, int W, int C, int act_dtype,
+                                        const int32_t* valid, void* stream);
+
 /* ---- next row (f4): demo preprocessing, reference demo_convnext.py:52-67 --------------------- */
 /* torchaudio.functional.resample (sinc_interp_hann polyphase FIR, demo_convnext.py:53-59) fused with the demo's
  * constant pad / crop to a fixed clip length (demo_convnext.py:61-67):
