@@ -60,6 +60,12 @@ SIGNATURES = {
     "acx_dwconv_ln_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "acx_head_ragged": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "acx_nhwc_to_nchw_f32_ragged": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
+    # windows of one long recording: recording, its length, the (B,) int64 window offsets and the optional ragged lengths
+    # first, then the arguments of the dense prep entry point
+    "acx_wave_prep_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
+    "acx_wave_prep_pcm16_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
+    "acx_frame_fold_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
+    "acx_frame_fold_pcm16_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
 }
 
 

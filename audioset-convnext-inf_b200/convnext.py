@@ -22,6 +22,7 @@ import torch.nn as nn
 from . import _native
 from .engine import DEPTHS, DIMS, Engine, out_time_dims
 from .frontend_consts import slaney_mel_filterbank, windowed_dft
+from .windows import plan_windows
 
 HF_PYTORCH_WEIGHTS_NAME = "model.safetensors"
 HF_CONFIG_NAME = "config.yaml"
@@ -177,16 +178,24 @@ class ConvNeXt(nn.Module):
             self._engine_key = key
         return self._engine
 
-    def _prep(self, x, mixup_lambda):
+    def _check_inference(self, mixup_lambda):
         if self.training:
             raise RuntimeError("inference only: call model.eval() first (the reference's training-mode branches -- "
                                "augmentation, SpecAugment, mixup, BatchNorm updates -- are out of scope)")
         if mixup_lambda is not None:
             raise NotImplementedError("mixup is training-only")
+
+    def _prep(self, x, mixup_lambda):
+        self._check_inference(mixup_lambda)
         if x.dim() != 2:
             raise ValueError(f"expected a (batch, samples) waveform, got shape {tuple(x.shape)}")
         eng = self._get_engine()
         x = x.detach().to(device=eng.device, dtype=torch.float32).contiguous()
+        self._check_amplitude(eng, x)
+        return eng, x
+
+    @staticmethod
+    def _check_amplitude(eng, x):
         if os.environ.get("ACX_CHECK_AMPLITUDE") == "1" and eng.precision == "bf16" and x.numel():
             # debugging aid (one reduction + sync per call): the bf16-mode front end carries samples as 2^8-scaled fp16
             # pairs, so |x| must stay below 255 (INTEGRATION.md, input contract); the fp32-accurate mode has no such bound
@@ -194,7 +203,6 @@ class ConvNeXt(nn.Module):
             if not amax < 255.0:
                 raise ValueError(f"waveform amplitude {amax:g} exceeds the bf16-mode front end's range (|x| < 255): "
                                  "normalise to [-1, 1] like torchaudio.load / int16 / 32767, or use set_precision('fp32')")
-        return eng, x
 
     # ---- the three inference entry points --------------------------------------------------------
     def forward(self, x, mixup_lambda=None):
@@ -226,6 +234,61 @@ class ConvNeXt(nn.Module):
         if lengths is not None:
             h3 = [out_time_dims(int(n))[1][3] for n in lengths]
             res["frame_lengths"] = torch.tensor(h3, dtype=torch.int64).to(x.device)
+        return res
+
+    def forward_windows(self, recordings, window_samples=320000, hop_samples=32000, frame_embeddings=False):
+        """Tag long recordings window by window, each window as a clip of its own (the model's training condition).
+
+        recordings: one 1-D tensor or a sequence of 1-D tensors of any lengths, on the host or the device; float32, int16
+        PCM (converted x / 32767. in the prep kernel) or any other float dtype (converted to float32).  Windows of
+        `window_samples` start every `hop_samples` samples; a recording whose windows do not end at its last sample gets
+        one more, end-aligned window, and one shorter than a window gets one window at its own length
+        (windows.plan_windows).  The windows are read in place from one buffer holding the recordings end to end (int16
+        when every recording is int16, else float32), never copied out, and may overlap.
+
+        Returns, on the model's device, one row per window in recording order, start ascending: "clipwise_output" and
+        "clipwise_logits" (N, 527), "scene_embeddings" (N, 768), and (N,) int64 "recording", "start" and "length"; with
+        frame_embeddings=True also "frame_embeddings" (N, 768, T', 7), T' the frame count of a full window, zero past each
+        window's own count, which "frame_lengths" gives.  Row i equals
+        forward_all(recordings[recording_i][start_i : start_i + length_i][None]) bit for bit, and a window never reads a
+        sample outside itself.  Every argument is checked before anything is launched."""
+        self._check_inference(None)
+        if isinstance(recordings, torch.Tensor):
+            recordings = [recordings]
+        recs = [r if isinstance(r, torch.Tensor) else torch.as_tensor(r) for r in recordings]
+        for i, r in enumerate(recs):
+            if r.dim() != 1:
+                raise ValueError(f"recording {i} must be 1-D (samples), got shape {tuple(r.shape)}")
+            if not (r.dtype == torch.int16 or r.is_floating_point()):
+                raise ValueError(f"recording {i} has dtype {r.dtype}: expected a float dtype or int16 PCM")
+        plan = plan_windows([r.numel() for r in recs], window_samples, hop_samples)
+        eng = self._get_engine()
+        dev = eng.device
+        pcm = bool(recs) and all(r.dtype == torch.int16 for r in recs)
+        if len(recs) == 1 and recs[0].device == dev and recs[0].dtype in (torch.float32, torch.int16) and recs[0].is_contiguous():
+            buf = recs[0].detach()
+        else:
+            buf = torch.empty(sum(r.numel() for r in recs),
+                              dtype=torch.int16 if pcm else torch.float32, device=dev)
+            base = 0
+            for r in recs:
+                dst = buf[base:base + r.numel()]
+                if r.dtype == torch.int16 and not pcm:
+                    # the prep kernels' conversion, a correctly rounded fp32 division (not a reciprocal multiply)
+                    torch.div(r.detach().to(dev).to(torch.float32), torch.tensor(32767.0, device=dev), out=dst)
+                else:
+                    dst.copy_(r.detach())
+                base += r.numel()
+        if not pcm:
+            self._check_amplitude(eng, buf)
+        want = ("logits", "scene", "frame") if frame_embeddings else ("logits", "scene")
+        out = eng.run_windows(buf, plan, want)
+        res = {"clipwise_output": out["probs"], "clipwise_logits": out["logits"], "scene_embeddings": out["scene"],
+               "recording": plan.recording.to(dev), "start": plan.start.to(dev), "length": plan.length.to(dev)}
+        if frame_embeddings:
+            res["frame_embeddings"] = out["frame"]
+            h3 = [out_time_dims(n)[1][3] for n in plan.length.tolist()]
+            res["frame_lengths"] = torch.tensor(h3, dtype=torch.int64).to(dev)
         return res
 
     def forward_logmel(self, x):

@@ -306,10 +306,14 @@ __device__ __forceinline__ float ff_sample(const int16_t* p) { return __fdiv_rn(
 
 // RAG: row b is a clip of valid[b] samples (clamped to [n_fft/2 + 1, L]) at row pitch ld_wave, reflected at its own end and
 // zero past the reflected range; samples past valid[b] are never read.
-template <typename TIn, bool RAG = false>
+// WIN: row b is the window that starts offsets[b] samples into ONE recording of rec_len samples (windows may overlap), of
+// L samples or with RAG its own valid[b]; offsets are 64-bit.  Length and offset are clamped to the recording, so no table
+// value can make the kernel read outside it.
+template <typename TIn, bool RAG = false, bool WIN = false>
 __global__ void __launch_bounds__(256) frame_fold_kernel(const TIn* __restrict__ wave, __half* __restrict__ fhi, __half* __restrict__ flo,
                                                          int L, int T, int n_fft, int hop, int ld_wave,
-                                                         const int32_t* __restrict__ valid) {
+                                                         const int32_t* __restrict__ valid,
+                                                         const long long* __restrict__ offsets = nullptr, long long rec_len = 0) {
   // thread = (frame t, four consecutive fold indices j0 .. j0 + 3): 8-byte stores of E and O, hi and lo
   const int b = blockIdx.y;
   const int half_n = n_fft >> 1;
@@ -319,9 +323,13 @@ __global__ void __launch_bounds__(256) frame_fold_kernel(const TIn* __restrict__
   const int t = (int)(idx / per_frame), j0 = (int)(idx - (long long)t * per_frame) * 4;
   const TIn* w = wave + (size_t)b * (RAG ? ld_wave : L);
   if (RAG) L = min(max(__ldg(valid + b), half_n + 1), L);
+  if (WIN) {
+    L = (int)min((long long)L, rec_len);
+    w = wave + min(max(__ldg(offsets + b), 0LL), rec_len - L);
+  }
   const int s = t * hop - half_n;              // un-padded sample index of frame position 0 (center = True)
   auto x = [&](int m) {
-    if (RAG && m >= L + half_n) return 0.f;    // past the padded clip: only frames >= the clip's own frame count get here
+    if ((RAG || WIN) && m >= L + half_n) return 0.f;    // past the padded clip: only frames >= its own frame count get here
     if (m < 0) m = -m;                         // reflect (edge sample not repeated), as F.pad(mode="reflect")
     if (m >= L) m = 2 * (L - 1) - m;
     return ff_sample(w + m);
@@ -396,6 +404,40 @@ extern "C" int acx_frame_fold_ragged(const float* wave, void* f_hi, void* f_lo, 
 }
 extern "C" int acx_frame_fold_pcm16(const int16_t* pcm, void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
   return frame_fold_impl(pcm, 1, f_hi, f_lo, B, L, T, n_fft, hop, L, nullptr, stream);
+}
+
+template <typename TIn>
+static int frame_fold_windows(const TIn* rec, long long rec_len, const long long* offsets, const int32_t* valid, void* f_hi,
+                              void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
+  ACX_CHECK(rec && offsets, ACX_ERR_ARG, "frame_fold_windows: null recording or offsets");
+  ACX_CHECK(rec_len >= n_fft / 2 + 1, ACX_ERR_ARG, "frame_fold_windows: rec_len=%lld must be > n_fft/2 (reflect padding)",
+            rec_len);
+  ACX_CHECK(B >= 1, ACX_ERR_ARG, "frame_fold_windows: empty batch B=%d", B);
+  ACX_CHECK(f_hi && f_lo, ACX_ERR_ARG, "frame_fold_windows: null pointer");
+  ACX_CHECK(n_fft == 1024 && hop == 320, ACX_ERR_UNSUPPORTED, "frame_fold: built for n_fft=1024, hop=320 (reference convnext.py:161-174)");
+  ACX_CHECK(B <= 65535 && L > n_fft / 2 && T == L / hop + 1, ACX_ERR_ARG,
+            "frame_fold_windows: bad sizes B=%d L=%d T=%d (reflect padding needs L > n_fft/2, T = L / hop + 1)", B, L, T);
+  ACX_CHECK(((reinterpret_cast<uintptr_t>(f_hi) | reinterpret_cast<uintptr_t>(f_lo)) & 15) == 0, ACX_ERR_ARG, "frame_fold: 16-byte alignment");
+  const long long work = (long long)T * (n_fft / 8);
+  dim3 grid((unsigned)((work + 255) / 256), B);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  __half* hi = reinterpret_cast<__half*>(f_hi);
+  __half* lo = reinterpret_cast<__half*>(f_lo);
+  if (valid)
+    frame_fold_kernel<TIn, true, true><<<grid, 256, 0, st>>>(rec, hi, lo, L, T, n_fft, hop, L, valid, offsets, rec_len);
+  else
+    frame_fold_kernel<TIn, false, true><<<grid, 256, 0, st>>>(rec, hi, lo, L, T, n_fft, hop, L, nullptr, offsets, rec_len);
+  ACX_CUDA(cudaGetLastError());
+  return ACX_OK;
+}
+
+extern "C" int acx_frame_fold_windows(const float* rec, long long rec_len, const long long* offsets, const int32_t* valid,
+                                      void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
+  return frame_fold_windows<float>(rec, rec_len, offsets, valid, f_hi, f_lo, B, L, T, n_fft, hop, stream);
+}
+extern "C" int acx_frame_fold_pcm16_windows(const int16_t* rec, long long rec_len, const long long* offsets, const int32_t* valid,
+                                            void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream) {
+  return frame_fold_windows<int16_t>(rec, rec_len, offsets, valid, f_hi, f_lo, B, L, T, n_fft, hop, stream);
 }
 
 extern "C" int acx_frontend_folded(const void* f_hi, const void* f_lo, const void* w_hi, const void* w_lo, const void* mel_hi,

@@ -23,14 +23,23 @@ __device__ __forceinline__ float load_sample(const int16_t* p) { return __fdiv_r
 
 // RAG: row b is a clip of valid[b] samples (clamped to [pad + 1, L]) at row pitch ld_wave; it is reflected at its own end
 // and zero past it, exactly like a run at that length.  Samples past valid[b] are never read.
-template <bool kSplit, typename TIn, bool RAG = false>
+// WIN: row b is the window that starts offsets[b] samples into ONE recording of rec_len samples (windows may overlap); it
+// has L samples, or with RAG its own valid[b].  Offsets are 64-bit.  The length is clamped to rec_len and the offset to
+// [0, rec_len - length], so no table value can make the kernel read outside the recording.
+template <bool kSplit, typename TIn, bool RAG = false, bool WIN = false>
 __global__ void wave_prep_kernel(const TIn* __restrict__ wave, void* __restrict__ hi_, void* __restrict__ lo_,
-                                 int L, int pad, int ld_pad, int ld_wave, const int32_t* __restrict__ valid) {
+                                 int L, int pad, int ld_pad, int ld_wave, const int32_t* __restrict__ valid,
+                                 const long long* __restrict__ offsets = nullptr, long long rec_len = 0) {
   // 4 consecutive output samples per thread (ld_pad % 8 == 0): 8-byte bf16 / 16-byte fp32 stores
   const int b = blockIdx.y;
   const int j0 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (j0 >= ld_pad) return;
   if (RAG) L = min(max(__ldg(valid + b), pad + 1), L);
+  const TIn* win = wave;
+  if (WIN) {
+    L = (int)min((long long)L, rec_len);
+    win = wave + min(max(__ldg(offsets + b), 0LL), rec_len - L);
+  }
   float v[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -40,7 +49,7 @@ __global__ void wave_prep_kernel(const TIn* __restrict__ wave, void* __restrict_
       int s = j - pad;
       if (s < 0) s = -s;                       // reflect (edge sample not repeated)
       if (s >= L) s = 2 * (L - 1) - s;
-      v[i] = load_sample(wave + (size_t)b * (RAG ? ld_wave : L) + s);
+      v[i] = load_sample(WIN ? win + s : wave + (size_t)b * (RAG ? ld_wave : L) + s);
     }
   }
   const size_t o = (size_t)b * ld_pad + j0;
@@ -795,7 +804,8 @@ using namespace acx;
 
 template <typename TIn>
 static int wave_prep_launch(const TIn* wave, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
-                            int ld_wave, const int32_t* valid, void* stream) {
+                            int ld_wave, const int32_t* valid, void* stream, const long long* offsets = nullptr,
+                            long long rec_len = 0) {
   ACX_CHECK(wave && hi && B > 0 && L > 0, ACX_ERR_ARG, "wave_prep: null pointer or empty batch");
   ACX_CHECK(ld_wave >= L, ACX_ERR_ARG, "wave_prep: row pitch %d < L=%d", ld_wave, L);
   ACX_CHECK(L > n_fft / 2, ACX_ERR_ARG, "wave_prep: reflect padding needs L > n_fft/2 (L=%d)", L);
@@ -806,7 +816,16 @@ static int wave_prep_launch(const TIn* wave, void* hi, void* lo, int B, int L, i
   dim3 grid(ceil_div(ld_pad, 1024), B);
   ACX_CHECK(act_dtype != ACX_BF16 || lo != nullptr, ACX_ERR_ARG, "wave_prep: lo buffer required for bf16 split");
   constexpr bool kRagged = std::is_same<TIn, float>::value;     // ragged batches are fp32 waveforms only
-  if (kRagged && valid && act_dtype == ACX_BF16)
+  const int pad = n_fft / 2;
+  if (offsets && valid && act_dtype == ACX_BF16)                // windows of one recording (fp32 or int16)
+    wave_prep_kernel<true, TIn, true, true><<<grid, 256, 0, st>>>(wave, hi, lo, L, pad, ld_pad, L, valid, offsets, rec_len);
+  else if (offsets && valid)
+    wave_prep_kernel<false, TIn, true, true><<<grid, 256, 0, st>>>(wave, hi, lo, L, pad, ld_pad, L, valid, offsets, rec_len);
+  else if (offsets && act_dtype == ACX_BF16)
+    wave_prep_kernel<true, TIn, false, true><<<grid, 256, 0, st>>>(wave, hi, lo, L, pad, ld_pad, L, nullptr, offsets, rec_len);
+  else if (offsets)
+    wave_prep_kernel<false, TIn, false, true><<<grid, 256, 0, st>>>(wave, hi, lo, L, pad, ld_pad, L, nullptr, offsets, rec_len);
+  else if (kRagged && valid && act_dtype == ACX_BF16)
     wave_prep_kernel<true, TIn, kRagged><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, valid);
   else if (kRagged && valid)
     wave_prep_kernel<false, TIn, kRagged><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, valid);
@@ -816,6 +835,16 @@ static int wave_prep_launch(const TIn* wave, void* hi, void* lo, int B, int L, i
     wave_prep_kernel<false, TIn><<<grid, 256, 0, st>>>(wave, hi, lo, L, n_fft / 2, ld_pad, ld_wave, nullptr);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
+}
+
+template <typename TIn>
+static int wave_prep_windows(const TIn* rec, long long rec_len, const long long* offsets, const int32_t* valid, void* hi,
+                             void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype, void* stream) {
+  ACX_CHECK(rec && offsets, ACX_ERR_ARG, "wave_prep_windows: null recording or offsets");
+  ACX_CHECK(rec_len >= n_fft / 2 + 1, ACX_ERR_ARG, "wave_prep_windows: rec_len=%lld must be > n_fft/2 (reflect padding)",
+            rec_len);
+  ACX_CHECK(B >= 1, ACX_ERR_ARG, "wave_prep_windows: empty batch B=%d", B);
+  return wave_prep_launch<TIn>(rec, hi, lo, B, L, n_fft, ld_pad, act_dtype, L, valid, stream, offsets, rec_len);
 }
 
 extern "C" {
@@ -834,6 +863,16 @@ int acx_wave_prep_ragged(const float* wave, void* hi, void* lo, int B, int L, in
 int acx_wave_prep_pcm16(const int16_t* pcm, void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype,
                         void* stream) {
   return wave_prep_launch<int16_t>(pcm, hi, lo, B, L, n_fft, ld_pad, act_dtype, L, nullptr, stream);
+}
+
+int acx_wave_prep_windows(const float* rec, long long rec_len, const long long* offsets, const int32_t* valid, void* hi,
+                          void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype, void* stream) {
+  return wave_prep_windows<float>(rec, rec_len, offsets, valid, hi, lo, B, L, n_fft, ld_pad, act_dtype, stream);
+}
+
+int acx_wave_prep_pcm16_windows(const int16_t* rec, long long rec_len, const long long* offsets, const int32_t* valid,
+                                void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype, void* stream) {
+  return wave_prep_windows<int16_t>(rec, rec_len, offsets, valid, hi, lo, B, L, n_fft, ld_pad, act_dtype, stream);
 }
 
 int acx_power_mel_log(const float* spec, int ld_spec, int n_bins, const float* melT, const int32_t* mel_lo,

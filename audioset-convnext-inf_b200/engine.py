@@ -319,6 +319,7 @@ class Engine:
         ws["probs"] = torch.empty(n, N_CLASSES, device=dev, dtype=torch.float32)
         ws["frame"] = torch.empty(n, DIMS[3], hs[3], 7, device=dev, dtype=torch.float32)
         ws["valid"] = torch.empty(6 * n, device=dev, dtype=torch.int32)     # ragged batches: ragged_table of the chunk
+        ws["offsets"] = torch.empty(n, device=dev, dtype=torch.int64)       # windows: each row's first sample in the recording
         ws["graphs"] = {}         # (n, trunk, head, frame) -> (CUDAGraph, launches per replay); dies with the buffers
         ws["uses"] = {}
         while len(self._ws) >= max(1, self.max_workspaces):
@@ -413,24 +414,28 @@ class Engine:
         return "hbm", 0.0
 
     # ---- stages (each is one libacx call) ----------------------------------------------------------
-    def _wave_prep(self, wave, ws, n, L, st, rv=None):
-        """Reads the caller's tensor -> stays outside any captured graph.  rv: the ragged chunk's bound pointers or None."""
+    def _wave_prep(self, wave, ws, n, L, st, rv=None, windows=False):
+        """Reads the caller's tensor -> stays outside any captured graph.  rv: the ragged chunk's bound pointers or None.
+        windows: `wave` is one 1-D recording and row b is its window at ws["offsets"][b] (the acx_*_windows forms)."""
         ld_pad = ws["ld_pad"]
         fn = "acx_wave_prep_pcm16" if wave.dtype == torch.int16 else "acx_wave_prep"
         if self.frontend == "folded":
             fn = "acx_frame_fold_pcm16" if wave.dtype == torch.int16 else "acx_frame_fold"
-            args = (wave.data_ptr(), ws["f_hi"].data_ptr(), ws["f_lo"].data_ptr(), n, L, ws["T"], N_FFT, HOP)
+            args = (ws["f_hi"].data_ptr(), ws["f_lo"].data_ptr(), n, L, ws["T"], N_FFT, HOP)
             tag = "frame_fold"
         elif self.frontend == "fused":
-            args = (wave.data_ptr(), ws["wav_hi"].data_ptr(), ws["wav_lo"].data_ptr(), n, L, N_FFT, ld_pad, N.ACX_BF16)
+            args = (ws["wav_hi"].data_ptr(), ws["wav_lo"].data_ptr(), n, L, N_FFT, ld_pad, N.ACX_BF16)
             tag = "wave_prep"
         else:
-            args = (wave.data_ptr(), ws["wav_pad"].data_ptr(), 0, n, L, N_FFT, ld_pad, N.ACX_F32)
+            args = (ws["wav_pad"].data_ptr(), 0, n, L, N_FFT, ld_pad, N.ACX_F32)
             tag = "wave_prep"
-        if rv:
-            self._call(tag, fn + "_ragged", *args, L, rv[0], st)       # rows of the (n, L) chunk are L samples apart
+        if windows:
+            self._call(tag, fn + "_windows", wave.data_ptr(), wave.numel(), ws["offsets"].data_ptr(), rv[0] if rv else 0,
+                       *args, st)
+        elif rv:
+            self._call(tag, fn + "_ragged", wave.data_ptr(), *args, L, rv[0], st)   # rows of the (n, L) chunk are L samples apart
         else:
-            self._call(tag, fn, *args, st)
+            self._call(tag, fn, wave.data_ptr(), *args, st)
 
     def _frontend(self, ws, n, L, st):
         w = self.w
@@ -637,26 +642,81 @@ class Engine:
             for b0 in range(0, B, self.chunk):
                 n = min(self.chunk, B - b0)
                 ws = self._workspace(min(self.chunk, B), L)
-                rv = None
-                if ragged:
-                    # a fresh pinned host tensor per chunk: the caching host allocator keeps it until the copy has run
-                    tab = ragged_table(lengths[b0:b0 + n]).pin_memory()
-                    ws["valid"][:6 * n].view(6, n).copy_(tab, non_blocking=True)
-                    rv = self._ragged_ptrs(ws, n, True)
-                self._wave_prep(wave[b0:b0 + n], ws, n, L, st, rv)
-                trunk = need_head or "frame" in want
-                key = (n, L, trunk, need_head, "frame" in want, ragged)
-                g = ws["graphs"].get(key) if (self.use_graph and self._prof is None) else None
-                if g is None and self.use_graph and self._prof is None:
-                    ws["uses"][key] = ws["uses"].get(key, 0) + 1
-                    if ws["uses"][key] >= self.graph_after:      # a shape seen once (odd length, ragged tail) runs eagerly
-                        g = ws["graphs"][key] = self._capture(ws, n, L, *key[2:])
-                if g is not None:
-                    g[0].replay()
-                    self.launches += g[1]
-                else:
-                    self._body(ws, n, L, st, *key[2:])
+                self._run_chunk(ws, n, L, st, want, lengths[b0:b0 + n] if ragged else None,
+                                lambda rv: self._wave_prep(wave[b0:b0 + n], ws, n, L, st, rv))
                 for name in ("logmel", "scene", "logits", "probs", "frame"):
                     if name in out:
                         out[name][b0:b0 + n].copy_(ws[name][:n])
+        return out
+
+    def _run_chunk(self, ws, n, L, st, want, lengths, prep):
+        """One chunk of n clips on workspace ws (canvas L), the chunk loop body of run and run_windows: the ragged bound
+        table when `lengths` (n ints) is given, then prep(rv) -- the prep launch, outside any graph because it reads the
+        caller's buffer -- then everything after it, replayed from a CUDA graph or run eagerly.  Results stay in ws."""
+        ragged = lengths is not None
+        rv = None
+        if ragged:
+            # a fresh pinned host tensor per chunk: the caching host allocator keeps it until the copy has run
+            tab = ragged_table(lengths).pin_memory()
+            ws["valid"][:6 * n].view(6, n).copy_(tab, non_blocking=True)
+            rv = self._ragged_ptrs(ws, n, True)
+        prep(rv)
+        need_head = "logits" in want or "scene" in want
+        trunk = need_head or "frame" in want
+        key = (n, L, trunk, need_head, "frame" in want, ragged)
+        g = ws["graphs"].get(key) if (self.use_graph and self._prof is None) else None
+        if g is None and self.use_graph and self._prof is None:
+            ws["uses"][key] = ws["uses"].get(key, 0) + 1
+            if ws["uses"][key] >= self.graph_after:      # a shape seen once (odd length, ragged tail) runs eagerly
+                g = ws["graphs"][key] = self._capture(ws, n, L, *key[2:])
+        if g is not None:
+            g[0].replay()
+            self.launches += g[1]
+        else:
+            self._body(ws, n, L, st, *key[2:])
+
+    def run_windows(self, rec, plan, want=("logits",)):
+        """Windows of one recording buffer, read in place.  rec: 1-D contiguous float32 or int16 PCM CUDA tensor (the
+        recordings laid end to end); plan: windows.WindowPlan, whose `offset`s index rec.  Row i of every output equals a
+        run of rec[offset_i : offset_i + length_i] alone.  Full-length windows run non-ragged on a canvas of plan.window,
+        so they share run()'s workspace and CUDA graphs for that shape; own-length windows run ragged.  frame (N, 768,
+        h3(plan.window), 7) has zeros past each window's own h3.  The plan is checked against rec before any launch."""
+        from .windows import window_batches
+        assert rec.is_cuda and rec.dim() == 1 and rec.is_contiguous()
+        assert rec.dtype in (torch.float32, torch.int16), "recording must be float32 or int16 PCM"
+        if "logmel" in want:
+            raise ValueError("windows have no log-mel output")
+        Nw, W = plan.length.numel(), int(plan.window)
+        if Nw and not (int(plan.length.min()) >= MIN_RAGGED_LEN and int(plan.length.max()) <= W
+                       and int(plan.offset.min()) >= 0 and int((plan.offset + plan.length).max()) <= rec.numel()):
+            raise ValueError(f"window plan does not fit a recording buffer of {rec.numel()} samples "
+                             f"(lengths must lie in [{MIN_RAGGED_LEN}, {W}] and every window inside the buffer)")
+        batches = window_batches(plan, self.chunk)
+        rows = {r: min(self.chunk, sum(len(idx) for _, ls, idx in batches if (ls is not None) == r)) for r in (False, True)}
+        h3 = out_time_dims(W)[1][3]
+        dev = self.device
+        f32 = dict(device=dev, dtype=torch.float32)
+        out = {}
+        with torch.cuda.device(dev):
+            st = torch.cuda.current_stream(dev).cuda_stream
+            if "logits" in want or "scene" in want:
+                out["scene"] = torch.empty(Nw, DIMS[3], **f32)
+                out["logits"] = torch.empty(Nw, N_CLASSES, **f32)
+                out["probs"] = torch.empty(Nw, N_CLASSES, **f32)
+            if "frame" in want:
+                out["frame"] = torch.empty(Nw, DIMS[3], h3, 7, **f32)
+            for L, lengths, idx in batches:
+                n = len(idx)
+                ws = self._workspace(rows[lengths is not None], L)
+                ws["offsets"][:n].copy_(plan.offset[idx].pin_memory(), non_blocking=True)
+                self._run_chunk(ws, n, L, st, want, lengths, lambda rv: self._wave_prep(rec, ws, n, L, st, rv, windows=True))
+                dst = torch.tensor(idx, dtype=torch.int64).to(dev, non_blocking=True)
+                for name in ("scene", "logits", "probs"):
+                    if name in out:
+                        out[name].index_copy_(0, dst, ws[name][:n])
+                if "frame" in out:
+                    fr = ws["frame"][:n, :, :h3]               # a ragged canvas may have more rows than the window ...
+                    if fr.shape[2] < h3:                       # ... or fewer: those are past every window's own h3
+                        fr = torch.nn.functional.pad(fr, (0, 0, 0, h3 - fr.shape[2]))
+                    out["frame"].index_copy_(0, dst, fr)
         return out

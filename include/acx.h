@@ -235,6 +235,29 @@ ACX_API int acx_head_ragged(const void* x, const float* ln_w, const float* ln_b,
 ACX_API int acx_nhwc_to_nchw_f32_ragged(const void* x, float* out, int B, int H, int W, int C, int act_dtype,
                                         const int32_t* valid, void* stream);
 
+/* ---- windows of a long recording: prep kernels that read each window in place --------------------------------------
+ * Row b of the batch is the window that starts offsets[b] samples into ONE recording `rec` of rec_len samples (fp32, or
+ * int16 PCM converted x / 32767. like acx_wave_prep_pcm16).  Windows may overlap and offsets are 64-bit, so a recording
+ * may be longer than 2^31 samples.  Every size argument is the CANVAS size, as for the ragged entry points; the outputs
+ * are exactly those of acx_wave_prep / acx_frame_fold on the batch of copied windows, so every later kernel is unchanged.
+ *   valid == NULL   every window has L samples;
+ *   valid != NULL   row 0 of the chunk's ragged bound table (B int32 entries): window b has its own L_b samples and is
+ *                   reflected at its own end, as in acx_wave_prep_ragged; the later kernels then run their _ragged forms.
+ * A window never reads a sample outside [offsets[b], offsets[b] + L_b).  Each length is clamped to rec_len (and, with
+ * valid, to [n_fft/2 + 1, L]), each offset to [0, rec_len - length], so no value can make the kernels read outside the
+ * recording; whether the values are right is for the caller to check.  A null rec or offsets, rec_len <= n_fft/2 or
+ * B < 1 returns ACX_ERR_ARG. */
+ACX_API int acx_wave_prep_windows(const float* rec, long long rec_len, const long long* offsets, const int32_t* valid,
+                                  void* hi, void* lo, int B, int L, int n_fft, int ld_pad, int act_dtype, void* stream);
+ACX_API int acx_wave_prep_pcm16_windows(const int16_t* rec, long long rec_len, const long long* offsets,
+                                        const int32_t* valid, void* hi, void* lo, int B, int L, int n_fft, int ld_pad,
+                                        int act_dtype, void* stream);
+ACX_API int acx_frame_fold_windows(const float* rec, long long rec_len, const long long* offsets, const int32_t* valid,
+                                   void* f_hi, void* f_lo, int B, int L, int T, int n_fft, int hop, void* stream);
+ACX_API int acx_frame_fold_pcm16_windows(const int16_t* rec, long long rec_len, const long long* offsets,
+                                         const int32_t* valid, void* f_hi, void* f_lo, int B, int L, int T, int n_fft,
+                                         int hop, void* stream);
+
 /* ---- next row (f4): demo preprocessing, reference demo_convnext.py:52-67 --------------------- */
 /* torchaudio.functional.resample (sinc_interp_hann polyphase FIR, demo_convnext.py:53-59) fused with the demo's
  * constant pad / crop to a fixed clip length (demo_convnext.py:61-67):
