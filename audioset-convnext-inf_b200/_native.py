@@ -11,6 +11,7 @@ _lock = threading.Lock()
 _lib = None
 
 ACX_BF16, ACX_F32 = 0, 1
+ACX_ERR_ARG, ACX_ERR_UNSUPPORTED = 1, 3
 EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_SCALE_RESID = 0, 1, 2
 
 _vp, _i, _ll = ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong
@@ -66,6 +67,10 @@ SIGNATURES = {
     "acx_wave_prep_pcm16_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "acx_frame_fold_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "acx_frame_fold_pcm16_windows": [_vp, _ll, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
+    # any sample rate: segments packed in one buffer, (S, 4) int64 table and per-segment first tiles on the device
+    "acx_resample_segments_tiling": [_i, _i, _i, _vp, _vp],
+    "acx_resample_segments": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
+    "acx_resample_segments_pcm16": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
 }
 
 

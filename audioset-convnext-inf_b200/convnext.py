@@ -19,7 +19,7 @@ import os
 import torch
 import torch.nn as nn
 
-from . import _native
+from . import _native, preprocess
 from .engine import DEPTHS, DIMS, Engine, out_time_dims
 from .frontend_consts import slaney_mel_filterbank, windowed_dft
 from .windows import plan_windows
@@ -236,7 +236,8 @@ class ConvNeXt(nn.Module):
             res["frame_lengths"] = torch.tensor(h3, dtype=torch.int64).to(x.device)
         return res
 
-    def forward_windows(self, recordings, window_samples=320000, hop_samples=32000, frame_embeddings=False):
+    def forward_windows(self, recordings, window_samples=320000, hop_samples=32000, frame_embeddings=False,
+                        sample_rate=32000):
         """Tag long recordings window by window, each window as a clip of its own (the model's training condition).
 
         recordings: one 1-D tensor or a sequence of 1-D tensors of any lengths, on the host or the device; float32, int16
@@ -251,34 +252,29 @@ class ConvNeXt(nn.Module):
         frame_embeddings=True also "frame_embeddings" (N, 768, T', 7), T' the frame count of a full window, zero past each
         window's own count, which "frame_lengths" gives.  Row i equals
         forward_all(recordings[recording_i][start_i : start_i + length_i][None]) bit for bit, and a window never reads a
-        sample outside itself.  Every argument is checked before anything is launched."""
+        sample outside itself.  Every argument is checked before anything is launched.
+
+        sample_rate: the recordings' rate in Hz, a positive int or one per recording.  Recordings not at 32 kHz are first
+        resampled on the GPU (preprocess.resample: torchaudio's filter, exact length ceil(32000 * n / rate)) into one
+        float32 buffer, and the windows are planned on the resampled lengths: window_samples, hop_samples and the returned
+        "start" / "length" are then in 32 kHz samples of the RESAMPLED recording (seconds = start / 32000), and row i
+        equals forward_windows of the resampled recordings passed at 32 kHz, bit for bit.  A recording whose resampled
+        length is under 7360 samples raises ValueError.  With every rate at 32 kHz (the default) nothing is resampled and
+        int16 recordings stay int16."""
         self._check_inference(None)
-        if isinstance(recordings, torch.Tensor):
-            recordings = [recordings]
-        recs = [r if isinstance(r, torch.Tensor) else torch.as_tensor(r) for r in recordings]
-        for i, r in enumerate(recs):
-            if r.dim() != 1:
-                raise ValueError(f"recording {i} must be 1-D (samples), got shape {tuple(r.shape)}")
-            if not (r.dtype == torch.int16 or r.is_floating_point()):
-                raise ValueError(f"recording {i} has dtype {r.dtype}: expected a float dtype or int16 PCM")
-        plan = plan_windows([r.numel() for r in recs], window_samples, hop_samples)
+        recs = preprocess.check_waveforms(recordings, "recording")
+        rates = preprocess.sample_rates(sample_rate, len(recs))
+        resample = any(r != preprocess.SAMPLE_RATE for r in rates)
+        lengths = [preprocess.resampled_length(r.numel(), sr) for r, sr in zip(recs, rates)]
+        plan = plan_windows(lengths, window_samples, hop_samples)
         eng = self._get_engine()
         dev = eng.device
-        pcm = bool(recs) and all(r.dtype == torch.int16 for r in recs)
-        if len(recs) == 1 and recs[0].device == dev and recs[0].dtype in (torch.float32, torch.int16) and recs[0].is_contiguous():
-            buf = recs[0].detach()
+        if resample:
+            buf = preprocess.resample_packed(recs, rates, preprocess.SAMPLE_RATE, dev)[0]
+            pcm = False
         else:
-            buf = torch.empty(sum(r.numel() for r in recs),
-                              dtype=torch.int16 if pcm else torch.float32, device=dev)
-            base = 0
-            for r in recs:
-                dst = buf[base:base + r.numel()]
-                if r.dtype == torch.int16 and not pcm:
-                    # the prep kernels' conversion, a correctly rounded fp32 division (not a reciprocal multiply)
-                    torch.div(r.detach().to(dev).to(torch.float32), torch.tensor(32767.0, device=dev), out=dst)
-                else:
-                    dst.copy_(r.detach())
-                base += r.numel()
+            buf = preprocess.pack_waveforms(recs, dev)
+            pcm = buf.dtype == torch.int16
         if not pcm:
             self._check_amplitude(eng, buf)
         want = ("logits", "scene", "frame") if frame_embeddings else ("logits", "scene")

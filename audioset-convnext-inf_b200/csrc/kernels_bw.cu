@@ -740,6 +740,107 @@ __global__ void __launch_bounds__(256)
   out[(size_t)blockIdx.y * ld_out + i] = acc;
 }
 
+// ---- segmented resampler: many recordings of any length packed in one buffer, 64-bit indices ----------------------
+// Segment s is (in_off, in_len, out_off, out_len) int64: output j of the segment is what resample_fit_kernel computes for
+// a row of in_len samples (frame f = j / newf, phase p = j % newf, the same fmaf chain over k = 0..K-1), with the input
+// zero outside [0, in_len) of the SEGMENT.  Each entry is clamped to x_len / out_len, so no table value can make the
+// kernel read or write outside its buffers.
+//
+// A block computes one tile: RS_THREADS / 32 warps, lanes = 32 consecutive frames, each thread RS_R consecutive phases
+// (one float4 of taps per k, reused by its RS_R outputs; every output keeps its own sequential k order).  The tile's
+// P phases' taps (K x P) and its input span ((F-1) * orig + K samples, converted to fp32 and zero-filled outside the
+// segment) are staged in shared memory once, so the tap table is read from global memory once per block instead of
+// once per output.  Tiles of all segments form one 1-D grid: tile_start[s] is segment s's first tile (a host-built
+// prefix over ceil(frames / F) * G tiles per segment), which the block finds by binary search.  So one launch spreads
+// a single long segment over every SM and also serves thousands of short clips.
+constexpr int RS_R = 4, RS_WARPS = 8, RS_THREADS = 32 * RS_WARPS;
+constexpr int RS_MAX_SMEM = 227 * 1024;
+
+struct ResampleTiling {
+  int P, F, G;          // phases and frames per tile, phase groups per frame tile
+  long long smem;       // dynamic shared memory bytes
+};
+
+// Phase warps WP = the smallest power of two >= ceil(newf / RS_R), at most RS_WARPS; the other warps take more frames.
+static inline ResampleTiling resample_tiling(int orig, int newf, int width) {
+  const int quads = (newf + RS_R - 1) / RS_R;
+  int wp = 1;
+  while (wp < quads && wp < RS_WARPS) wp *= 2;
+  ResampleTiling t;
+  t.P = wp * RS_R;
+  t.F = 32 * (RS_WARPS / wp);
+  t.G = (newf + t.P - 1) / t.P;
+  const long long K = 2LL * width + orig;
+  t.smem = (K * t.P + (long long)(t.F - 1) * orig + K) * (long long)sizeof(float);
+  return t;
+}
+
+template <typename TIn>
+__global__ void __launch_bounds__(RS_THREADS)
+    resample_segments_kernel(const TIn* __restrict__ x, long long x_len, const long long* __restrict__ seg,
+                             const long long* __restrict__ tile_start, int S, const float* __restrict__ taps, int orig,
+                             int newf, int width, int P, int F, int G, float* __restrict__ out, long long out_len) {
+  extern __shared__ float4 rs_smem[];
+  const int K = 2 * width + orig;
+  float* s_taps = reinterpret_cast<float*>(rs_smem);      // [K][P]
+  float* s_x = s_taps + (size_t)K * P;                     // [(F-1) * orig + K]
+  const long long tile = blockIdx.x;
+  int lo = 0, hi = S - 1;                                  // last segment whose first tile is <= this one
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(tile_start + mid) <= tile) lo = mid; else hi = mid - 1;
+  }
+  const long long local = tile - __ldg(tile_start + lo);
+  if (local < 0) return;
+  const long long* e = seg + 4 * (size_t)lo;
+  const long long in_off = min(max(__ldg(e), 0LL), x_len);
+  const long long in_len = min(max(__ldg(e + 1), 0LL), x_len - in_off);
+  const long long out_off = min(max(__ldg(e + 2), 0LL), out_len);
+  const long long n_out = min(max(__ldg(e + 3), 0LL), out_len - out_off);
+  const long long ft = local / G;
+  const int p0 = (int)(local - ft * G) * P;
+  const long long f0 = ft * F;
+  if (f0 * newf >= n_out) return;                          // whole block: no barrier is skipped by part of it
+
+  for (int i = threadIdx.x; i < K * P; i += RS_THREADS) {
+    const int k = i / P, p = p0 + (i - k * P);
+    s_taps[i] = p < newf ? __ldg(taps + (size_t)k * newf + p) : 0.f;
+  }
+  const TIn* xs = x + in_off;
+  const long long i0 = f0 * orig - width;
+  const int span = (F - 1) * orig + K;
+  for (int i = threadIdx.x; i < span; i += RS_THREADS) {
+    const long long idx = i0 + i;
+    s_x[i] = (idx >= 0 && idx < in_len) ? load_sample(xs + idx) : 0.f;
+  }
+  __syncthreads();
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int wp = P / RS_R;
+  const int pl = (warp % wp) * RS_R;                       // first of this thread's RS_R phases in the tile
+  const int fl = (warp / wp) * 32 + lane;                  // this thread's frame in the tile
+  const float* xv = s_x + fl * orig;
+  const float4* tv = reinterpret_cast<const float4*>(s_taps + pl);
+  const int tstride = P / RS_R;
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+#pragma unroll 4
+  for (int k = 0; k < K; ++k) {
+    const float v = xv[k];
+    const float4 t = tv[k * tstride];
+    a0 = fmaf(t.x, v, a0);
+    a1 = fmaf(t.y, v, a1);
+    a2 = fmaf(t.z, v, a2);
+    a3 = fmaf(t.w, v, a3);
+  }
+  const int p = p0 + pl;
+  const long long j = (f0 + fl) * newf + p;
+  float* o = out + out_off;
+  if (p < newf && j < n_out) o[j] = a0;
+  if (p + 1 < newf && j + 1 < n_out) o[j + 1] = a1;
+  if (p + 2 < newf && j + 2 < n_out) o[j + 2] = a2;
+  if (p + 3 < newf && j + 3 < n_out) o[j + 3] = a3;
+}
+
 // ---- launch helpers ---------------------------------------------------------------------------
 template <typename T, int C, int S, int PF = 2, bool RAG = false>
 static int launch_dwconv(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
@@ -1075,6 +1176,64 @@ int acx_resample_fit(const float* x, int ld_in, const float* taps, float* out, i
                                                                                 newf, width, n_out, target);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
+}
+
+}  // extern "C"
+
+static int resample_tiling_checked(int orig, int newf, int width, ResampleTiling* t) {
+  ACX_CHECK(orig > 0 && newf > 0 && width > 0, ACX_ERR_ARG, "resample_segments: bad rates %d -> %d (width %d)", orig,
+            newf, width);
+  *t = resample_tiling(orig, newf, width);
+  ACX_CHECK(t->smem <= RS_MAX_SMEM, ACX_ERR_UNSUPPORTED,
+            "resample_segments: rate ratio %d/%d (K=%lld taps) needs %lld bytes of shared memory per tile, over %d",
+            orig, newf, 2LL * width + orig, t->smem, RS_MAX_SMEM);
+  return ACX_OK;
+}
+
+template <typename TIn>
+static int resample_segments_impl(const TIn* x, long long x_len, const long long* seg, int S, const long long* tile_start,
+                                  long long n_tiles, const float* taps, int orig, int newf, int width, float* out,
+                                  long long out_len, void* stream) {
+  ACX_CHECK(x && seg && tile_start && taps && out, ACX_ERR_ARG, "resample_segments: null pointer");
+  ACX_CHECK(S >= 1 && x_len >= 1 && out_len >= 1, ACX_ERR_ARG,
+            "resample_segments: bad sizes S=%d x_len=%lld out_len=%lld", S, x_len, out_len);
+  ACX_CHECK(n_tiles >= 1 && n_tiles <= 0x7fffffffLL, ACX_ERR_ARG, "resample_segments: n_tiles=%lld out of [1, 2^31)",
+            n_tiles);
+  ResampleTiling t;
+  const int rc = resample_tiling_checked(orig, newf, width, &t);
+  if (rc != ACX_OK) return rc;
+  auto kern = resample_segments_kernel<TIn>;
+  ACX_SET_MAX_SMEM(kern, RS_MAX_SMEM);
+  kern<<<(unsigned)n_tiles, RS_THREADS, (size_t)t.smem, reinterpret_cast<cudaStream_t>(stream)>>>(
+      x, x_len, seg, tile_start, S, taps, orig, newf, width, t.P, t.F, t.G, out, out_len);
+  ACX_CUDA(cudaGetLastError());
+  return ACX_OK;
+}
+
+extern "C" {
+
+int acx_resample_segments_tiling(int orig, int newf, int width, int* tile_frames_host, int* phase_groups_host) {
+  ACX_CHECK(tile_frames_host && phase_groups_host, ACX_ERR_ARG, "resample_segments_tiling: null pointer");
+  ResampleTiling t;
+  const int rc = resample_tiling_checked(orig, newf, width, &t);
+  if (rc != ACX_OK) return rc;
+  *tile_frames_host = t.F;
+  *phase_groups_host = t.G;
+  return ACX_OK;
+}
+
+int acx_resample_segments(const float* x, long long x_len, const long long* seg, int S, const long long* tile_start,
+                          long long n_tiles, const float* taps, int orig, int newf, int width, float* out,
+                          long long out_len, void* stream) {
+  return resample_segments_impl<float>(x, x_len, seg, S, tile_start, n_tiles, taps, orig, newf, width, out, out_len,
+                                       stream);
+}
+
+int acx_resample_segments_pcm16(const int16_t* x, long long x_len, const long long* seg, int S,
+                                const long long* tile_start, long long n_tiles, const float* taps, int orig, int newf,
+                                int width, float* out, long long out_len, void* stream) {
+  return resample_segments_impl<int16_t>(x, x_len, seg, S, tile_start, n_tiles, taps, orig, newf, width, out, out_len,
+                                         stream);
 }
 
 }  // extern "C"

@@ -268,6 +268,32 @@ ACX_API int acx_frame_fold_pcm16_windows(const int16_t* rec, long long rec_len, 
 ACX_API int acx_resample_fit(const float* x, int ld_in, const float* taps, float* out, int ld_out, int B, int L_in,
                      int orig, int newf, int width, int n_out, void* stream);
 
+/* ---- any sample rate: recordings of any lengths resampled in one launch per rate ---------------------------------------
+ * x holds S segments packed in one buffer of x_len samples (fp32, or int16 PCM converted x / 32767. with a correctly
+ * rounded division, like acx_wave_prep_pcm16); out is one fp32 buffer of out_len samples.  seg is a DEVICE (S, 4) int64
+ * table, row s = (in_off, in_len, out_off, out_len) in samples of x and out.  Output j < out_len of segment s is
+ *   sum_{k<K} taps[k*newf + p] * v(f*orig - width + k),   f = j / newf, p = j % newf,
+ * accumulated with fmaf in k order, where v(i) = x[in_off + i] for 0 <= i < in_len and ZERO outside the segment: a
+ * segment never reads its neighbours' samples.  So each segment equals acx_resample_fit of that segment alone with
+ * n_out = ceil(newf * in_len / orig), bit for bit, and out_len is normally that ceil.  Indices are 64-bit, so a segment
+ * may exceed 2^31 samples.  Each entry is clamped to x_len / out_len, so no table value makes the kernel read or write
+ * outside its buffers; whether the values are right is for the caller to check.
+ * Work distribution: one block per tile of tile_frames frames x (taps' phases / phase_groups) phases of one segment.
+ * Segment s owns ceil(ceil(out_len_s / newf) / tile_frames) * phase_groups tiles, starting at tile_start[s] (DEVICE (S,)
+ * int64, non-decreasing, tile_start[0] = 0); n_tiles is the total.  acx_resample_segments_tiling gives tile_frames and
+ * phase_groups for a rate pair (host call, no launch), and returns ACX_ERR_UNSUPPORTED when the tile's taps and input span
+ * exceed shared memory (about 58 000 floats: K * 4 * phase warps + (tile_frames - 1) * orig + K; 8 to 192 kHz -> 32 kHz
+ * and 11.025 / 22.05 / 44.1 / 88.2 kHz all fit).
+ * A null pointer, S < 1, x_len < 1, out_len < 1, n_tiles outside [1, 2^31) or a rate or width <= 0 returns ACX_ERR_ARG
+ * before any launch. */
+ACX_API int acx_resample_segments_tiling(int orig, int newf, int width, int* tile_frames_host, int* phase_groups_host);
+ACX_API int acx_resample_segments(const float* x, long long x_len, const long long* seg, int S,
+                                  const long long* tile_start, long long n_tiles, const float* taps, int orig, int newf,
+                                  int width, float* out, long long out_len, void* stream);
+ACX_API int acx_resample_segments_pcm16(const int16_t* x, long long x_len, const long long* seg, int S,
+                                        const long long* tile_start, long long n_tiles, const float* taps, int orig,
+                                        int newf, int width, float* out, long long out_len, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
