@@ -71,6 +71,11 @@ SIGNATURES = {
     "acx_resample_segments_tiling": [_i, _i, _i, _vp, _vp],
     "acx_resample_segments": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
     "acx_resample_segments_pcm16": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
+    # live streams: packed chunks scattered into per-stream rings ((S, 6) int64 table), and the resampler reading and
+    # writing rings ((S, 8) int64 table; otherwise the arguments of acx_resample_segments)
+    "acx_stream_append": [_vp, _ll, _vp, _i, _vp, _ll, _vp],
+    "acx_stream_append_pcm16": [_vp, _ll, _vp, _i, _vp, _ll, _vp],
+    "acx_resample_stream": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
 }
 
 

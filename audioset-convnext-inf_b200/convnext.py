@@ -287,6 +287,34 @@ class ConvNeXt(nn.Module):
             res["frame_lengths"] = torch.tensor(h3, dtype=torch.int64).to(dev)
         return res
 
+    def open_stream(self, n_streams=1, window_samples=320000, hop_samples=32000, sample_rate=32000,
+                    frame_embeddings=False, piece_seconds=10):
+        """Tag `n_streams` live audio streams window by window as their samples arrive; returns a stream.StreamTagger.
+
+        s.push(chunks) appends new samples: one 1-D tensor (n_streams == 1) or a sequence of n_streams entries, each a
+        1-D tensor or array of any length (1 sample, or far more than a window) on the host or the device; float32, int16
+        PCM (read x / 32767. with a correctly rounded division) or any other float dtype; None or empty for nothing new.
+        s.close(streams=None) ends the given streams (an index, a sequence, or None for every open one).  Both return
+        the rows of the windows that became complete during the call, in the dict forward_windows returns: rows
+        stream-major with "start" ascending ("recording" is the stream index), possibly zero rows.  A regular window
+        [k hop, k hop + window) comes back from the call in which its last sample arrives; close adds the end-aligned
+        tail window and, for a stream shorter than a window, its one own-length window (windows.plan_windows' rules).
+
+        For every stream i, its rows from all calls in order equal forward_windows(rec_i, window_samples, hop_samples,
+        frame_embeddings=frame_embeddings, sample_rate=rate_i) bit for bit, however the stream was cut into chunks;
+        rec_i is the stream's chunks concatenated (int16 chunks converted x / 32767 first).  sample_rate is an int or one
+        per stream; a stream not at 32 kHz is resampled on the GPU as it arrives, and "start" / "length" are in 32 kHz
+        samples of the resampled stream.
+
+        Device memory is allocated here and does not grow: one float32 ring per stream (window + one piece of samples,
+        plus a window-long mirror) and, for streams not at 32 kHz, an input ring of one piece plus the filter's taps.
+        A push longer than `piece_seconds` of a stream's audio is appended and tagged piece by piece within the call.
+        Work runs on the current CUDA stream.  A wrong chunk count, a chunk that is not 1-D or has a bad dtype, a push
+        to a closed stream, a bad rate, or a stream under 7360 samples (after resampling) at close raises ValueError
+        before anything is copied or launched, and leaves every stream unchanged."""
+        from .stream import StreamTagger
+        return StreamTagger(self, n_streams, window_samples, hop_samples, sample_rate, frame_embeddings, piece_seconds)
+
     def forward_logmel(self, x):
         """Normalised log-mel (B, T, 224): the tensor the reference has after bn0 (CX:298-306)."""
         eng, x = self._prep(x, None)

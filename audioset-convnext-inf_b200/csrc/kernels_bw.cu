@@ -775,7 +775,13 @@ static inline ResampleTiling resample_tiling(int orig, int newf, int width) {
   return t;
 }
 
-template <typename TIn>
+//
+// STREAM (acx_resample_stream): segment s is a live stream whose input and output are rings.  Its row is 8 int64:
+// (in_base, in_cap, in_end, f0, n_out, out_base, out_cap, out_mirror).  Input sample idx of the stream is read from
+// x[in_base + idx mod in_cap] and is zero for idx < 0 or idx >= in_end.  The block computes outputs f0 * newf + jl for
+// jl < n_out (f0 a 64-bit stream frame), each by the same fmaf chain as above, and writes output j to
+// out[out_base + j mod out_cap], and also to out[out_base + out_cap + j mod out_cap] when j mod out_cap < out_mirror.
+template <typename TIn, bool STREAM = false>
 __global__ void __launch_bounds__(RS_THREADS)
     resample_segments_kernel(const TIn* __restrict__ x, long long x_len, const long long* __restrict__ seg,
                              const long long* __restrict__ tile_start, int S, const float* __restrict__ taps, int orig,
@@ -792,11 +798,25 @@ __global__ void __launch_bounds__(RS_THREADS)
   }
   const long long local = tile - __ldg(tile_start + lo);
   if (local < 0) return;
-  const long long* e = seg + 4 * (size_t)lo;
-  const long long in_off = min(max(__ldg(e), 0LL), x_len);
-  const long long in_len = min(max(__ldg(e + 1), 0LL), x_len - in_off);
-  const long long out_off = min(max(__ldg(e + 2), 0LL), out_len);
-  const long long n_out = min(max(__ldg(e + 3), 0LL), out_len - out_off);
+  const long long* e = seg + (STREAM ? 8 : 4) * (size_t)lo;
+  long long in_off, in_len, out_off, n_out, in_cap = 0, fbase = 0, out_cap = 0, out_mirror = 0;
+  if constexpr (STREAM) {
+    in_off = min(max(__ldg(e), 0LL), x_len);
+    in_cap = min(max(__ldg(e + 1), 0LL), x_len - in_off);
+    in_len = max(__ldg(e + 2), 0LL);                       // in_end: samples of the stream received so far
+    // bounded so that every stream index below ((fbase + tile frames) * orig, fbase * newf + j) fits in int64
+    fbase = min(max(__ldg(e + 3), 0LL), (1LL << 62) / max(orig, newf));
+    n_out = max(__ldg(e + 4), 0LL);
+    out_off = min(max(__ldg(e + 5), 0LL), out_len);
+    out_cap = min(max(__ldg(e + 6), 0LL), out_len - out_off);
+    out_mirror = min(max(__ldg(e + 7), 0LL), min(out_cap, out_len - out_off - out_cap));
+    if (in_cap < 1 || out_cap < 1) return;
+  } else {
+    in_off = min(max(__ldg(e), 0LL), x_len);
+    in_len = min(max(__ldg(e + 1), 0LL), x_len - in_off);
+    out_off = min(max(__ldg(e + 2), 0LL), out_len);
+    n_out = min(max(__ldg(e + 3), 0LL), out_len - out_off);
+  }
   const long long ft = local / G;
   const int p0 = (int)(local - ft * G) * P;
   const long long f0 = ft * F;
@@ -807,11 +827,24 @@ __global__ void __launch_bounds__(RS_THREADS)
     s_taps[i] = p < newf ? __ldg(taps + (size_t)k * newf + p) : 0.f;
   }
   const TIn* xs = x + in_off;
-  const long long i0 = f0 * orig - width;
+  const long long i0 = (fbase + f0) * orig - width;
   const int span = (F - 1) * orig + K;
-  for (int i = threadIdx.x; i < span; i += RS_THREADS) {
-    const long long idx = i0 + i;
-    s_x[i] = (idx >= 0 && idx < in_len) ? load_sample(xs + idx) : 0.f;
+  if constexpr (STREAM) {
+    long long slot = i0 % in_cap;                          // the span's first ring slot, reduced once
+    if (slot < 0) slot += in_cap;
+    slot += threadIdx.x;
+    while (slot >= in_cap) slot -= in_cap;
+    for (int i = threadIdx.x; i < span; i += RS_THREADS) {
+      const long long idx = i0 + i;
+      s_x[i] = (idx >= 0 && idx < in_len) ? load_sample(xs + slot) : 0.f;
+      slot += RS_THREADS;
+      while (slot >= in_cap) slot -= in_cap;               // once when in_cap >= RS_THREADS
+    }
+  } else {
+    for (int i = threadIdx.x; i < span; i += RS_THREADS) {
+      const long long idx = i0 + i;
+      s_x[i] = (idx >= 0 && idx < in_len) ? load_sample(xs + idx) : 0.f;
+    }
   }
   __syncthreads();
 
@@ -835,10 +868,57 @@ __global__ void __launch_bounds__(RS_THREADS)
   const int p = p0 + pl;
   const long long j = (f0 + fl) * newf + p;
   float* o = out + out_off;
-  if (p < newf && j < n_out) o[j] = a0;
-  if (p + 1 < newf && j + 1 < n_out) o[j + 1] = a1;
-  if (p + 2 < newf && j + 2 < n_out) o[j + 2] = a2;
-  if (p + 3 < newf && j + 3 < n_out) o[j + 3] = a3;
+  if constexpr (STREAM) {
+    const float a[RS_R] = {a0, a1, a2, a3};
+    long long slot = (fbase * newf + j) % out_cap;        // ring slot of stream output fbase * newf + j
+#pragma unroll
+    for (int r = 0; r < RS_R; ++r) {
+      if (p + r < newf && j + r < n_out) {
+        o[slot] = a[r];
+        if (slot < out_mirror) o[out_cap + slot] = a[r];
+      }
+      if (++slot == out_cap) slot = 0;
+    }
+  } else {
+    if (p < newf && j < n_out) o[j] = a0;
+    if (p + 1 < newf && j + 1 < n_out) o[j + 1] = a1;
+    if (p + 2 < newf && j + 2 < n_out) o[j + 2] = a2;
+    if (p + 3 < newf && j + 3 < n_out) o[j + 3] = a3;
+  }
+}
+
+// ---- live streams: one push's chunks scattered into every stream's ring in one launch -------------------------------
+// tab is a DEVICE (S, 6) int64 table, row s = (src_off, n, ring_base, cap, pos, mirror): chunk s is src[src_off, src_off
+// + n), and its sample i goes to ring[ring_base + (pos + i) mod cap], and also to ring[ring_base + cap + (pos + i) mod cap]
+// when that slot is below `mirror`.  Rows are in src order (src_off non-decreasing); a thread finds its sample's row by
+// binary search, so one launch serves one long chunk or thousands of short ones.  n <= cap, mirror <= cap and the region
+// [ring_base, ring_base + cap + mirror) inside ring_len are enforced by clamping: no table value writes outside its row's
+// region of the ring.  int16 PCM is converted x / 32767 with a correctly rounded division (load_sample).
+template <typename TIn>
+__global__ void __launch_bounds__(256)
+    stream_append_kernel(const TIn* __restrict__ src, long long src_len, const long long* __restrict__ tab, int S,
+                         float* __restrict__ ring, long long ring_len) {
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= src_len) return;
+  int lo = 0, hi = S - 1;                                  // last row whose chunk starts at or before g
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(tab + 6 * (size_t)mid) <= g) lo = mid; else hi = mid - 1;
+  }
+  const long long* e = tab + 6 * (size_t)lo;
+  const long long base = min(max(__ldg(e + 2), 0LL), ring_len);
+  const long long cap = min(max(__ldg(e + 3), 0LL), ring_len - base);
+  const long long n = min(max(__ldg(e + 1), 0LL), cap);
+  const long long i = g - min(max(__ldg(e), 0LL), src_len);
+  if (i < 0 || i >= n) return;
+  const long long mirror = min(max(__ldg(e + 5), 0LL), min(cap, ring_len - base - cap));
+  long long pos = max(__ldg(e + 4), 0LL);
+  if (pos >= cap) pos %= cap;                              // the planner passes pos < cap; any other value is reduced
+  long long slot = pos + i;                                // < 2 cap: no overflow for any table value
+  if (slot >= cap) slot -= cap;
+  const float v = load_sample(src + g);
+  ring[base + slot] = v;
+  if (slot < mirror) ring[base + cap + slot] = v;
 }
 
 // ---- launch helpers ---------------------------------------------------------------------------
@@ -1190,19 +1270,19 @@ static int resample_tiling_checked(int orig, int newf, int width, ResampleTiling
   return ACX_OK;
 }
 
-template <typename TIn>
+template <typename TIn, bool STREAM = false>
 static int resample_segments_impl(const TIn* x, long long x_len, const long long* seg, int S, const long long* tile_start,
                                   long long n_tiles, const float* taps, int orig, int newf, int width, float* out,
                                   long long out_len, void* stream) {
-  ACX_CHECK(x && seg && tile_start && taps && out, ACX_ERR_ARG, "resample_segments: null pointer");
-  ACX_CHECK(S >= 1 && x_len >= 1 && out_len >= 1, ACX_ERR_ARG,
-            "resample_segments: bad sizes S=%d x_len=%lld out_len=%lld", S, x_len, out_len);
-  ACX_CHECK(n_tiles >= 1 && n_tiles <= 0x7fffffffLL, ACX_ERR_ARG, "resample_segments: n_tiles=%lld out of [1, 2^31)",
-            n_tiles);
+  const char* what = STREAM ? "resample_stream" : "resample_segments";
+  ACX_CHECK(x && seg && tile_start && taps && out, ACX_ERR_ARG, "%s: null pointer", what);
+  ACX_CHECK(S >= 1 && x_len >= 1 && out_len >= 1, ACX_ERR_ARG, "%s: bad sizes S=%d x_len=%lld out_len=%lld", what, S,
+            x_len, out_len);
+  ACX_CHECK(n_tiles >= 1 && n_tiles <= 0x7fffffffLL, ACX_ERR_ARG, "%s: n_tiles=%lld out of [1, 2^31)", what, n_tiles);
   ResampleTiling t;
   const int rc = resample_tiling_checked(orig, newf, width, &t);
   if (rc != ACX_OK) return rc;
-  auto kern = resample_segments_kernel<TIn>;
+  auto kern = resample_segments_kernel<TIn, STREAM>;
   ACX_SET_MAX_SMEM(kern, RS_MAX_SMEM);
   kern<<<(unsigned)n_tiles, RS_THREADS, (size_t)t.smem, reinterpret_cast<cudaStream_t>(stream)>>>(
       x, x_len, seg, tile_start, S, taps, orig, newf, width, t.P, t.F, t.G, out, out_len);
@@ -1234,6 +1314,39 @@ int acx_resample_segments_pcm16(const int16_t* x, long long x_len, const long lo
                                 int width, float* out, long long out_len, void* stream) {
   return resample_segments_impl<int16_t>(x, x_len, seg, S, tile_start, n_tiles, taps, orig, newf, width, out, out_len,
                                          stream);
+}
+
+int acx_resample_stream(const float* x, long long x_len, const long long* table, int S, const long long* tile_start,
+                        long long n_tiles, const float* taps, int orig, int newf, int width, float* out, long long out_len,
+                        void* stream) {
+  return resample_segments_impl<float, true>(x, x_len, table, S, tile_start, n_tiles, taps, orig, newf, width, out,
+                                             out_len, stream);
+}
+
+}  // extern "C"
+
+template <typename TIn>
+static int stream_append_impl(const TIn* src, long long src_len, const long long* table, int S, float* ring,
+                              long long ring_len, void* stream) {
+  ACX_CHECK(src && table && ring, ACX_ERR_ARG, "stream_append: null pointer");
+  ACX_CHECK(S >= 1 && src_len >= 1 && src_len <= 0x7fffffffLL * 256 && ring_len >= 1, ACX_ERR_ARG,
+            "stream_append: bad sizes S=%d src_len=%lld ring_len=%lld", S, src_len, ring_len);
+  stream_append_kernel<TIn><<<(unsigned)((src_len + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      src, src_len, table, S, ring, ring_len);
+  ACX_CUDA(cudaGetLastError());
+  return ACX_OK;
+}
+
+extern "C" {
+
+int acx_stream_append(const float* src, long long src_len, const long long* table, int S, float* ring, long long ring_len,
+                      void* stream) {
+  return stream_append_impl<float>(src, src_len, table, S, ring, ring_len, stream);
+}
+
+int acx_stream_append_pcm16(const int16_t* src, long long src_len, const long long* table, int S, float* ring,
+                            long long ring_len, void* stream) {
+  return stream_append_impl<int16_t>(src, src_len, table, S, ring, ring_len, stream);
 }
 
 }  // extern "C"

@@ -149,15 +149,16 @@ def _pcm_to_float(src, dst):
     torch.div(src.to(dst.device).to(torch.float32), torch.tensor(32767.0, device=dst.device), out=dst)
 
 
-def pack_waveforms(waveforms, device):
+def pack_waveforms(waveforms, device, pin_memory=False):
     """The waveforms end to end in one device buffer: int16 when every one is int16, else float32 (int16 converted by a
     correctly rounded x / 32767, other float dtypes cast).  A single contiguous float32 / int16 waveform already on the
-    device is returned as it is, not copied."""
+    device is returned as it is, not copied.  pin_memory: a new host buffer is allocated in pinned memory."""
     w0 = waveforms[0] if len(waveforms) == 1 else None
     if w0 is not None and w0.device == device and w0.dtype in (torch.float32, torch.int16) and w0.is_contiguous():
         return w0.detach()
     pcm = bool(waveforms) and all(w.dtype == torch.int16 for w in waveforms)
-    buf = torch.empty(sum(w.numel() for w in waveforms), dtype=torch.int16 if pcm else torch.float32, device=device)
+    buf = torch.empty(sum(w.numel() for w in waveforms), dtype=torch.int16 if pcm else torch.float32, device=device,
+                      pin_memory=pin_memory)
     base = 0
     for w in waveforms:
         dst = buf[base:base + w.numel()]

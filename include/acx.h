@@ -294,6 +294,35 @@ ACX_API int acx_resample_segments_pcm16(const int16_t* x, long long x_len, const
                                         const long long* tile_start, long long n_tiles, const float* taps, int orig,
                                         int newf, int width, float* out, long long out_len, void* stream);
 
+/* ---- live streams: per-stream rings in one fp32 buffer ---------------------------------------------------------------
+ * acx_stream_append(_pcm16) scatters one push's chunks, packed end to end in src (src_len samples; fp32, or int16 PCM
+ * converted x / 32767. with a correctly rounded division), into the streams' rings in ONE launch.  table is a DEVICE
+ * (S, 6) int64 table, row s = (src_off, n, ring_base, cap, pos, mirror), rows in src order: sample i < n of chunk s goes
+ * to ring[ring_base + (pos + i) mod cap], and also to ring[ring_base + cap + (pos + i) mod cap] when that slot is below
+ * `mirror` (so a window of up to `mirror` samples starting anywhere in the ring is contiguous).  Each entry is clamped
+ * (src_off to [0, src_len], n <= cap, pos reduced mod cap, mirror <= cap, [ring_base, ring_base + cap + mirror) inside
+ * ring_len): no table value makes the kernel write outside its row's region.  A null pointer, S < 1, src_len outside [1, 2^39) or ring_len < 1 returns
+ * ACX_ERR_ARG before any launch. */
+ACX_API int acx_stream_append(const float* src, long long src_len, const long long* table, int S, float* ring,
+                              long long ring_len, void* stream);
+ACX_API int acx_stream_append_pcm16(const int16_t* src, long long src_len, const long long* table, int S, float* ring,
+                                    long long ring_len, void* stream);
+
+/* acx_resample_stream: the streaming form of acx_resample_segments (same taps, tiling, tile prefix and argument checks;
+ * fp32 input only).  table is a DEVICE (S, 8) int64 table, row s = (in_base, in_cap, in_end, f0, n_out, out_base,
+ * out_cap, out_mirror) for one stream: its input sample idx is x[in_base + idx mod in_cap] for 0 <= idx < in_end and
+ * zero otherwise, and the row computes the n_out outputs j = f0 * newf + jl (jl < n_out; f0 a 64-bit stream frame) with
+ * the same fmaf chain as acx_resample_segments.  Output j goes to out[out_base + j mod out_cap], and also to
+ * out[out_base + out_cap + j mod out_cap] when that slot is below out_mirror.  So outputs computed piece by piece equal
+ * acx_resample_segments of the whole stream bit for bit, as long as the ring still holds every sample a frame reads
+ * (the caller's invariant).  Tiles are counted on n_out as segments count them on out_len.  Entries are clamped to
+ * x_len / out_len like the segments' are (in_cap and out_cap >= 1 or the row is skipped, out_mirror <= out_cap, f0 to
+ * [0, 2^62 / max(orig, newf)] so that no index overflows): no table value makes the kernel read or write outside its
+ * row's regions.  x and out may be one buffer when the regions do not overlap. */
+ACX_API int acx_resample_stream(const float* x, long long x_len, const long long* table, int S,
+                                const long long* tile_start, long long n_tiles, const float* taps, int orig, int newf,
+                                int width, float* out, long long out_len, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
