@@ -76,6 +76,10 @@ SIGNATURES = {
     "acx_stream_append": [_vp, _ll, _vp, _i, _vp, _ll, _vp],
     "acx_stream_append_pcm16": [_vp, _ll, _vp, _i, _vp, _ll, _vp],
     "acx_resample_stream": [_vp, _ll, _vp, _i, _vp, _ll, _vp, _i, _i, _i, _vp, _ll, _vp],
+    # sound event detection: bins averaged from (M, 4) int64 row ranges; events from (S, 6) int64 sequences, in a count
+    # phase (0) and a write phase (1)
+    "acx_window_activity": [_vp, _ll, _vp, _ll, _vp, _vp],
+    "acx_detect_events": [_vp, _ll, _vp, _i, _vp, _vp, _ll, _ll, _ll, _vp, _vp, _vp, _i, _vp, _vp, _ll, _vp],
 }
 
 

@@ -288,7 +288,7 @@ class ConvNeXt(nn.Module):
         return res
 
     def open_stream(self, n_streams=1, window_samples=320000, hop_samples=32000, sample_rate=32000,
-                    frame_embeddings=False, piece_seconds=10):
+                    frame_embeddings=False, piece_seconds=10, detection=None):
         """Tag `n_streams` live audio streams window by window as their samples arrive; returns a stream.StreamTagger.
 
         s.push(chunks) appends new samples: one 1-D tensor (n_streams == 1) or a sequence of n_streams entries, each a
@@ -311,9 +311,18 @@ class ConvNeXt(nn.Module):
         A push longer than `piece_seconds` of a stream's audio is appended and tagged piece by piece within the call.
         Work runs on the current CUDA stream.  A wrong chunk count, a chunk that is not 1-D or has a bad dtype, a push
         to a closed stream, a bad rate, or a stream under 7360 samples (after resampling) at close raises ValueError
-        before anything is copied or launched, and leaves every stream unchanged."""
+        before anything is copied or launched, and leaves every stream unchanged.
+
+        detection: None, or a sed.Detection.  With one, every push / close result also has "activity" (the activity bins
+        that became final during the call) and "events" (the events that became final), keyed as sed.detect returns
+        them, "recording" being the stream index.  For every stream, its activity rows from all calls equal the rows of
+        sed.detect(forward_windows(whole stream, sample_rate=rate), detection)["activity"], and its events from all calls,
+        stably sorted by (class, onset), equal that recording's events, bit for bit.  It needs hop_samples <=
+        window_samples and adds a fixed row ring and event state per stream (s.detection_bytes; stream.BinPlanner);
+        each call with new bins reads one event count back from the device per piece.  None changes nothing."""
         from .stream import StreamTagger
-        return StreamTagger(self, n_streams, window_samples, hop_samples, sample_rate, frame_embeddings, piece_seconds)
+        return StreamTagger(self, n_streams, window_samples, hop_samples, sample_rate, frame_embeddings, piece_seconds,
+                            detection)
 
     def forward_logmel(self, x):
         """Normalised log-mel (B, T, 224): the tensor the reference has after bn0 (CX:298-306)."""

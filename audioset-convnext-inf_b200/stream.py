@@ -32,7 +32,7 @@ import os
 import numpy as np
 import torch
 
-from . import _native, preprocess
+from . import _native, preprocess, sed
 from .engine import MIN_RAGGED_LEN, N_CLASSES, DIMS, out_time_dims
 from .windows import WindowPlan, plan_windows
 
@@ -182,17 +182,99 @@ class StreamPlanner:
                      {r: np.array(rows, dtype=np.int64) for r, rows in res.items()}, plan)
 
 
+class BinPlanner:
+    """Host side of sound event detection on live streams (sed.py has the definitions): which activity bins became
+    final, which window rows they read, and where those rows sit in the device row ring.  No device work happens here.
+
+    Finality: while stream i is open, bin j is final iff (j + 1) R <= n_final_i - window.  No window still to come can
+    then intersect it (a regular one starts at or after n_final - window + 1 and the end-aligned tail at n - window >=
+    n_final - window), and every window that does is already complete.  At close every remaining bin is final.
+
+    Row ring: stream i owns `cap` rows (rows i cap .. i cap + cap - 1 of one (S cap, 527) float32 buffer); its k-th window
+    row goes to slot k mod cap.  A row is held until every bin it intersects is final, i.e. while start + window > j R
+    for the first bin j not yet final, so the held rows start after n_final - 2 window - R; a piece adds rows starting up
+    to n_final + piece_out - window, and close one end-aligned tail.  So cap = (window + R + piece_out) // hop + 2 rows
+    (piece_out: the most 32 kHz samples one piece makes final) holds every row a not-yet-final bin reads.  hop > window
+    leaves bins no window covers, so it is refused."""
+
+    def __init__(self, n_streams, window, hop, resolution, piece_out):
+        if hop > window:
+            raise ValueError(f"detection needs hop_samples <= window_samples (got {hop} > {window}): with gaps between "
+                             "windows some bins would be covered by no window")
+        self.window, self.hop, self.R = int(window), int(hop), int(resolution)
+        self.cap = (self.window + self.R + int(piece_out)) // self.hop + 2
+        self.n_rows = [0] * n_streams         # window rows received: the next row's k
+        self.first = [0] * n_streams          # k of the oldest held row
+        self.starts = [np.zeros(0, np.int64) for _ in range(n_streams)]   # held rows' starts and ends
+        self.ends = [np.zeros(0, np.int64) for _ in range(n_streams)]
+        self.n_bins = [0] * n_streams         # final bins
+        self.closed = [False] * n_streams
+
+    def step(self, rec, start, length, n_final, close=()):
+        """One piece: its window rows (recording = stream, start, length; stream-major), every stream's final 32 kHz
+        samples after it, and the streams it closes.  Returns (slots (N,) int64 ring rows of the piece's rows, table
+        (M, 4) int64 for acx_window_activity, bins {recording, start, length} (M,) int64, seq (S, 6) int64 for
+        acx_detect_events or None when no bin became final and no stream closes)."""
+        close = set(close)
+        W, R, cap = self.window, self.R, self.cap
+        slots = np.empty(len(rec), np.int64)
+        for i in np.unique(rec).tolist():
+            sel = np.flatnonzero(rec == i)
+            slots[sel] = i * cap + (self.n_rows[i] + np.arange(sel.size)) % cap
+            self.n_rows[i] += sel.size
+            self.starts[i] = np.concatenate([self.starts[i], start[sel]])
+            self.ends[i] = np.concatenate([self.ends[i], start[sel] + length[sel]])
+            assert self.n_rows[i] - self.first[i] <= cap, "row ring bound violated"
+        tables, b_rec, b_start, b_len, seq = [], [], [], [], []
+        row0 = 0
+        for i, n in enumerate(n_final):
+            closing = i in close
+            j0 = self.n_bins[i]
+            total = -(-n // R) if closing else (j0 if self.closed[i] else max(j0, (n - W) // R))
+            if total > j0:
+                first, count = sed.bin_ranges(self.starts[i], self.ends[i], j0, total, R, n)
+                assert (count >= 1).all(), "a final bin is covered by no window"
+                tables.append(np.stack([self.first[i] + first, count, np.full_like(count, i * cap),
+                                        np.full_like(count, cap)], axis=1))
+                j = np.arange(j0, total, dtype=np.int64)
+                b_rec.append(np.full(j.size, i, np.int64))
+                b_start.append(j * R)
+                b_len.append(np.minimum((j + 1) * R, n) - j * R)
+                drop = int(np.searchsorted(self.ends[i], total * R, side="right"))   # no later bin reads these
+                self.first[i] += drop
+                self.starts[i], self.ends[i] = self.starts[i][drop:], self.ends[i][drop:]
+            seq.append((i, row0, total - j0, j0, n if closing else total * R, int(closing)))
+            row0 += total - j0
+            self.n_bins[i] = total
+            self.closed[i] |= closing
+
+        def cat(parts, k=None):
+            return np.concatenate(parts).astype(np.int64) if parts else np.zeros((0,) if k is None else (0, k), np.int64)
+
+        bins = {"recording": cat(b_rec), "start": cat(b_start), "length": cat(b_len)}
+        busy = row0 > 0 or bool(close)
+        return slots, cat(tables, 4), bins, (np.array(seq, dtype=np.int64) if busy else None)
+
+
 class StreamTagger:
     """n live streams tagged by one model (ConvNeXt.open_stream).  push() appends chunks and returns the windows that
-    became complete; close() ends streams and returns their last windows.  See the module docstring for the layout."""
+    became complete; close() ends streams and returns their last windows.  See the module docstring for the layout.
+    With a sed.Detection, every result also carries the activity bins and events that became final (BinPlanner)."""
 
     def __init__(self, model, n_streams=1, window_samples=320000, hop_samples=32000, sample_rate=32000,
-                 frame_embeddings=False, piece_seconds=10):
+                 frame_embeddings=False, piece_seconds=10, detection=None):
         model._check_inference(None)
         if isinstance(n_streams, bool) or not isinstance(n_streams, numbers.Integral) or n_streams < 1:
             raise ValueError(f"n_streams = {n_streams!r}: expected a positive int")
         rates = preprocess.sample_rates(sample_rate, int(n_streams))
         self.planner = StreamPlanner(rates, window_samples, hop_samples, piece_seconds)
+        self.detection = detection
+        if detection is not None:
+            if not isinstance(detection, sed.Detection):
+                raise ValueError("detection must be a sed.Detection or None")
+            p = self.planner
+            self.bins = BinPlanner(p.n_streams, p.window, p.hop, detection.resolution,
+                                   max(c - p.window for c in p.out_cap))
         self.model = model
         self.frame_embeddings = bool(frame_embeddings)
         eng = model._get_engine()
@@ -203,10 +285,22 @@ class StreamTagger:
             self._filters[r] = (taps, width, orig, new) + preprocess.segment_tiling(orig, new, width)
         # NaN until written: a read of a slot no sample has reached shows in the results
         self.ring = torch.full((self.planner.ring_len,), float("nan"), dtype=torch.float32, device=self.device)
+        if detection is not None:
+            self.row_ring = torch.full((self.planner.n_streams * self.bins.cap, N_CLASSES), float("nan"),
+                                       dtype=torch.float32, device=self.device)
+            self.sed_state = sed.new_state(self.planner.n_streams, self.device)
 
     @property
     def ring_bytes(self):
         return self.ring.numel() * self.ring.element_size()
+
+    @property
+    def detection_bytes(self):
+        """Device memory of detection, fixed at open: the row ring (BinPlanner.cap rows of 527 float32 per stream) and
+        the per-track event state (3 int64 + 1 float32 per stream and class); 0 without detection."""
+        if self.detection is None:
+            return 0
+        return sum(t.numel() * t.element_size() for t in (self.row_ring,) + self.sed_state)
 
     def _chunks(self, chunks):
         S = self.planner.n_streams
@@ -298,15 +392,26 @@ class StreamTagger:
                          ring.numel(), st)
         self._check_amplitude(eng, old_final)
         plan = piece.plan
-        if not plan.length.numel():
-            return None
-        want = ("logits", "scene", "frame") if self.frame_embeddings else ("logits", "scene")
-        out = eng.run_windows(ring, plan, want)
-        res = {"clipwise_output": out["probs"], "clipwise_logits": out["logits"], "scene_embeddings": out["scene"],
-               "recording": plan.recording, "start": plan.start, "length": plan.length}
-        if self.frame_embeddings:
-            res["frame_embeddings"] = out["frame"]
-        return res
+        res = None
+        if plan.length.numel():
+            want = ("logits", "scene", "frame") if self.frame_embeddings else ("logits", "scene")
+            out = eng.run_windows(ring, plan, want)
+            res = {"clipwise_output": out["probs"], "clipwise_logits": out["logits"], "scene_embeddings": out["scene"],
+                   "recording": plan.recording, "start": plan.start, "length": plan.length}
+            if self.frame_embeddings:
+                res["frame_embeddings"] = out["frame"]
+        return res, (self._detect(plan, res, close) if self.detection is not None else None)
+
+    def _detect(self, plan, res, close):
+        """The piece's rows into the row ring, then the bins that became final and the events they finalise."""
+        slots, table, bins, seq = self.bins.step(plan.recording.numpy(), plan.start.numpy(), plan.length.numpy(),
+                                                 self.planner.n_final, close)
+        if len(slots):
+            idx = torch.from_numpy(slots).pin_memory().to(self.device, non_blocking=True)
+            self.row_ring.index_copy_(0, idx, res["clipwise_output"])
+        act = sed.window_activity(self.row_ring, table)
+        events = sed.detect_events(act, seq, self.detection, self.sed_state) if seq is not None else None
+        return act, bins, events
 
     def _check_amplitude(self, eng, old_final):
         """ACX_CHECK_AMPLITUDE=1: the 32 kHz samples that became final in this piece (resampled where the stream is not at
@@ -325,8 +430,37 @@ class StreamTagger:
             self.model._check_amplitude(eng, torch.stack(parts))
 
     def _gather(self, parts):
-        """The rows of all pieces of one call, stream-major with start ascending, on the device."""
-        parts = [p for p in parts if p is not None]
+        """The rows of all pieces of one call, stream-major with start ascending, on the device; with detection also its
+        activity bins (stream-major, start ascending) and events (stream, class, onset)."""
+        res = self._gather_rows([p[0] for p in parts if p[0] is not None])
+        if self.detection is not None:
+            res["activity"], res["events"] = self._gather_sed([p[1] for p in parts])
+        return res
+
+    def _gather_sed(self, parts):
+        dev = self.device
+        host = {k: np.concatenate([p[1][k] for p in parts] + [np.zeros(0, np.int64)]) for k in sed.ACTIVITY_KEYS[1:]}
+        acts = [p[0] for p in parts if len(p[0])]
+        act = torch.cat(acts) if acts else torch.empty(0, N_CLASSES, dtype=torch.float32, device=dev)
+        if len(acts) > 1:                 # pieces come in time order: a stable sort on the stream keeps start ascending
+            order = np.argsort(host["recording"], kind="stable")
+            host = {k: v[order] for k, v in host.items()}
+            act = act.index_select(0, torch.from_numpy(order).to(dev, non_blocking=True))
+        activity = {"activity": act}
+        activity.update({k: torch.from_numpy(v).to(dev) for k, v in host.items()})
+        evs = [p[2] for p in parts if p[2] is not None and p[2]["onset"].numel()]
+        if not evs:
+            empty = torch.zeros(0, dtype=torch.int64, device=dev)
+            events = {k: empty for k in sed.EVENT_KEYS[:-1]}
+            events["peak"] = torch.empty(0, dtype=torch.float32, device=dev)
+        else:
+            events = {k: torch.cat([e[k] for e in evs]) for k in sed.EVENT_KEYS}
+            if len(evs) > 1:              # a track's events come in onset order, piece after piece
+                order = torch.sort(events["recording"] * N_CLASSES + events["class"], stable=True).indices
+                events = {k: v.index_select(0, order) for k, v in events.items()}
+        return activity, events
+
+    def _gather_rows(self, parts):
         dev = self.device
         h3w = out_time_dims(self.planner.window)[1][3]
         if not parts:

@@ -323,6 +323,39 @@ ACX_API int acx_resample_stream(const float* x, long long x_len, const long long
                                 const long long* tile_start, long long n_tiles, const float* taps, int orig, int newf,
                                 int width, float* out, long long out_len, void* stream);
 
+/* ---- sound event detection: window rows -> activity bins -> timed events (527 classes) --------------------------------
+ * acx_window_activity: probs is (p_rows, 527) fp32 clipwise rows (a forward_windows result, or a ring of a stream's
+ * recent rows); table is a DEVICE (M, 4) int64 table, one row per output bin, row m = (row_first, n, ring_base, ring_cap).
+ * Row t < n of bin m is probs[ring_base + (row_first + t) mod ring_cap], and
+ *   act[m, c] = (sum over t of those rows' column c) / n,
+ * the sum taken with plain fp32 adds in t order starting from the first row, the division correctly rounded (act is
+ * (M, 527) fp32).  A whole recording uses ring_base = 0, ring_cap = p_rows.  Every entry is clamped (ring_cap to
+ * [1, p_rows], ring_base to [0, p_rows - ring_cap], n to [0, ring_cap], row_first reduced mod ring_cap): no table value
+ * reads outside probs; a bin with n = 0 reads nothing and is NaN.  A null pointer, p_rows < 1, M < 1 or M > 2^40 / 527
+ * returns ACX_ERR_ARG before any launch. */
+ACX_API int acx_window_activity(const float* probs, long long p_rows, const long long* table, long long M, float* act,
+                                void* stream);
+
+/* acx_detect_events: one thread per (sequence, class) track walks the sequence's new bins through the hysteresis state
+ * machine (open at act >= on[c], stay open while act >= off[c], end at the first bin where !(act >= off[c]); consecutive
+ * events merge when next onset - previous offset < merge_gap; an event is kept when offset - onset >= min_duration).  seq
+ * is a DEVICE (S, 6) int64 table, row s = (recording, row0, n_bins, j0, limit, close): the sequence's new bins are act
+ * rows row0 .. row0 + n_bins - 1 with bin indices j0 .. j0 + n_bins - 1, bin j spans [j resolution, min((j + 1)
+ * resolution, limit)), and close != 0 ends the sequence.  state ((3, S * 527) int64: phase 0 idle / 1 open / 2 ended but
+ * may merge, onset bin, last bin) and state_peak ((S * 527) fp32) carry each track from call to call; zeros are a fresh
+ * track.  An event is emitted once no later bin can change it: at close, or once the next bin's start minus its offset
+ * reaches merge_gap.  phase 0 writes the number of events each track emits to slots[s * 527 + c] and changes nothing
+ * else; the caller turns the counts into their exclusive prefix in place, and phase 1 writes the events from those slots
+ * and stores the state: out is (4, E) int64 rows (recording, class, onset, offset) in samples and out_peak (E,) fp32 the
+ * max activity over the event's bins, ordered (sequence, class, onset).  row0 and n_bins are clamped to act_rows, and no
+ * event is written outside [0, E).  A null pointer (act may be null with act_rows = 0, out / out_peak with E = 0 or in
+ * phase 0), S outside [1, 2^30 / 527], act_rows outside [0, 2^40 / 527], E < 0, resolution < 1, merge_gap < 0,
+ * min_duration < 0 or a phase other than 0 / 1 returns ACX_ERR_ARG before any launch. */
+ACX_API int acx_detect_events(const float* act, long long act_rows, const long long* seq, int S,
+                              const float* on_threshold, const float* off_threshold, long long resolution,
+                              long long merge_gap, long long min_duration, long long* state, float* state_peak,
+                              long long* slots, int phase, long long* out, float* out_peak, long long E, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
