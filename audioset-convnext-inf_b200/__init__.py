@@ -10,6 +10,6 @@ from .convnext import (Block, ConvNeXt, LayerNorm, LogmelFilterBank, Spectrogram
 from .engine import Engine, PackedWeights, out_time_dims  # noqa: F401
 from .pipeline import HostPipeline  # noqa: F401
 from . import evalloop  # noqa: F401
-from . import extract, preprocess, sed, stream, windows  # noqa: F401
+from . import extract, preprocess, search, sed, stream, windows  # noqa: F401
 
 __all__ = ["ConvNeXt", "convnext_tiny", "Block", "LayerNorm", "Engine", "HostPipeline", "load_checkpoint"]

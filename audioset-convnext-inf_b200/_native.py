@@ -80,6 +80,12 @@ SIGNATURES = {
     # phase (0) and a write phase (1)
     "acx_window_activity": [_vp, _ll, _vp, _ll, _vp, _vp],
     "acx_detect_events": [_vp, _ll, _vp, _i, _vp, _vp, _ll, _ll, _ll, _vp, _vp, _vp, _i, _vp, _vp, _ll, _vp],
+    # query by example: fp64 row norms, the (Q, N) fp32 cosine score block, and the per-query top k over it (optional
+    # (N, 2) int64 neighbour ranges, caller-owned workspace sized by the host query)
+    "acx_row_norms": [_vp, _ll, _i, _vp, _vp],
+    "acx_cosine_scores": [_vp, _vp, _ll, _vp, _vp, _ll, _i, _vp, _vp],
+    "acx_search_topk_workspace": [_ll, _ll, _vp],
+    "acx_search_topk": [_vp, _ll, _ll, _vp, _i, _vp, _vp, _vp, _vp],
 }
 
 

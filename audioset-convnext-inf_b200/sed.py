@@ -34,6 +34,7 @@ import torch
 
 from . import _native
 from .engine import N_CLASSES
+from .windows import check_rows
 
 ACTIVITY_KEYS = ("activity", "recording", "start", "length")
 EVENT_KEYS = ("recording", "class", "onset", "offset", "peak")
@@ -104,23 +105,7 @@ def _host_rows(windows):
     if not isinstance(probs, torch.Tensor) or probs.dim() != 2 or probs.shape[1] != N_CLASSES \
             or probs.dtype != torch.float32:
         raise ValueError(f"clipwise_output must be a (N, {N_CLASSES}) float32 tensor")
-    cols = []
-    for k in ("recording", "start", "length"):
-        v = windows[k]
-        if not isinstance(v, torch.Tensor) or v.dim() != 1 or v.dtype != torch.int64:
-            raise ValueError(f"{k} must be a 1-D int64 tensor")
-        if v.numel() != probs.shape[0]:
-            raise ValueError(f"{k} has {v.numel()} rows, clipwise_output {probs.shape[0]}")
-        cols.append(v.cpu().numpy())
-    rec, start, length = cols
-    if (rec < 0).any() or (start < 0).any() or (length < 1).any():
-        raise ValueError("recording and start must be >= 0 and length >= 1")
-    if (np.diff(rec) < 0).any():
-        raise ValueError("rows must be recording-major (recording non-decreasing)")
-    same = np.diff(rec) == 0
-    end = start + length
-    if (np.diff(start)[same] <= 0).any() or (np.diff(end)[same] < 0).any():
-        raise ValueError("within a recording, rows must have start ascending and start + length non-decreasing")
+    rec, start, length = check_rows(windows, probs.shape[0], "clipwise_output")
     return probs.contiguous(), rec, start, length
 
 

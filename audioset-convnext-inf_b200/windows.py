@@ -72,3 +72,27 @@ def window_batches(plan, chunk):
         rows = [short[j] for j in idx]
         out.append((canvas, [length[i] for i in rows], rows))
     return out
+
+
+def check_rows(windows, n_rows, rows_key):
+    """The "recording", "start" and "length" columns of a windows dict checked on the host, as numpy int64: each a 1-D
+    int64 tensor of n_rows rows (the row count of windows[rows_key]), recording and start >= 0, length >= 1, rows
+    recording-major with start ascending and start + length non-decreasing within a recording.  Raises ValueError."""
+    cols = []
+    for k in ("recording", "start", "length"):
+        v = windows[k]
+        if not isinstance(v, torch.Tensor) or v.dim() != 1 or v.dtype != torch.int64:
+            raise ValueError(f"{k} must be a 1-D int64 tensor")
+        if v.numel() != n_rows:
+            raise ValueError(f"{k} has {v.numel()} rows, {rows_key} {n_rows}")
+        cols.append(v.cpu().numpy())
+    rec, start, length = cols
+    if (rec < 0).any() or (start < 0).any() or (length < 1).any():
+        raise ValueError("recording and start must be >= 0 and length >= 1")
+    if (np.diff(rec) < 0).any():
+        raise ValueError("rows must be recording-major (recording non-decreasing)")
+    same = np.diff(rec) == 0
+    end = start + length
+    if (np.diff(start)[same] <= 0).any() or (np.diff(end)[same] < 0).any():
+        raise ValueError("within a recording, rows must have start ascending and start + length non-decreasing")
+    return rec, start, length

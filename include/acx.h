@@ -356,6 +356,32 @@ ACX_API int acx_detect_events(const float* act, long long act_rows, const long l
                               long long merge_gap, long long min_duration, long long* state, float* state_peak,
                               long long* slots, int phase, long long* out, float* out_peak, long long E, void* stream);
 
+/* ---- query by example: exact cosine search over embedding rows -------------------------------------------------------
+ * acx_row_norms: out[r] = sqrt(sum_i x[r, i]^2) (fp64) for the (rows, d) fp32 rows x, the sum taken in fp64 in i order
+ * from 0.0.  A null pointer, rows outside [1, 2^40] or d < 1 returns ACX_ERR_ARG before any launch. */
+ACX_API int acx_row_norms(const float* x, long long rows, int d, double* out, void* stream);
+
+/* acx_cosine_scores: scores (Q, N) fp32, row-major, scores[q, n] = float32(dot / (query_norms[q] * key_norms[n])), where
+ * dot = sum_i queries[q, i] * keys[n, i] is the fp64 fma chain over i = 0 .. d-1 in order from 0.0 (every product of two
+ * fp32 values is exact in fp64, so it equals the plain fp64 sum), the product and quotient are rounded once each in fp64
+ * and the conversion rounds to nearest even; a NaN result is stored as 0x7fc00000.  queries (Q, d) and keys (N, d) fp32
+ * are row-major, the norms are acx_row_norms results.  Indices are 64-bit: Q * N may exceed 2^31.  A null pointer, Q
+ * outside [1, 65535 * 64], N outside [1, 2^31 - 1] or d < 1 returns ACX_ERR_ARG before any launch. */
+ACX_API int acx_cosine_scores(const float* queries, const double* query_norms, long long Q, const float* keys,
+                              const double* key_norms, long long N, int d, float* scores, void* stream);
+
+/* acx_search_topk: for every row q of scores ((Q, N) fp32, an acx_cosine_scores result), the top k' = min(k, eligible)
+ * rows under the order "a beats b when score_a > score_b, or the scores are equal and a < b" (-0.0 equals +0.0; NaN ranks
+ * below every number and NaNs tie).  Row w is eligible when it beats every row j != w in [lo_w, hi_w), (lo_w, hi_w) = row
+ * w of ranges, a DEVICE (N, 2) int64 table, each entry clamped to [0, N]; ranges = null makes every row eligible.
+ * out_score (Q, k) fp32 and out_index (Q, k) int64 receive the hits best first; slots k' .. k-1 get score NaN
+ * (0x7fc00000) and index -1.  workspace is DEVICE scratch of acx_search_topk_workspace(Q, N) bytes (a host query, no
+ * launch).  Two launches, no allocation and no synchronisation.  A null pointer (ranges excepted), Q or N outside
+ * [1, 2^31 - 1] or k outside [1, 1024] returns ACX_ERR_ARG before any launch. */
+ACX_API int acx_search_topk_workspace(long long Q, long long N, long long* bytes_host);
+ACX_API int acx_search_topk(const float* scores, long long Q, long long N, const long long* ranges, int k,
+                            float* out_score, long long* out_index, void* workspace, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
