@@ -30,18 +30,29 @@ def test_device_is_b200():
     assert N.load().acx_device_ok() == 1, N.last_error()
 
 
+@pytest.mark.parametrize("pcm", [False, True])
 @pytest.mark.parametrize("L", [320000, 1000, 40123])
-def test_wave_prep_reflect_pad_and_split(L):
+def test_wave_prep_reflect_pad_and_split(L, pcm):
+    """acx_wave_prep (fp32 input) and acx_wave_prep_pcm16 (int16 PCM, converted x / 32767 with one correct rounding):
+    bit-exact reflect padding in fp32 mode, the scaled fp16 hi / lo split in bf16 mode."""
     w = weights.make_waveforms(2, n_samples=L, kind="tones", seed=2).to(DEV)
+    entry = "acx_wave_prep"
+    if pcm:
+        wi = (w * 30000).round().clamp(-32768, 32767).to(torch.int16)
+        wi[:, :3] = torch.tensor([-32768, 32767, 0], device=DEV, dtype=torch.int16)
+        # utils/utilities.py:226 (true division), correctly rounded: IEEE fp32 division in numpy
+        w = torch.from_numpy(wi.cpu().numpy().astype(np.float32) / np.float32(32767.0)).to(DEV)
+        entry = "acx_wave_prep_pcm16"
+    src = wi if pcm else w
     ld = (L + 1024 + 7) // 8 * 8
     ref = F.pad(w[:, None], (512, 512), mode="reflect")[:, 0]
     pad32 = torch.full((2, ld), 7.0, device=DEV)
-    N.call("acx_wave_prep", w.data_ptr(), pad32.data_ptr(), 0, 2, L, 1024, ld, N.ACX_F32, _st())
+    N.call(entry, src.data_ptr(), pad32.data_ptr(), 0, 2, L, 1024, ld, N.ACX_F32, _st())
     assert torch.equal(pad32[:, : L + 1024], ref)            # bit-exact copy
     assert (pad32[:, L + 1024:] == 0).all()
     hi = torch.empty(2, ld, device=DEV, dtype=torch.float16)       # fp16 pair of 2^8 * x (include/acx.h)
     lo = torch.empty_like(hi)
-    N.call("acx_wave_prep", w.data_ptr(), hi.data_ptr(), lo.data_ptr(), 2, L, 1024, ld, N.ACX_BF16, _st())
+    N.call(entry, src.data_ptr(), hi.data_ptr(), lo.data_ptr(), 2, L, 1024, ld, N.ACX_BF16, _st())
     assert torch.equal(hi[:, : L + 1024], (ref * 256.0).to(torch.float16))
     rec = (hi.float() + lo.float()) / 256.0
     assert (rec[:, : L + 1024] - ref).abs().max() <= ref.abs().max() * 2.0 ** -21
@@ -299,7 +310,7 @@ def test_downsample_fused_implicit_gemm(sd, stage, H, B, out_gp):
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-@pytest.mark.parametrize("H", [31, 9])
+@pytest.mark.parametrize("H", [31, 9, 1, 2, 3])
 def test_head_and_frame_layout(sd, H, dtype):
     B = 3
     x = torch.randn(B, H, 7, 768, generator=torch.Generator().manual_seed(H))

@@ -219,7 +219,7 @@ def test_eval_loop_drop_in_matches_reference_loop_semantics(models, parity_sd):
 
 
 @pytest.mark.parametrize("prec", ["fp32", "bf16"])
-def test_edge_shapes(models, prec):
+def test_edge_shapes(models, parity_sd, prec):
     """B=1, batch larger than the chunk, the shortest clip the 4-stage trunk accepts, non-contiguous input."""
     m = models[prec]
     eng = m._get_engine()
@@ -233,8 +233,9 @@ def test_edge_shapes(models, prec):
     assert torch.equal(m(nc)["clipwise_logits"], full)
     short = weights.make_waveforms(2, n_samples=7 * 320 * 4 + 1, kind="noise", seed=51).to(DEV)   # T'=1 at stage 3
     fr = m.forward_frame_embeddings(short)
-    ref = O.forward_frame_embeddings(short.cpu(), weights.make_state_dict("parity", 8))
+    ref = O.forward_frame_embeddings(short.cpu().double(), parity_sd, torch.float64)
     assert fr.shape == ref.shape and fr.shape[2] >= 1
+    assert (fr.cpu().double() - ref).abs().max().item() < TOL[prec]["frame"]
     empty = m(torch.zeros(0, L, device=DEV))                         # empty batch: empty outputs, no launch
     assert empty["clipwise_output"].shape == (0, 527) and empty["clipwise_logits"].shape == (0, 527)
     assert m.forward_scene_embeddings(torch.zeros(0, L, device=DEV)).shape == (0, 768)
