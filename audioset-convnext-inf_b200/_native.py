@@ -5,8 +5,7 @@ import os
 import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# ACX_LIBACX points at an alternative build of the same library (A/B experiments with ACX_NVCC_EXTRA variants)
-_LIB_PATH = os.environ.get("ACX_LIBACX") or os.path.join(_HERE, "libacx.so")
+_LIB_PATH = os.path.join(_HERE, "libacx.so")
 _lock = threading.Lock()
 _lib = None
 

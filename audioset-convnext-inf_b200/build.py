@@ -14,8 +14,6 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
          "-shared", "-cudart", "static"]
-# extra compile flags for A/B experiments (e.g. ACX_NVCC_EXTRA="-DACX_GELU_PLAIN"); part of the digest
-FLAGS += os.environ.get("ACX_NVCC_EXTRA", "").split()
 
 
 def _sources():

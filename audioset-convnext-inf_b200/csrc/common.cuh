@@ -213,11 +213,7 @@ __device__ __forceinline__ void gelu_stage_ta4(GeluPair* t, GeluPair* a, const u
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       float2 b;
-#ifdef ACX_AB_NO_FOLD_EPI     /* A/B experiment: statistics pass on, plain bias epilogue */
-      if (false) {
-#else
       if (kFold) {
-#endif
         float2 sj;
         asm("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
             : "=f"(b.x), "=f"(b.y), "=f"(sj.x), "=f"(sj.y)

@@ -33,21 +33,7 @@ struct DsArgs {
   int H, W, Ho, Wo;      // input map / output map
   int Mo;                // output rows = B * Ho * Wo
   int out_gp;            // 1: output group-planar [2C/8][Mp_out][8]; 0: row-major (Mo, 2C)
-  long long* trace;      // debug builds (-DACX_DS_TRACE): per-role SM-clock sums of CTA 0
 };
-#ifdef ACX_DS_TRACE
-#define DS_T0() long long tr_t = clock64(), tr_w = 0, tr_w2 = 0, tr_s = tr_t, tr_a = 0, tr_b = 0, tr_d = 0
-#define DS_OUT3(i, cond) do { if (a.trace && blockIdx.x == 0 && (cond)) { a.trace[i] = tr_a; a.trace[i + 1] = tr_b; a.trace[i + 2] = tr_d; } } while (0)
-#define DS_ACC(acc) do { const long long t_ = clock64(); acc += t_ - tr_t; tr_t = t_; } while (0)
-#define DS_MARK() do { tr_t = clock64(); } while (0)
-#define DS_OUT(i, cond) do { if (a.trace && blockIdx.x == 0 && (cond)) { a.trace[i] = clock64() - tr_s; a.trace[i + 1] = tr_w; a.trace[i + 2] = tr_w2; } } while (0)
-#else
-#define DS_T0() do { } while (0)
-#define DS_ACC(acc) do { } while (0)
-#define DS_MARK() do { } while (0)
-#define DS_OUT(i, cond) do { } while (0)
-#define DS_OUT3(i, cond) do { } while (0)
-#endif
 
 template <int C>
 struct DsCfg {
@@ -177,13 +163,10 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
     if (ptx::elect_one()) {
       int stage = 0;
       uint32_t phase = 0;
-      DS_T0();
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         const int n0 = (tile % Cfg::N_TILES) * Cfg::TILE_N;
         for (int kb = 0; kb < Cfg::NKB; ++kb) {
-          DS_MARK();
           ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
-          DS_ACC(tr_w);
           uint8_t* sb = smem + stage * Cfg::STAGE_BYTES + Cfg::A_BYTES;
           ptx::mbar_arrive_expect_tx(&full_bar[stage], Cfg::B_BYTES);
 #pragma unroll
@@ -195,7 +178,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
           }
         }
       }
-      DS_OUT(0, true);
     }
   } else if (warp == 1) {
     // ================================ MMA issuer ================================
@@ -204,19 +186,14 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
-      DS_T0();
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
         const int acc = Cfg::NACC == 2 ? (it & 1) : 0;
         const uint32_t acc_phase = Cfg::NACC == 2 ? ((it >> 1) & 1) : (it & 1);
-        DS_MARK();
         ptx::mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        DS_ACC(tr_w2);
         ptx::tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * Cfg::ACC_STRIDE;
         for (int kb = 0; kb < Cfg::NKB; ++kb) {
-          DS_MARK();
           ptx::mbar_wait(&full_bar[stage], phase);
-          DS_ACC(tr_w);
           ptx::tc_fence_after();
           const uint32_t sa = ptx::smem_u32(smem + stage * Cfg::STAGE_BYTES);
           const uint64_t da = ptx::umma_desc_sw128_kmajor(sa);
@@ -236,7 +213,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
         }
         ptx::umma_commit(&tfull_bar[acc]);
       }
-      DS_OUT(3, true);
     }
   } else if (warp >= 4 && warp < 4 + Cfg::NGATHER) {
     // ================================ gather + LayerNorm: the A operand ================================
@@ -299,7 +275,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
     uint32_t phase = 0;
     int it = 0;
     bool valid;
-    DS_T0();
     const uint4* src0 = tile_src(blockIdx.x, valid);
     {
       bool v1;
@@ -368,7 +343,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
       // (the loop is unrolled by two; copying `nxt` into `cur` at the end of an iteration made every block wait for the
       // loads it had just issued: ncu source view, the MOV after the stores was the kernel's top stall).
       auto step = [&](const int kb, uint4 (&cur)[4], uint4 (&nxt)[4]) {
-        DS_MARK();
         prefetch_part(t2, v2, kb);
         if (has_next) {
           if (kb == 1) stats_reset(sp[0], sp[1], nvalid);
@@ -378,7 +352,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
           }
           stats_issue(kb);
         }
-        DS_ACC(tr_a);
         if (kb + 1 < Cfg::NKB) load_kb(src0, valid, kb + 1, nxt);
         else if (has_next) load_kb(nsrc0, nvalid, 0, nxt);
         const int dy = kb / Cfg::KB_PER_DY;
@@ -413,9 +386,7 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
             o[u * 2 + dx] = make_uint4(ov[0], ov[1], ov[2], ov[3]);
           }
         }
-        DS_ACC(tr_b);
         ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
-        DS_ACC(tr_w);
         const uint32_t row = smem_a + stage * Cfg::STAGE_BYTES + r * 128;
 #pragma unroll
         for (int i = 0; i < 4; ++i)      // 16-byte slot (2 hs + u) * 2 + dx of the 128-byte row, SWIZZLE_128B: slot ^ (row & 7)
@@ -423,7 +394,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
         ptx::fence_proxy_async_smem();   // generic-proxy stores -> visible to the tensor core's async-proxy reads
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&full_bar[stage]);
-        DS_ACC(tr_d);
         if (++stage == Cfg::STAGES) {
           stage = 0;
           phase ^= 1;
@@ -439,16 +409,11 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
         stats_add(sp[0], sp[1]);
         stats_add(sp[2], sp[3]);
         stats_store(sstat_a + ((it + 1) & 1) * (Cfg::BM * 4 * 8));
-        DS_MARK();
         asm volatile("bar.sync 1, 256;" ::: "memory");      // next tile's statistics complete; this tile's no longer read
-        DS_ACC(tr_w2);
       }
       src0 = nsrc0;
       valid = nvalid;
     }
-    DS_OUT(6, t == 0);
-    DS_OUT(9, t == 255);
-    DS_OUT3(16, t == 0);
   } else if (warp >= 4 + Cfg::NGATHER) {
     // ================================ epilogue ================================
     const int ew = warp - 4 - Cfg::NGATHER;
@@ -458,16 +423,13 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
     const uint32_t sbias_a = ptx::smem_u32(sbias);
     int it = 0;
     uint32_t store_parity = 0;
-    DS_T0();
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
       const int acc = Cfg::NACC == 2 ? (it & 1) : 0;
       const uint32_t acc_phase = Cfg::NACC == 2 ? ((it >> 1) & 1) : (it & 1);
       const int m0 = (tile / Cfg::N_TILES) * Cfg::BM;
       const int n0 = (tile % Cfg::N_TILES) * Cfg::TILE_N;
       const int row0 = m0 + quad * 32;
-      DS_MARK();
       ptx::mbar_wait(&tfull_bar[acc], acc_phase);
-      DS_ACC(tr_w);
       ptx::tc_fence_after();
       const uint32_t t_base = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * Cfg::ACC_STRIDE;
       uint32_t ra[32], rb[32];
@@ -510,7 +472,6 @@ __global__ void __launch_bounds__(DsCfg<C>::THREADS, 1)
       }
     }
     if (lane == 0) ptx::tma_store_wait_read<0>();   // smem must stay valid until the last store has read it
-    DS_OUT(12, ew == 0 && lane == 0);
   }
 
   ptx::tc_fence_before();
@@ -537,10 +498,6 @@ static int launch(const void* x, const float* ln_w, const float* ln_b, const voi
   a.Wo = W / 2;
   a.Mo = B * a.Ho * a.Wo;
   a.out_gp = out_gp;
-  a.trace = nullptr;
-#ifdef ACX_DS_TRACE     // debug builds only (ACX_NVCC_EXTRA=-DACX_DS_TRACE, tools/trace_ds.py)
-  if (getenv("ACX_DS_TRACE_PTR")) a.trace = reinterpret_cast<long long*>(strtoull(getenv("ACX_DS_TRACE_PTR"), nullptr, 0));
-#endif
   CUtensorMap tmW, tmOut;
   int rc = make_tmap_2d_bf16(&tmW, w, (uint64_t)Cfg::K, (uint64_t)Cfg::N, (uint64_t)Cfg::K * 2, 64, Cfg::BN);
   if (rc != ACX_OK) return rc;

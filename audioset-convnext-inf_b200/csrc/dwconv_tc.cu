@@ -69,21 +69,15 @@ __device__ __forceinline__ void tmem_ld_32x32b_x8(uint32_t taddr, uint32_t (&r)[
                : "memory");
 }
 
-// W = image width of the stage (56 / 28 / 14 / 7; <= 32 uses one K window).
-// GP = group-planar activations: x and v are [C/8][Mp][8] (M = clips * H * W pixels, Mp = M rounded up to 128 = the plane
-// stride; every 16-byte group of 8 channels is a plane).  With NHWC tensors a unit's 16-byte pieces sit 2 C bytes apart: each costs the LSU a 32-byte sector
-// request and the staging / write-out phases ran at ~5 useful B/clk/SM (24 k + 8 k of a unit's 54 k cycles, in-kernel
-// clock trace; TMA gathers the same pieces at 14 B/clk/SM, tools/ubench/tma_gather.cu).  In the planar layout a unit's
-// image rows are contiguous: fragment loads are full 128-byte lines and the results leave as 512-byte runs.
+// W = image width of the stage (56 / 28 / 14 / 7; <= 32 uses one K window).  x and v are NHWC.
 // RAG = ragged batch: clip n has valid[n] rows (clamped to [0, H]); the rows past it are staged as the conv's zero padding,
 // so its first valid[n] output rows equal a run at that height (the rows past it are computed but carry no meaning).
-template <int W, bool GP, bool RAG = false>
+template <int W, bool RAG = false>
 __global__ void __launch_bounds__(THREADS, 2)
     dwconv_tc_kernel(const bf16* __restrict__ x, const bf16* __restrict__ taps /*[49][C]*/,
                      const float* __restrict__ bias, bf16* __restrict__ v, int n_clips, int H, int C,
-                     long long* __restrict__ trace, const int32_t* __restrict__ valid) {
+                     const int32_t* __restrict__ valid) {
   constexpr int NHALF = W > 32 ? 2 : 1;
-  constexpr int HW = NHALF == 2 ? 28 : W;       // output pixels per half row
   constexpr int WB = (W + 7) / 8;               // 8-pixel blocks per image row
   constexpr int NM = AR * WB;                   // 8 x 8 fragments per unit
   constexpr int NG = (NM + 3) / 4;              // stmatrix.x4 groups
@@ -127,40 +121,19 @@ __global__ void __launch_bounds__(THREADS, 2)
 
   const int tiles = (H + TR - 1) / TR, groups = C / CG;
   const int units = n_clips * tiles * groups;
-#ifdef ACX_ENABLE_TRACE
-  long long tr_t0 = 0, tr_taps = 0, tr_stage = 0, tr_mma = 0, tr_epi = 0, tr_units = 0;
-#define DWTC_MARK(acc)                            \
-  do {                                            \
-    if (trace) {                                  \
-      const long long t_ = clock64();             \
-      acc += t_ - tr_t0;                          \
-      tr_t0 = t_;                                 \
-    }                                             \
-  } while (0)
-#else
-#define DWTC_MARK(acc) do { } while (0)
-#endif
   uint32_t bc = 0;          // band-slot uses so far (the MMA thread and the builders count the same sequence)
   uint32_t dphase = 0;
   for (int unit = blockIdx.x; unit < units; unit += gridDim.x) {
     const int g = unit % groups, t = (unit / groups) % tiles, n = unit / (groups * tiles);
     const int h0 = t * TR, c0 = g * CG;
-#ifdef ACX_ENABLE_TRACE
-    if (trace) tr_t0 = clock64();
-    ++tr_units;
-#endif
     // ---- taps of the 8 channels -> smem [c][49] -------------------------------------------------------------------
     for (int i = tid; i < 49 * CG; i += THREADS) {
       const int tap = i >> 3, c = i & 7;
       taps_s[c * 49 + tap] = reinterpret_cast<const uint16_t*>(taps)[tap * C + c0 + c];
     }
-    DWTC_MARK(tr_taps);
     // ---- stage: NHWC -> channel-planar A tiles ------------------------------------------------------------------------
     {
-      const size_t mtot = ((size_t)n_clips * H * W + 127) / 128 * 128;   // plane stride: rows rounded up to 128
-      const bf16* xin = GP ? x + ((size_t)g * mtot + (size_t)n * H * W) * 8 + 2 * (lane & 3)
-                           : x + (size_t)n * H * W * C + c0 + 2 * (lane & 3);
-      constexpr int kPix = GP ? 8 : 0;            // element stride between pixels: 8 (planar) or C (NHWC)
+      const bf16* xin = x + (size_t)n * H * W * C + c0 + 2 * (lane & 3);
       const int px = lane >> 2;                           // pixel of the fragment this lane loads
       const int sj = lane & 7, smi = lane >> 3;           // stored row (channel) / matrix this lane addresses
       const int hv = RAG ? min(max(__ldg(valid + n), 0), H) : H;      // RAG only
@@ -176,7 +149,7 @@ __global__ void __launch_bounds__(THREADS, 2)
             const int r = m / WB, wb = m - r * WB;
             const int h = h0 - 3 + r, w = wb * 8 + px;
             const bool ok = m < NM && (RAG ? (unsigned)h < (unsigned)hv : (h >= 0 && h < H)) && w < W;
-            q[u][mi] = ok ? ldg_nc_u32(xin + ((size_t)h * W + w) * (GP ? kPix : C)) : 0u;
+            q[u][mi] = ok ? ldg_nc_u32(xin + ((size_t)h * W + w) * C) : 0u;
           }
         }
 #pragma unroll
@@ -194,7 +167,6 @@ __global__ void __launch_bounds__(THREADS, 2)
     }
     ptx::fence_proxy_async_smem();
     __syncthreads();
-    DWTC_MARK(tr_stage);
 
 #pragma unroll 1
     for (int half = 0; half < NHALF; ++half) {
@@ -244,7 +216,6 @@ __global__ void __launch_bounds__(THREADS, 2)
       ptx::mbar_wait(d_full, dphase);
       dphase ^= 1;
       ptx::tc_fence_after();
-      DWTC_MARK(tr_mma);
       {
         const int q4 = warp & 3, side = warp >> 2;          // TMEM lane quadrant; which 16 accumulator columns
         const int m = q4 * 16 + lane;                        // M = 64: row m sits in lane (m / 16) * 32 + m % 16
@@ -255,9 +226,6 @@ __global__ void __launch_bounds__(THREADS, 2)
 #pragma unroll
         for (int c = 0; c < CG; ++c) bs[c] = bias[c0 + c];
         bf16* vrow = v + (((size_t)n * H + (row_ok ? h : 0)) * W) * C + c0;
-        // GP: results are staged in the (now idle) band slots as [row][pixel] 16-byte pieces, rotated by the row index
-        // so that the 16 rows a warp writes at once hit different banks, and leave as contiguous runs afterwards
-        uint8_t* stg_row = smem + OFF_BAND + m * (HW * 16);
 #pragma unroll
         for (int b = 0; b < 2; ++b) {
           const int col0 = side * 16 + b * 8;                // accumulator columns [col0, col0 + 8)
@@ -277,62 +245,30 @@ __global__ void __launch_bounds__(THREADS, 2)
               o.y = Pair<bf16>::pack(__uint_as_float(r[2][j]) + bs[2], __uint_as_float(r[3][j]) + bs[3]);
               o.z = Pair<bf16>::pack(__uint_as_float(r[4][j]) + bs[4], __uint_as_float(r[5][j]) + bs[5]);
               o.w = Pair<bf16>::pack(__uint_as_float(r[6][j]) + bs[6], __uint_as_float(r[7][j]) + bs[7]);
-              if (GP) {
-                const int p = half == 0 ? col : col - 4;     // pixel within the half row
-                int rot = p + m;
-                rot -= rot >= HW ? HW : 0;
-                rot -= rot >= HW ? HW : 0;
-                rot -= rot >= HW ? HW : 0;
-                *reinterpret_cast<uint4*>(stg_row + rot * 16) = o;
-              } else {
-                *reinterpret_cast<uint4*>(vrow + (size_t)w * C) = o;
-              }
+              *reinterpret_cast<uint4*>(vrow + (size_t)w * C) = o;
             }
           }
         }
       }
-      if (GP) {
-        ptx::tc_fence_before();
-        __syncthreads();
-        // coalesced copy-out: piece id -> (row, pixel); a half row is HW * 16 contiguous bytes of the group's plane
-        const size_t mtot = ((size_t)n_clips * H * W + 127) / 128 * 128;   // plane stride: rows rounded up to 128
-        bf16* vg = v + ((size_t)g * mtot + ((size_t)n * H + h0) * W + (half == 0 ? 0 : 28)) * 8;
-        const int rows = min(TR, H - h0);
-        for (int id = tid; id < rows * HW; id += THREADS) {
-          const int row = id / HW, p = id - row * HW;
-          int rot = p + row;
-          rot -= rot >= HW ? HW : 0;
-          rot -= rot >= HW ? HW : 0;
-          rot -= rot >= HW ? HW : 0;
-          const uint4 o = *reinterpret_cast<const uint4*>(smem + OFF_BAND + row * (HW * 16) + rot * 16);
-          *reinterpret_cast<uint4*>(vg + ((size_t)row * W + p) * 8) = o;
-        }
-        __syncthreads();
-        // the band slots must be all-zero off the diagonals again before the builders come back
-        for (int i = tid; i < (TR * HW * 16 + 15) / 16; i += THREADS)
-          reinterpret_cast<uint4*>(smem + OFF_BAND)[i] = make_uint4(0, 0, 0, 0);
-        ptx::fence_proxy_async_smem();
-      }
       ptx::tc_fence_before();
       __syncthreads();                  // accumulators drained (next half / unit overwrites them); A tiles free after the last half
       ptx::tc_fence_after();
-      DWTC_MARK(tr_epi);
     }
   }
-#ifdef ACX_ENABLE_TRACE
-  if (trace && tid == 0 && blockIdx.x < 4) {
-    long long* o = trace + blockIdx.x * 8;
-    o[0] = tr_units, o[1] = tr_taps, o[2] = tr_stage, o[3] = tr_mma, o[4] = tr_epi;
-  }
-#endif
   if (warp == 0) ptx::tmem_dealloc(tmem, 256);
 }
 
 // =====================================================================================================================
 // v3 (group-planar only): ONE persistent CTA per SM that owns a FIXED 8-channel group.
+// Group-planar activations: x and v are [C/8][Mp][8] (M = clips * H * W pixels, Mp = M rounded up to 128 = the plane
+// stride; every 16-byte group of 8 channels is a plane).  With NHWC tensors a unit's 16-byte pieces sit 2 C bytes apart:
+// each costs the LSU a 32-byte sector request and the staging / write-out phases of the kernel above ran at ~5 useful
+// B/clk/SM (24 k + 8 k of a unit's 54 k cycles, in-kernel clock trace, commit 17b9d13; TMA gathers the same pieces at
+// 14 B/clk/SM, tools/ubench/tma_gather.cu).  In the planar layout a unit's image rows are contiguous: fragment loads are
+// full 128-byte lines and the results leave as contiguous runs.
 //   * the 8 x 7 band matrices of its channels (112 KB) are built once and stay in shared memory: no per-channel band
-//     build / hand-off in steady state (in-kernel clock traces of the kernel above: ~1.0 k cycles per channel against
-//     0.34 k of MMA time, bands + MMA were 44 % of a unit);
+//     build / hand-off in steady state (in-kernel clock traces of the kernel above, commit 17b9d13: ~1.0 k cycles per
+//     channel against 0.34 k of MMA time, bands + MMA were 44 % of a unit);
 //   * the work item is a (clip, 63-row tile, half row): its A tile holds only the 32-column K window of that half
 //     (64-byte rows, SWIZZLE_64B, 36.5 KB for 8 channels), so TWO of them fit and the accumulators of two items fit the
 //     512 TMEM columns -- loaders, the MMA thread and the write-out warps work on three different items at once:
@@ -363,8 +299,7 @@ static_assert(SMEM_BYTES <= 227 * 1024, "smem budget");
 template <int W, bool RAG = false>
 __global__ void __launch_bounds__(THREADS, 1)
     dwconv_tc3_kernel(const bf16* __restrict__ x, const bf16* __restrict__ taps /*[49][C]*/, const float* __restrict__ bias,
-                      bf16* __restrict__ v, int n_clips, int H, int C, long long* __restrict__ trace,
-                      const int32_t* __restrict__ valid) {
+                      bf16* __restrict__ v, int n_clips, int H, int C, const int32_t* __restrict__ valid) {
   constexpr int NHALF = W > 32 ? 2 : 1;
   constexpr int HW = NHALF == 2 ? 28 : W;
   // W = 14: an item takes the rows of TWO clips side by side in one 32-column K window -- clip A in columns 0..13, three
@@ -373,14 +308,6 @@ __global__ void __launch_bounds__(THREADS, 1)
   constexpr bool PAIR = W == 14;
   constexpr int KS = 2;                         // K steps per (channel, dy)
   constexpr int NMI = 4;                        // 8-pixel blocks per A row
-#ifdef ACX_ENABLE_TRACE
-  long long tr_wait = 0, tr_wait2 = 0, tr_work = 0, tr_t = 0, tr_n = 0;
-#define V3_T0() do { if (trace) tr_t = clock64(); } while (0)
-#define V3_ACC(acc) do { if (trace) { const long long t_ = clock64(); acc += t_ - tr_t; tr_t = t_; } } while (0)
-#else
-#define V3_T0() do { } while (0)
-#define V3_ACC(acc) do { } while (0)
-#endif
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const uint32_t s_base = ptx::smem_u32(smem);
@@ -444,11 +371,8 @@ __global__ void __launch_bounds__(THREADS, 1)
       for (int item = rank; item < items; item += ng, ++it) {
         const int buf = it & 1;
         const uint32_t par = (it >> 1) & 1;
-        V3_T0();
         ptx::mbar_wait(&a_full[buf], par);
-        V3_ACC(tr_wait);
         ptx::mbar_wait(&d_empty[buf], par ^ 1);
-        V3_ACC(tr_wait2);
         ptx::tc_fence_after();
 #pragma unroll 1
         for (int c = 0; c < CG; ++c) {
@@ -463,17 +387,7 @@ __global__ void __launch_bounds__(THREADS, 1)
         }
         ptx::umma_commit(&a_empty[buf]);
         ptx::umma_commit(&d_full[buf]);
-        V3_ACC(tr_work);
-#ifdef ACX_ENABLE_TRACE
-        ++tr_n;
-#endif
       }
-#ifdef ACX_ENABLE_TRACE
-      if (trace && blockIdx.x < 2) {
-        long long* o = trace + blockIdx.x * 16;
-        o[0] = tr_n, o[1] = tr_wait, o[2] = tr_wait2, o[3] = tr_work;
-      }
-#endif
     }
   } else if (warp >= 1 && warp <= NLOAD) {
     // ===================== loaders ==========================================================================================
@@ -486,9 +400,7 @@ __global__ void __launch_bounds__(THREADS, 1)
       const int half = item % NHALF, t = (item / NHALF) % tiles, n = (item / (NHALF * tiles)) * (PAIR ? 2 : 1);
       const int h0 = t * TR, kw0 = half ? 24 : 0;
       const int buf = it & 1;
-      V3_T0();
       ptx::mbar_wait(&a_empty[buf], ((it >> 1) & 1) ^ 1);
-      V3_ACC(tr_wait);
       const bf16* xin = xg + ((size_t)n * H * W + kw0) * 8;
       const bool b_ok = PAIR && n + 1 < n_clips;        // the pair's second clip exists
       const int hv_a = RAG ? min(max(__ldg(valid + n), 0), H) : H;
@@ -531,14 +443,7 @@ __global__ void __launch_bounds__(THREADS, 1)
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(&a_full[buf]);
-      V3_ACC(tr_work);
     }
-#ifdef ACX_ENABLE_TRACE
-    if (trace && blockIdx.x < 2 && warp == 1 && lane == 0) {
-      long long* o = trace + blockIdx.x * 16;
-      o[4] = tr_wait, o[5] = tr_work;
-    }
-#endif
   } else if (warp >= 8) {
     // ===================== write-out =========================================================================================
     // An M = 64 accumulator occupies lanes 0..15 of each 32-lane TMEM quadrant, so the 32x32b load shape would move
@@ -559,9 +464,7 @@ __global__ void __launch_bounds__(THREADS, 1)
       const int half = item % NHALF, t = (item / NHALF) % tiles, n = (item / (NHALF * tiles)) * (PAIR ? 2 : 1);
       const int h0 = t * TR;
       const int buf = it & 1;
-      V3_T0();
       ptx::mbar_wait(&d_full[buf], (it >> 1) & 1);
-      V3_ACC(tr_wait);
       ptx::tc_fence_after();
       uint32_t r[2][CG][4];
 #pragma unroll
@@ -616,15 +519,8 @@ __global__ void __launch_bounds__(THREADS, 1)
                      : "memory");
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
       }
-      V3_ACC(tr_work);
     }
     asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");    // all stores complete before the CTA exits
-#ifdef ACX_ENABLE_TRACE
-    if (trace && blockIdx.x < 2 && warp == 8 && lane == 0) {
-      long long* o = trace + blockIdx.x * 16;
-      o[6] = tr_wait, o[7] = tr_work;
-    }
-#endif
   }
   ptx::tc_fence_before();
   __syncthreads();
@@ -643,30 +539,21 @@ static int launch(const void* x, const void* taps, const float* bias, void* v, i
   const long long work = (long long)G * (W == 14 ? (B + 1) / 2 : B) * ceil_div(H, TR) * (W > 32 ? 2 : 1);
   const int sms = sm_count();
   const int grid = work < sms ? (int)work : sms;       // >= G whenever there is at least one item per group
-  long long* trace = nullptr;
-#ifdef ACX_ENABLE_TRACE
-  if (getenv("ACX_DWTC_TRACE")) trace = reinterpret_cast<long long*>(strtoull(getenv("ACX_DWTC_TRACE"), nullptr, 0));
-#endif
   ACX_CUDA(launch_pdl(kern, dim3(grid), dim3(THREADS), SMEM_BYTES, st, 1, PDL_DWTC, reinterpret_cast<const bf16*>(x),
-                      reinterpret_cast<const bf16*>(taps), bias, reinterpret_cast<bf16*>(v), B, H, C, trace, valid));
+                      reinterpret_cast<const bf16*>(taps), bias, reinterpret_cast<bf16*>(v), B, H, C, valid));
   return ACX_OK;
 }
 }  // namespace v3
 
-template <int W, bool GP, bool RAG>
+template <int W, bool RAG>
 static int launch(const void* x, const void* taps, const float* bias, void* v, int B, int H, int C, const int32_t* valid,
                   cudaStream_t st) {
-  auto kern = dwconv_tc_kernel<W, GP, RAG>;
+  auto kern = dwconv_tc_kernel<W, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM_BYTES);
   const int units = B * ceil_div(H, TR) * (C / CG);
   const int grid = units < 2 * sm_count() ? units : 2 * sm_count();
-  // debug: ACX_DWTC_TRACE=<device pointer to 32 x int64> collects per-phase SM-clock sums of CTAs 0..3 (tools/time_dwtc.py)
-  long long* trace = nullptr;
-#ifdef ACX_ENABLE_TRACE
-  if (getenv("ACX_DWTC_TRACE")) trace = reinterpret_cast<long long*>(strtoull(getenv("ACX_DWTC_TRACE"), nullptr, 0));
-#endif
   kern<<<grid, THREADS, SMEM_BYTES, st>>>(reinterpret_cast<const bf16*>(x), reinterpret_cast<const bf16*>(taps), bias,
-                                          reinterpret_cast<bf16*>(v), B, H, C, trace, valid);
+                                          reinterpret_cast<bf16*>(v), B, H, C, valid);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }
@@ -763,10 +650,10 @@ static int dwconv_tc_impl(const void* x, const void* w, const float* bias, void*
             "dwconv_tc: x and v must be 16-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   switch (W) {
-    case 56: return dwtc::launch<56, false, RAG>(x, w, bias, v, B, H, C, valid, st);
-    case 28: return dwtc::launch<28, false, RAG>(x, w, bias, v, B, H, C, valid, st);
-    case 14: return dwtc::launch<14, false, RAG>(x, w, bias, v, B, H, C, valid, st);
-    case 7: return dwtc::launch<7, false, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 56: return dwtc::launch<56, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 28: return dwtc::launch<28, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 14: return dwtc::launch<14, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 7: return dwtc::launch<7, RAG>(x, w, bias, v, B, H, C, valid, st);
     default:
       set_error("dwconv_tc: W=%d not supported (the ConvNeXt stages are 56 / 28 / 14 / 7 wide)", W);
       return ACX_ERR_UNSUPPORTED;
@@ -795,14 +682,9 @@ static int dwconv_tc_gp_impl(const void* x, const void* w, const float* bias, vo
   ACX_CHECK(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(w)) & 15) == 0,
             ACX_ERR_ARG, "dwconv_tc_gp: x, v and w must be 16-byte aligned");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  static const bool use_v1 = getenv("ACX_DWTC_V1") != nullptr;      // the two-CTA-per-SM kernel, kept for A/B timing
   switch (W) {
-    case 56:
-      return use_v1 ? dwtc::launch<56, true, RAG>(x, w, bias, v, B, H, C, valid, st)
-                    : dwtc::v3::launch<56, RAG>(x, w, bias, v, B, H, C, valid, st);
-    case 28:
-      return use_v1 ? dwtc::launch<28, true, RAG>(x, w, bias, v, B, H, C, valid, st)
-                    : dwtc::v3::launch<28, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 56: return dwtc::v3::launch<56, RAG>(x, w, bias, v, B, H, C, valid, st);
+    case 28: return dwtc::v3::launch<28, RAG>(x, w, bias, v, B, H, C, valid, st);
     case 14: return dwtc::v3::launch<14, RAG>(x, w, bias, v, B, H, C, valid, st);
     default:
       set_error("dwconv_tc_gp: W=%d not supported (stages 0 - 2: 56 / 28 / 14)", W);

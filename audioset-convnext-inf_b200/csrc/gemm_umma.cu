@@ -401,17 +401,16 @@ static int dispatch_bn(const CUtensorMap& tmA, const void* W, const GemmArgs& g,
     }
   }
   ACX_CHECK(bn != 0, ACX_ERR_UNSUPPORTED, "gemm_bf16: N=%d is not a multiple of 96/128/192/256", g.N);
-  static const bool pair_ok = getenv("ACX_GEMM_PAIR") == nullptr || atoi(getenv("ACX_GEMM_PAIR")) != 0;
   const long long pairs = sm_count() / 2;     // 74 on a B200
   // Wave quantisation: a persistent grid of `pairs` CTA pairs runs ceil(tiles / pairs) rounds of BN-wide tiles, so when both
   // 256 and 192 divide N the cheaper of  rounds(BN) * BN  wins (ties keep 256: fewer A re-reads).  Stage 3 at 64 clips:
   // N = 768 is 165 tiles = 3 rounds at BN 256 (2.2 needed) but 220 tiles = 3 rounds at BN 192 -- a quarter less work.
-  if (pair_ok && bn == 256 && g.N % 192 == 0) {
+  if (bn == 256 && g.N % 192 == 0) {
     const long long mt = ceil_div(g.M, 256);
     const long long r256 = (mt * (g.N / 256) + pairs - 1) / pairs * 256, r192 = (mt * (g.N / 192) + pairs - 1) / pairs * 192;
     if (mt * (g.N / 192) >= pairs && r192 < r256) bn = 192;
   }
-  const bool pair = pair_ok && (bn == 256 || bn == 192) && (long long)ceil_div(g.M, 256) * (g.N / bn) >= pairs;
+  const bool pair = (bn == 256 || bn == 192) && (long long)ceil_div(g.M, 256) * (g.N / bn) >= pairs;
   CUtensorMap tmB;
   int rc = make_tmap_2d_bf16(&tmB, W, (uint64_t)g.K, (uint64_t)g.N, (uint64_t)g.K * 2, 64,
                              (uint32_t)(pair ? bn / 2 : bn));
@@ -464,9 +463,8 @@ static int gemm_bf16_impl(const void* A, const void* W, void* out, int M, int N,
   g.a_gp = a_gp;
   g.stats = reinterpret_cast<const float2*>(stats);
   g.ln_s = ln_s;
-  static const bool rev_ok = getenv("ACX_GEMM_REVERSE") == nullptr || atoi(getenv("ACX_GEMM_REVERSE")) != 0;
   // the pwconv2 GEMMs (residual epilogue) consume what pwconv1 has just written front to back
-  g.reverse = rev_ok && epilogue == ACX_EPI_BIAS_SCALE_RESID && (size_t)M * K * 2 > (size_t)96 << 20;
+  g.reverse = epilogue == ACX_EPI_BIAS_SCALE_RESID && (size_t)M * K * 2 > (size_t)96 << 20;
   CUtensorMap tmA;
   int rc = a_gp ? make_tmap_gp_bf16(&tmA, A, (uint64_t)M, (uint64_t)K / 8, 128, 8)
                 : make_tmap_2d_bf16(&tmA, A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, 64, 128);

@@ -108,14 +108,15 @@ __global__ void power_mel_log_kernel(const float* __restrict__ spec, int ld_spec
 //  * LayerNorm statistics need no cross-thread traffic at all;
 //  * the warp's 32 x 96 outputs (contiguous in HBM) are transposed through padded smem and stored coalesced.
 // =============================================================================================
+// fp32 mode only (bf16 mode runs the tensor-core stem, stem_umma.cu).
 // RAG: clip b has valid[b] frames (clamped to [0, Tn]); later rows are read as the conv's zero padding.
-template <typename T, bool RAG = false>
+template <bool RAG = false>
 __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ logmel, const float* __restrict__ w,
                                                    const float* __restrict__ bias, const float* __restrict__ ln_w,
-                                                   const float* __restrict__ ln_b, T* __restrict__ out, int B,
+                                                   const float* __restrict__ ln_b, float* __restrict__ out, int B,
                                                    int Tn, int n_mels, int H0, int W0, const int32_t* __restrict__ valid) {
   constexpr int CO = 96;
-  constexpr int ROW_BYTES = CO * (int)sizeof(T);       // 192 (bf16) / 384 (fp32)
+  constexpr int ROW_BYTES = CO * 4;                    // 384
   constexpr int ROW_PITCH = ROW_BYTES + 16;            // +16 B: conflict-free 16-byte row writes
   extern __shared__ __align__(16) uint8_t ssm[];
   float* sw = reinterpret_cast<float*>(ssm);           // [16][96] taps, then bias / ln_w / ln_b [3][96]
@@ -180,7 +181,7 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ log
     sq = fmaf(acc[c].y, acc[c].y, sq);
   }
   const float rstd = rsqrtf(sq * (1.0f / CO) + 1e-6f);
-  // normalise, convert, and write this pixel's row into the warp tile
+  // normalise and write this pixel's row into the warp tile
   uint8_t* myrow = stile + lane * ROW_PITCH;
 #pragma unroll
   for (int c = 0; c < CO / 2; c += 2) {
@@ -188,11 +189,7 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ log
     const float4 h4 = *reinterpret_cast<const float4*>(sw + 18 * CO + 2 * c);
     const float o0 = acc[c].x * rstd * g4.x + h4.x, o1 = acc[c].y * rstd * g4.y + h4.y;
     const float o2 = acc[c + 1].x * rstd * g4.z + h4.z, o3 = acc[c + 1].y * rstd * g4.w + h4.w;
-    if (sizeof(T) == 2) {
-      *reinterpret_cast<uint2*>(myrow + c * 4) = make_uint2(Pair<bf16>::pack(o0, o1), Pair<bf16>::pack(o2, o3));
-    } else {
-      *reinterpret_cast<float4*>(myrow + c * 8) = make_float4(o0, o1, o2, o3);
-    }
+    *reinterpret_cast<float4*>(myrow + c * 8) = make_float4(o0, o1, o2, o3);
   }
   __syncwarp();
   // coalesced copy-out: the warp's 32 rows are contiguous in global memory
@@ -210,8 +207,8 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ log
 // depthwise 7x7 + LayerNorm (reference convnext.py:76-78).
 // Thread = one channel pair x a strip of 7 output pixels along W x R = 4 consecutive output rows.
 //  * the two channels of a pair are processed by ONE packed fp32x2 FMA (FFMA2, new on sm_100);
-//  * the R+6 input rows slide through registers: each row is loaded ONCE (13 channel-pair words, prefetched one
-//    row ahead) and feeds up to 4 output rows -> 3.25 loads + 6.5 unpack ops per 98 FMAs;
+//  * the R+6 input rows slide through registers: each row is loaded ONCE (13 channel-pair words, prefetched two
+//    rows ahead) and feeds up to 4 output rows -> 3.25 loads + 6.5 unpack ops per 98 FMAs;
 //  * the 49 taps of every channel live in shared memory as fp32 pairs (one conflict-free LDS.64 per 14 FMAs),
 //    which keeps the kernel at ~110 registers instead of 168-195 when the taps sat in registers;
 //  * LayerNorm statistics are fp32; the R*7 per-pixel partial sums are reduce-scattered inside each 16-lane group
@@ -247,7 +244,7 @@ __device__ __forceinline__ int slot_of_lane(int lane) {
 constexpr int dw_min_blocks(int threads) { return threads <= 96 ? 5 : (threads <= 192 ? 2 : 1); }
 
 // RAG: clip b has valid[b] rows (clamped to [0, H]); rows past it are read as the conv's zero padding and not written.
-template <typename T, int C, int S, int PF, bool RAG = false>
+template <typename T, int C, int S, bool RAG = false>
 __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
     dwconv_ln_kernel(const T* __restrict__ x, const T* __restrict__ w, const float* __restrict__ bias,
                      const float* __restrict__ ln_w, const float* __restrict__ ln_b, T* __restrict__ y, int H,
@@ -294,6 +291,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
   };
   // The first PF input rows are requested BEFORE the tap fill so that their L2/HBM latency overlaps the fill's own
   // round trip and barrier (ncu: the serial prologue was ~30 % of a block's lifetime).
+  constexpr int PF = 2;             // rows in flight ahead of the one being used
   static_assert((R + 6) % PF == 0, "prefetch ring must divide the row count");
   pdl_trigger();       // programmatic dependent launch (common.cuh); x is the previous kernel's output
   pdl_wait();
@@ -922,23 +920,21 @@ __global__ void __launch_bounds__(256)
 }
 
 // ---- launch helpers ---------------------------------------------------------------------------
-template <typename T, int C, int S, int PF = 2, bool RAG = false>
+template <typename T, int C, int S, bool RAG = false>
 static int launch_dwconv(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
                          void* y, int B, int H, int W, const int32_t* valid, cudaStream_t st) {
   const int strips = W / 7;
   ACX_CHECK(strips % S == 0, ACX_ERR_ARG, "dwconv_ln: W/7=%d not a multiple of strips-per-block %d", strips, S);
   constexpr int NV = sizeof(T) == 4 ? 32 : 64;
   constexpr int SMEM = (2 * 49 * (C / 2) + S * (C / 32) * NV + S * NV) * (int)sizeof(float);
-  auto kern = dwconv_ln_kernel<T, C, S, PF, RAG>;
+  auto kern = dwconv_ln_kernel<T, C, S, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM);
   const int row_groups = ceil_div(H, DW_R);
   // Row groups per block.  With the first input rows requested ahead of the tap fill (and the next group's rows
   // ahead of the LayerNorm phase) one group per block is fastest everywhere except the tiny stage-4 maps, where the
   // 150 KB tap fill dominates (measured, 64 clips: C=768 0.137 / 0.133 / 0.129 ms at 1 / 2 / 4 groups; C=384
-  // 0.688 / 0.703 / 0.779; C=96 0.783 / 0.807 / 0.829).  ACX_DW_GPB overrides for experiments.
-  static const int gpb_env = [] { const char* e = getenv("ACX_DW_GPB"); return e ? atoi(e) : 0; }();
-  int gpb = (C >= 768 && row_groups >= 4) ? 4 : 1;
-  if (gpb_env > 0) gpb = gpb_env < row_groups ? gpb_env : row_groups;
+  // 0.688 / 0.703 / 0.779; C=96 0.783 / 0.807 / 0.829).
+  const int gpb = (C >= 768 && row_groups >= 4) ? 4 : 1;
   dim3 grid(strips / S, ceil_div(row_groups, gpb), B);
   ACX_CUDA(launch_pdl(kern, grid, dim3(S * C / 2), SMEM, st, 1, PDL_SMALL, reinterpret_cast<const T*>(x), reinterpret_cast<const T*>(w), bias,
                       ln_w, ln_b, reinterpret_cast<T*>(y), H, W, gpb, valid));
@@ -949,20 +945,15 @@ template <typename T, bool RAG>
 static int dispatch_dwconv(const void* x, const void* w, const float* bias, const float* ln_w, const float* ln_b,
                            void* y, int B, int H, int W, int C, const int32_t* valid, cudaStream_t st) {
   const int strips = W / 7;
-  // A/B switches (development only): ACX_DW_PF=1 -> one-row prefetch, ACX_DW_NARROW=1 -> half-width blocks
-  static const bool pf1 = [] { const char* e = getenv("ACX_DW_PF"); return e && e[0] == '1'; }();
-  static const bool narrow = [] { const char* e = getenv("ACX_DW_NARROW"); return e && e[0] == '1'; }();
-#define ACX_DW_LAUNCH(CC, SS) \
-  (pf1 ? launch_dwconv<T, CC, SS, 1, RAG>(x, w, bias, ln_w, ln_b, y, B, H, W, valid, st) \
-       : launch_dwconv<T, CC, SS, 2, RAG>(x, w, bias, ln_w, ln_b, y, B, H, W, valid, st))
+#define ACX_DW_LAUNCH(CC, SS) launch_dwconv<T, CC, SS, RAG>(x, w, bias, ln_w, ln_b, y, B, H, W, valid, st)
   switch (C) {
     case 96:
-      if (strips % 4 == 0 && !narrow) return ACX_DW_LAUNCH(96, 4);
+      if (strips % 4 == 0) return ACX_DW_LAUNCH(96, 4);
       if (strips % 2 == 0) return ACX_DW_LAUNCH(96, 2);
       set_error("dwconv_ln: C=96 needs an even number of 7-pixel strips per row (W=%d)", W);
       return ACX_ERR_UNSUPPORTED;
     case 192:
-      if (strips % 2 == 0 && !narrow) return ACX_DW_LAUNCH(192, 2);
+      if (strips % 2 == 0) return ACX_DW_LAUNCH(192, 2);
       return ACX_DW_LAUNCH(192, 1);
     case 384:
       return ACX_DW_LAUNCH(384, 1);
@@ -1075,21 +1066,13 @@ static int stem_impl(const float* logmel, const float* w, const float* bias, con
   const long long total = (long long)B * H0 * W0;
   const int blocks = (int)((total + 127) / 128);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  // bf16 mode: tensor-core stem (stem_umma.cu); ACX_STEM=simt selects the CUDA-core kernel for A/B timing
-  static const bool stem_simt = [] { const char* e = getenv("ACX_STEM"); return e && e[0] == 's'; }();
-  if (act_dtype == ACX_BF16 && !stem_simt)
-    return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 0, valid, st);
-  if (act_dtype == ACX_BF16) {
-    const int smem = 19 * 96 * 4 + 4 * 32 * (96 * 2 + 16);
-    auto kern = valid ? stem_kernel<bf16, true> : stem_kernel<bf16>;
-    kern<<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<bf16*>(out), B, T, n_mels, H0, W0, valid);
-  } else {
-    const int smem = 19 * 96 * 4 + 4 * 32 * (96 * 4 + 16);
-    auto kern = valid ? stem_kernel<float, true> : stem_kernel<float>;
-    if (valid) ACX_SET_MAX_SMEM((stem_kernel<float, true>), smem);
-    else ACX_SET_MAX_SMEM(stem_kernel<float>, smem);
-    kern<<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<float*>(out), B, T, n_mels, H0, W0, valid);
-  }
+  // bf16 mode: tensor-core stem (stem_umma.cu)
+  if (act_dtype == ACX_BF16) return launch_stem_umma(logmel, w, bias, ln_w, ln_b, out, B, T, n_mels, 0, valid, st);
+  const int smem = 19 * 96 * 4 + 4 * 32 * (96 * 4 + 16);
+  auto kern = valid ? stem_kernel<true> : stem_kernel<>;
+  if (valid) ACX_SET_MAX_SMEM(stem_kernel<true>, smem);
+  else ACX_SET_MAX_SMEM(stem_kernel<>, smem);
+  kern<<<blocks, 128, smem, st>>>(logmel, w, bias, ln_w, ln_b, reinterpret_cast<float*>(out), B, T, n_mels, H0, W0, valid);
   ACX_CUDA(cudaGetLastError());
   return ACX_OK;
 }

@@ -34,7 +34,6 @@ struct MlpArgs {
   const float* ln_s;  // FOLD mode: s_j = sum_c W1'[j, c] of the LayerNorm-folded weights W1' = W1 diag(ln_w) (w1 / b1 then
                       // ARE W1' and b1 + W1 ln_b): the kernel only computes per-row statistics of the y tile and applies
                       // the LayerNorm as a rank-1 correction in the GELU epilogue (common.cuh, LnFold)
-  unsigned long long* trace;   // optional [16 tiles][2 roles][32 events] SM-clock stamps of CTA 0 (tools/trace_mlp.py)
 };
 
 // LayerNorm of one 128-row operand tile in place in shared memory: thread = row, `chunk(j)` = address of the row's j-th
@@ -555,7 +554,7 @@ __global__ void __launch_bounds__(512, 1)
 // K = 96 is split 64 + 32: the first 64 columns use 128B-swizzled tiles, the 32-column tail 64B-swizzled tiles, so no
 // shared memory is spent on zero padding (W1 48 + 24 KB, W2 72 KB, y tile 16 + 8 KB, hidden buffers 2 x 16 KB).
 //
-// Schedule (second version, driven by clock traces -- tools/trace_mlp.py -- and an ncu source-level capture):
+// Schedule (second version, driven by in-kernel clock traces -- commit 17b9d13 -- and an ncu source-level capture):
 //   * the 384 hidden columns are six chunks of 64; epilogue-1 group 0 (warps 4-7) takes the even chunks, group 1
 //     (warps 8-11) the odd ones, each into its OWN 128 x 64 hidden buffer (one GEMM2 k-block);
 //   * TMEM: D2 x 2 (columns 0 and 128: epilogue-2 of tile i overlaps GEMM2 of tile i+1), D1 x 4 (64 columns each,
@@ -564,11 +563,6 @@ __global__ void __launch_bounds__(512, 1)
 //     chunks ahead across tile boundaries, GEMM2 is issued as soon as its hidden buffer is full;
 //   * the GELU is software-pipelined in 16-column quarters (common.cuh: gelu_stage_ta4 / gelu_stage_c8_twice_bf16).
 // =====================================================================================================================
-#define ACX_TRACE(role, ev)                                                                    \
-  do {                                                                                         \
-    if (a.trace && blockIdx.x == 0 && it < 16) a.trace[(it * 2 + (role)) * 32 + (ev)] = clock64(); \
-  } while (0)
-
 struct Mlp96 {
   static constexpr int C = 96, HD = 384, BM = 128, NH = 64, NC = 6;   // 64-column hidden chunks
   static constexpr int OFF_W1M = 0;                        // 3 x [128 rows x 64 k]  SW128   48 KB
@@ -751,7 +745,6 @@ __global__ void __launch_bounds__(512, 1)
       auto gemm2 = [&](uint32_t g, int h, int it) {
         const int hb = g & 1;
         ptx::mbar_wait(&h_full[hb], (g >> 1) & 1);
-        ACX_TRACE(0, 2 * h);
         if (h == 0) ptx::mbar_wait(&d2_empty[it & 1], ((it >> 1) & 1) ^ 1);
         ptx::tc_fence_after();
         const uint32_t d2 = tmem_base + Cfg::D2_COL + (it & 1) * Cfg::D2_STRIDE;
@@ -761,7 +754,6 @@ __global__ void __launch_bounds__(512, 1)
         for (int k = 0; k < 4; ++k) ptx::umma_bf16(d2, da + 2 * k, db + 2 * k, idesc2, (h | k) != 0 ? 1u : 0u);
         ptx::umma_commit(&h_empty[hb]);
         if (h == Cfg::NC - 1) ptx::umma_commit(&d2_full[it & 1]);
-        ACX_TRACE(0, 2 * h + 1);
       };
       // GEMM1 look-ahead = ring depth: chunk g+4 reuses chunk g's buffer, which the epilogue released half-way
       // through chunk g, i.e. before the h_full(g) that gemm2(g) has just waited for
@@ -799,7 +791,6 @@ __global__ void __launch_bounds__(512, 1)
     const int group = ew >> 2;
     const int row_in_tile = quad * 32 + lane;
     const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
-    const bool tr = (warp == 4 && lane == 0);
     LnFold fold{0ull, 0ull, ptx::smem_u32(sb1), ptx::smem_u32(ss1)};
     int it = 0;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
@@ -813,10 +804,8 @@ __global__ void __launch_bounds__(512, 1)
         const int h = 2 * hc + group;
         const uint32_t gc = (uint32_t)Cfg::NC * it + h;
         const int buf = gc & 3;
-        if (tr) ACX_TRACE(1, 4 * hc);
         ptx::mbar_wait(&d1_full[buf], (gc >> 2) & 1);
         ptx::tc_fence_after();
-        if (tr) ACX_TRACE(1, 4 * hc + 1);
         const uint32_t t0 = lane_base + Cfg::D1_COL + buf * Cfg::NH;
         const uint32_t bias = ptx::smem_u32(sb1 + h * Cfg::NH);
         const uint32_t hrow = ptx::smem_u32(smem + Cfg::OFF_H + group * 16384 + row_in_tile * 128);
@@ -849,7 +838,6 @@ __global__ void __launch_bounds__(512, 1)
         ptx::tc_fence_before();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&d1_empty[buf]);          // all of this warp's D1 reads landed: free for GEMM1(g+4)
-        if (tr) ACX_TRACE(1, 4 * hc + 2);
         gelu_stage_ta4<true, true, FOLD>(gB, gA, raA, bias + 128, fold);                       // T(1) + A(2)
         gelu_stage_ta4<true, true, FOLD>(gB + 4, gA + 4, raA + 8, bias + 160, fold);
         gelu_stage_c8_twice_bf16(gB, pk);                                          // C(1)
@@ -865,7 +853,6 @@ __global__ void __launch_bounds__(512, 1)
         ptx::fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&h_full[group]);
-        if (tr) ACX_TRACE(1, 4 * hc + 3);
       }
     }
   } else if (warp >= 12) {
@@ -878,7 +865,6 @@ __global__ void __launch_bounds__(512, 1)
     const int quad = warp & 3;
     const uint32_t lane_base = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
     uint8_t* stg = smem + Cfg::OFF_STG + quad * 4096;            // 2 x 2 KB ping-pong tiles
-    const bool tr = (warp == 12 && lane == 0);
     const int sw64 = (lane >> 1) & 3;
     const int ld_piece = lane & 3, ld_row = lane >> 2;
     // LayerNorm mode: this warp normalises its 32 rows of tile `j` in place as soon as the tile has landed (columns
@@ -903,15 +889,9 @@ __global__ void __launch_bounds__(512, 1)
       const int r = quad * 32 + lane;
       uint8_t* am = smem + Cfg::OFF_AM + r * 128;
       uint8_t* at = smem + Cfg::OFF_AT + r * 64;
-#ifdef ACX_AB_NO_STATS      /* A/B experiment: folded epilogue without the statistics pass */
-      sstat[(j & 1) * Cfg::BM + r] = make_float2(1.f, 0.f);
-      (void)am;
-      (void)at;
-#else
       sstat[(j & 1) * Cfg::BM + r] =
           GP ? ln_row_stats_smem<C>([&](int ch) { return smem + Cfg::OFF_AM + ch * 2048 + r * 16; })
              : ln_row_stats_smem<C>([&](int ch) { return ch < 8 ? am + ((ch ^ (r & 7)) << 4) : at + (((ch - 8) ^ ((r >> 1) & 3)) << 4); });
-#endif
       __syncwarp();
       if (lane == 0) {
         ptx::mbar_arrive(a_ready);
@@ -943,7 +923,6 @@ __global__ void __launch_bounds__(512, 1)
       if (lane == 0) ptx::tma_store_wait_read<0>();              // previous tile's stores have read both tiles
       __syncwarp();
       fetch_resid(0);
-      if (tr) ACX_TRACE(1, 12);
       ptx::mbar_wait(&d2_full[it & 1], (it >> 1) & 1);
       ptx::tc_fence_after();
 #pragma unroll
@@ -968,7 +947,6 @@ __global__ void __launch_bounds__(512, 1)
           ptx::tc_fence_before();
           __syncwarp();
           if (lane == 0) ptx::mbar_arrive(&d2_empty[it & 1]);   // this D2 buffer is free for tile i+2's GEMM2
-          if (tr) ACX_TRACE(1, 13);
         }
         __syncwarp();
         uint4 res[4];
@@ -1004,7 +982,6 @@ __global__ void __launch_bounds__(512, 1)
           ptx::tma_store_commit();
         }
       }
-      if (tr) ACX_TRACE(1, 15);
     }
     if (lane == 0) ptx::tma_store_wait_read<0>();
   }
@@ -1057,11 +1034,6 @@ static int launch_mlp96_resident(const void* y, void* x, const void* w1, const f
   a.ln_w = ln_w;
   a.ln_b = ln_b;
   a.ln_s = ln_s;
-#ifdef ACX_ENABLE_TRACE   // debug builds only (ACX_NVCC_EXTRA="-DACX_ENABLE_TRACE", tools/trace_mlp.py): a raw device pointer
-  a.trace = getenv("ACX_TRACE_PTR") ? reinterpret_cast<unsigned long long*>(strtoull(getenv("ACX_TRACE_PTR"), nullptr, 0)) : nullptr;
-#else                     // from the environment has no place in the production entry point
-  a.trace = nullptr;
-#endif
   const int grid = tiles < sms ? tiles : sms;
   auto kern = gp && ln_s ? mlp_fused96_kernel<true, true> : gp ? mlp_fused96_kernel<true, false> : mlp_fused96_kernel<false, false>;
   ACX_CUDA(launch_pdl(kern, dim3(grid), dim3(512), Cfg::SMEM_BYTES, st, 1, PDL_MLP, tmYm, tmYt, tmW1m, tmW1t, tmW2, tmOut, a));
@@ -1101,7 +1073,6 @@ static int launch_mlp(const void* y, void* x, const void* w1, const float* b1, c
   a.ln_w = ln_w;
   a.ln_b = ln_b;
   a.ln_s = ln_s;
-  a.trace = nullptr;
   const int grid = tiles < sms ? tiles : sms;
   auto kern = gp && ln_s ? mlp_fused_kernel<C, true, true> : gp ? mlp_fused_kernel<C, true, false> : mlp_fused_kernel<C, false, false>;
   ACX_CUDA(launch_pdl(kern, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, 1, PDL_MLP, tmY, tmW1, tmW2, tmOut, a));
@@ -1124,10 +1095,7 @@ static int mlp_fused_dispatch(const char* who, const void* y, void* x, const voi
             ACX_ERR_ARG, "%s: y, x, w1 and w2 must be 16-byte aligned", who);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   switch (C) {
-    case 96:
-      // weight-resident kernel; the streaming variant stays reachable for A/B timing (ACX_MLP96_STREAM=1)
-      if (getenv("ACX_MLP96_STREAM") && !gp) return launch_mlp<96>(y, x, w1, b1, w2, b2, gamma, M, ln_w, ln_b, nullptr, false, st);
-      return launch_mlp96_resident(y, x, w1, b1, w2, b2, gamma, M, ln_w, ln_b, ln_s, gp, st);
+    case 96: return launch_mlp96_resident(y, x, w1, b1, w2, b2, gamma, M, ln_w, ln_b, ln_s, gp, st);
     case 192: return launch_mlp<192>(y, x, w1, b1, w2, b2, gamma, M, ln_w, ln_b, ln_s, gp, st);
     default:
       set_error("%s: C=%d not supported (the fused kernel covers stages 0-1: C = 96, 192; wider stages exceed "

@@ -39,7 +39,7 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
 // Blocking wait.  try_wait carries a suspend-time hint, so a waiting thread SLEEPS in hardware until the phase flips
 // (or the hint expires) instead of spinning: a tight try_wait/branch loop in the single-thread producer / MMA warps
 // stole issue slots from the epilogue warps sharing their scheduler and slowed every epilogue step ~5x (in-kernel
-// clock trace, tools/trace_mlp.py).  Watchdog: a mis-programmed pipeline traps (sticky CUDA error) instead of hanging.
+// clock trace, commit 17b9d13).  Watchdog: a mis-programmed pipeline traps (sticky CUDA error) instead of hanging.
 #ifndef ACX_MBAR_TIMEOUT_NS
 #define ACX_MBAR_TIMEOUT_NS 20000000000ull      /* 20 s of wall time (globaltimer), not a spin count: under
                                                    compute-sanitizer try_wait returns early and kernels run ~100x

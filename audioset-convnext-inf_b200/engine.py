@@ -466,8 +466,8 @@ class Engine:
         w = self.w
         x, y, hid = ws["x"].data_ptr(), ws["y"].data_ptr(), ws["hid"].data_ptr()
         xgp = ws["xg"].data_ptr() if "xg" in ws else 0      # planar residual stream; trades places with y at a fused downsample
-        fused0 = self.mlp == "fused" and self.dwconv == "tc" and 0 in self.dwconv_tc_stages and self.gp
-        stem_gp = fused0 and os.environ.get("ACX_STEM", "") != "simt"     # the stem writes stage 0's planar layout itself
+        # the stem writes stage 0's planar layout itself
+        stem_gp = self.mlp == "fused" and self.dwconv == "tc" and 0 in self.dwconv_tc_stages and self.gp
         rT = rv[1] if rv else 0
         if stem_gp:
             self._call_v("stem", "acx_stem_gp", rT, ws["logmel"].data_ptr(), w.stem_w.data_ptr(), w.stem_b.data_ptr(),

@@ -9,9 +9,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from audioset_convnext_inf_b200 import _native as N  # noqa: E402
 
 DEV = "cuda:0"
-TRACE = torch.zeros(32, dtype=torch.int64, device=DEV) if os.environ.get("ACX_NVCC_EXTRA", "").find("ACX_ENABLE_TRACE") >= 0 else None
-if TRACE is not None:
-    os.environ["ACX_DWTC_TRACE"] = str(TRACE.data_ptr())
 st = lambda: torch.cuda.current_stream().cuda_stream  # noqa: E731
 B = 64
 for stage, (C, H, W) in enumerate([(96, 252, 56), (192, 126, 28), (384, 63, 14), (768, 31, 7)]):
@@ -43,13 +40,4 @@ for stage, (C, H, W) in enumerate([(96, 252, 56), (192, 126, 28), (384, 63, 14),
         print(f"   group-planar: dwconv_tc_gp {gp:7.1f} us   gp_transpose {tr:7.1f} us")
     old = t(lambda i: N.call("acx_dwconv_ln", xs[i % 3].data_ptr(), w.data_ptr(), b.data_ptr(), lw.data_ptr(), lb.data_ptr(),
                              y.data_ptr(), B, H, W, C, N.ACX_BF16, st()))
-    if TRACE is not None:
-        N.call("acx_dwconv_tc_gp" if stage < 2 else "acx_dwconv_tc", xs[0].data_ptr(), w.data_ptr(), b.data_ptr(), v.data_ptr(), B, H, W, C, st())
-        torch.cuda.synchronize()
-        if stage < 2:
-            tr = TRACE.cpu().view(2, 16)
-            for k in range(2):
-                u = max(1, int(tr[k, 0]))
-                print(f"   v3 CTA {k}: {u} items; cycles per item: MMA thread waits A {int(tr[k,1])//u}, waits D {int(tr[k,2])//u}, issues {int(tr[k,3])//u} | "
-                      f"loader waits {int(tr[k,4])//u}, loads {int(tr[k,5])//u} | write-out waits {int(tr[k,6])//u}, works {int(tr[k,7])//u}")
     print(f"stage {stage} C={C}: dwconv_tc {tc:7.1f} us   layernorm_rows {ln:7.1f} us   (sum {tc + ln:7.1f})   dwconv_ln (CUDA cores) {old:7.1f} us")
