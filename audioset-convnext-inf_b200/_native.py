@@ -85,6 +85,10 @@ SIGNATURES = {
     "acx_cosine_scores": [_vp, _vp, _ll, _vp, _vp, _ll, _i, _vp, _vp],
     "acx_search_topk_workspace": [_ll, _ll, _vp],
     "acx_search_topk": [_vp, _ll, _ll, _vp, _i, _vp, _vp, _vp, _vp],
+    # tagging metrics: per-class (P, U2, S_lo, S_hi) counts of classes [c0, c0 + kc) of (N, K) scores and uint8 targets,
+    # caller-owned workspace sized by the host query
+    "acx_tagging_metrics_workspace": [_ll, _i, _vp],
+    "acx_tagging_metrics": [_vp, _ll, _i, _i, _i, _vp, _vp, _vp, _vp],
 }
 
 

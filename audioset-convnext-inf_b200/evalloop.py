@@ -1,14 +1,16 @@
 """Drop-in for the reference's batch inference loop `pytorch_utils.forward` (reference
-src/audioset_convnext_inf/pytorch/pytorch_utils.py:63-137, called by `Evaluator.evaluate`, evaluate.py:34-39).
+src/audioset_convnext_inf/pytorch/pytorch_utils.py:63-137) and for its caller `Evaluator` (evaluate.py:12-60).
 
 Same name, arguments, and return value (dict of concatenated numpy arrays), but the per-batch
 `move_data_to_device` -> `model(batch)` -> `.data.cpu().numpy()` sequence runs through `HostPipeline`, so the H2D
 copy of batch i+1 and the D2H copy of batch i-1 overlap the kernels of batch i.  Waveforms may be float32 or the
-int16 PCM the AudioSet HDF5 files hold (data_generator.py:70-74).
+int16 PCM the AudioSet HDF5 files hold (data_generator.py:70-74).  `Evaluator.evaluate` scores the clipwise output
+against the targets on the GPU (metrics.tagging_metrics) instead of with sklearn on the host.
 """
 import numpy as np
 import torch
 
+from . import metrics
 from .pipeline import HostPipeline
 
 
@@ -51,3 +53,22 @@ def forward(model, generator, use_torchaudio=False, return_input=False, return_t
     if return_target and targets:
         out["target"] = np.concatenate(targets, axis=0)
     return out
+
+
+class Evaluator:
+    """The reference's Evaluator (evaluate.py:12-60): Evaluator(model).evaluate(data_loader)."""
+
+    def __init__(self, model):
+        self.model = model
+
+    def evaluate(self, data_loader):
+        """forward(model, data_loader, return_target=True), then per-class metrics of the clipwise output against the
+        targets on the model's device.  Returns {"average_precision", "auc", "d_prime"}, each a (classes,) float64
+        numpy array.  Raises ValueError when the loader yields no "target"."""
+        out = forward(self.model, data_loader, return_target=True)
+        if "target" not in out:
+            raise ValueError("the data loader yields no \"target\": there is nothing to score the clipwise output against")
+        dev = next(self.model.parameters()).device
+        stats = metrics.tagging_metrics(torch.from_numpy(out["clipwise_output"]).to(dev), out["target"])
+        return {"average_precision": stats["average_precision"], "auc": stats["auc"],
+                "d_prime": metrics.d_prime(stats["auc"])}

@@ -382,6 +382,21 @@ ACX_API int acx_search_topk_workspace(long long Q, long long N, long long* bytes
 ACX_API int acx_search_topk(const float* scores, long long Q, long long N, const long long* ranges, int k,
                             float* out_score, long long* out_index, void* workspace, void* stream);
 
+/* ---- tagging metrics: exact integer counts behind per-class average precision and ROC AUC --------------------------
+ * acx_tagging_metrics: for every class c in [c0, c0 + kc) of the row-major (N, K) fp32 scores (finite) and (N, K) uint8
+ * targets (0 / non-zero), out[c - c0] = (P, U2, S mod 2^64, S >> 64) as four uint64, where, with the rows ordered by
+ * descending key (the score's bits mapped to an unsigned order, -0.0 taken as +0.0) and tie groups g of equal keys
+ * holding p_g positives and n_g negatives, TP_g = positives in groups >= g, C_g = rows in groups >= g, PA_g = TP_g - p_g:
+ *   P = sum_g p_g,  U2 = sum_g n_g (2 PA_g + p_g),  S = sum over g with p_g > 0 of floor(p_g TP_g 2^64 / C_g).
+ * Then AUC = U2 / (2 P (N - P)) and AP = S / (P 2^64) (metrics.py).  Everything is an integer, so the counts do not
+ * depend on row order or launch shape.  workspace is DEVICE scratch of acx_tagging_metrics_workspace(N, kc) bytes (a
+ * host query, no launch; 16 N + 4096 bytes per class).  A memset and two launches, no allocation and no
+ * synchronisation.  A null pointer, N outside [1, 2^31 - 1], K < 1 or a chunk outside [0, K) returns ACX_ERR_ARG
+ * before any launch. */
+ACX_API int acx_tagging_metrics_workspace(long long N, int kc, long long* bytes_host);
+ACX_API int acx_tagging_metrics(const float* scores, long long N, int K, int c0, int kc, const unsigned char* targets,
+                                void* workspace, unsigned long long* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
