@@ -214,7 +214,9 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ log
 //  * LayerNorm statistics are fp32; the R*7 per-pixel partial sums are reduce-scattered inside each 16-lane group
 //    (30 shuffles for 28 pixels) and combined across the C/32 groups through shared memory in a FIXED order, so a
 //    clip's result is bit-identical whatever else is in the batch.  The fp32 instantiation uses the two-pass
-//    variance of F.layer_norm; the bf16 one a single pass (sum and sum of squares together).
+//    variance of F.layer_norm; the bf16 one a single pass (sums and sums of squares together) over values shifted by
+//    the pixel's first channel, which does not cancel when a pixel's conv outputs share a large offset (unshifted, the
+//    rstd error reaches a bf16 half-ulp at mean / std ~ 100).
 // =============================================================================================
 constexpr int DW_R = 4;
 
@@ -262,6 +264,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
   float2* sw = reinterpret_cast<float2*>(dsm);                 // [49][TPS] taps as fp32 pairs
   float* part = dsm + 2 * 49 * TPS;                             // [S][G][NV]
   float* tot = part + S * G * NV;                               // [S][NV]
+  float* shf = tot + S * NV;                                    // [S][32] per-pixel shifts (single pass)
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int cp = tid % TPS;
@@ -409,14 +412,26 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
       }
     }
   } else {
-    // one pass: sums and sums of squares reduced together; ONE thread per pixel turns them into (rstd, -mean*rstd)
-    // so every other thread only does  out = acc * (rstd*g) + (-mean*rstd*g + b)  with three packed fp32x2 ops
+    // one pass over d = acc - x0 (x0 = the pixel's first channel, held by channel pair 0 and broadcast through shared
+    // memory): sums and sums of squares of d reduced together; ONE thread per pixel turns them into (rstd, mean) so every
+    // other thread only does  out = (acc - mean) * (rstd*g) + b  with three packed fp32x2 ops.  The previous group's
+    // shifts were last read before its second barrier, so channel pair 0 may overwrite them here.
+    float* my_shf = shf + s * 32;
+    if (cp == 0) {
+#pragma unroll
+      for (int q = 0; q < NP; ++q) my_shf[q] = acc[q / 7][q % 7].x;
+    }
+    __syncthreads();
     float v[NV];
 #pragma unroll
     for (int q = 0; q < 32; ++q) {
-      const float2 a2 = q < NP ? acc[q / 7][q % 7] : make_float2(0.f, 0.f);
-      const float2 sq = __fmul2_rn(a2, a2);
-      v[q] = a2.x + a2.y;
+      float2 d = make_float2(0.f, 0.f);
+      if (q < NP) {
+        const float x0 = my_shf[q];
+        d = __fadd2_rn(acc[q / 7][q % 7], make_float2(-x0, -x0));
+      }
+      const float2 sq = __fmul2_rn(d, d);
+      v[q] = d.x + d.y;
       v[32 + q] = sq.x + sq.y;
     }
     halfwarp_reduce_scatter<NV>(v, lane);
@@ -424,18 +439,17 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
 #pragma unroll
     for (int q = 0; q < PER_LANE; ++q) my_part[slot + q] = v[q];
     __syncthreads();
-    float2* my_stat = reinterpret_cast<float2*>(my_tot);       // [32] (rstd, -mean * rstd)
-    if (cp < 32) {
+    float2* my_stat = reinterpret_cast<float2*>(my_tot);       // [32] (rstd, mean)
+    if (cp < NP) {
       float su = part[(s * G) * NV + cp], sq = part[(s * G) * NV + 32 + cp];
 #pragma unroll
       for (int g = 1; g < G; ++g) {                             // fixed order
         su += part[(s * G + g) * NV + cp];
         sq += part[(s * G + g) * NV + 32 + cp];
       }
-      const float mean = su * (1.0f / C);
-      const float var = fmaxf(sq * (1.0f / C) - mean * mean, 0.f);
-      const float rs = rsqrtf(var + 1e-6f);
-      my_stat[cp] = make_float2(rs, -mean * rs);
+      const float md = su * (1.0f / C);                         // mean of the shifted values
+      const float var = fmaxf(sq * (1.0f / C) - md * md, 0.f);
+      my_stat[cp] = make_float2(rsqrtf(var + 1e-6f), md + my_shf[cp]);
     }
     __syncthreads();
 #pragma unroll
@@ -447,8 +461,7 @@ __global__ void __launch_bounds__(S* C / 2, dw_min_blocks(S* C / 2))
       for (int p = 0; p < 7; ++p) {
         const float2 st = my_stat[r * 7 + p];
         const float2 sc = __fmul2_rn(make_float2(st.x, st.x), gw);
-        const float2 of = __ffma2_rn(make_float2(st.y, st.y), gw, gb);
-        const float2 o = __ffma2_rn(acc[r][p], sc, of);
+        const float2 o = __ffma2_rn(__fadd2_rn(acc[r][p], make_float2(-st.y, -st.y)), sc, gb);
         orow[(size_t)p * TPS] = P::pack(o.x, o.y);
       }
     }
@@ -926,7 +939,7 @@ static int launch_dwconv(const void* x, const void* w, const float* bias, const 
   const int strips = W / 7;
   ACX_CHECK(strips % S == 0, ACX_ERR_ARG, "dwconv_ln: W/7=%d not a multiple of strips-per-block %d", strips, S);
   constexpr int NV = sizeof(T) == 4 ? 32 : 64;
-  constexpr int SMEM = (2 * 49 * (C / 2) + S * (C / 32) * NV + S * NV) * (int)sizeof(float);
+  constexpr int SMEM = (2 * 49 * (C / 2) + S * (C / 32) * NV + S * NV + S * 32) * (int)sizeof(float);
   auto kern = dwconv_ln_kernel<T, C, S, RAG>;
   ACX_SET_MAX_SMEM(kern, SMEM);
   const int row_groups = ceil_div(H, DW_R);

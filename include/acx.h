@@ -136,7 +136,7 @@ ACX_API int acx_gp_row_stats(const void* v, float* stats, long long M, int C, vo
 /* x (B,H,W,C) -> a (B*(H/2)*(W/2), 4C) with k = (dy*2+dx)*C + c  (the GEMM A operand). */
 ACX_API int acx_ln_patchify(const void* x, const float* ln_w, const float* ln_b, void* a, int B, int H, int W, int C,
                     int act_dtype, void* stream);
-/* same, x group-planar [C/8][B*H*W][8] bf16 (C = 96 / 192); `a` row-major as above */
+/* same, x group-planar [C/8][Mp][8] bf16 (Mp = B*H*W rounded up to 128; C = 96 / 192 / 384); `a` row-major as above */
 ACX_API int acx_ln_patchify_gp(const void* x, const float* ln_w, const float* ln_b, void* a, int B, int H, int W, int C,
                        void* stream);
 

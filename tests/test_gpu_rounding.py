@@ -8,7 +8,8 @@ arithmetic instead of by a loose multiple of the output magnitude:
      in fp32) and the output is the kernel's GELU rounded once to bf16 -- every bf16 value in [-12, 12] times four scales,
      the clamp region, +-0 and tiny magnitudes, on every GELU-bearing kernel.
 * B  LayerNorm readouts: rows +-u around a mean, whose statistics are exact in the kernels' shifted single-pass arithmetic,
-     with u^2 comparable to eps and with large common offsets.
+     with u^2 comparable to eps and with large common offsets; and full-mantissa rows with mean / sigma up to 400, on
+     which a variance without the shift cancels.
 * C  emulated-rounding bounds on random operands: fp64 emulation of the documented rounding points, per element and in
      aggregate (the fraction of outputs that differ from the round-to-nearest of the emulation).
 * D  stem at every frame count mod 4 (dense, planar and ragged forms), head at h3 = 1, power -> mel -> dB -> bn0, and the
@@ -197,31 +198,55 @@ def test_gelu_readout_gemm_and_fused_mlps(C):
 # ======================================================================================================================
 # B. LayerNorm readouts
 # ======================================================================================================================
-# (mean, u): rows mean +- u alternating by channel, every value bf16-exact.  u^2 comparable to eps = 1e-6 (a wrong eps
-# moves rstd by tens of percent), and large common offsets (a single-pass variance without the shift cancels).
+# (mean, u): rows mean +- u alternating by channel, every value bf16-exact, so every partial sum of the statistics is exact in
+# fp32 and rstd / mean are known in closed form.  u^2 comparable to eps = 1e-6 (a wrong eps moves rstd by tens of percent).
 LN_ROWS = [(0.0, 2.0 ** -10), (0.0, 2.0 ** -11), (0.0, 2.0 ** -9), (0.0, 2.0 ** -12), (0.0, 0.5), (64.0, 0.5),
            (128.0, 1.0), (-96.0, 0.5), (8.0, 2.0 ** -4), (1.0, 2.0 ** -7), (-2.0, 2.0 ** -6), (16.0, 2.0 ** -3)]
+# (mean, sigma): bf16 rows mean + sigma N(0, 1), mean / sigma from 64 to 400, whose sums round in fp32.  There a single-pass
+# variance without the shift (E[v^2] - mean^2) loses 1e-3 .. 1e-2 of rstd; shifted by the row's first channel, ~1e-6.
+LN_OFFSET_ROWS = [(16.0, 0.25), (64.0, 0.5), (128.0, 1.0), (100.0, 0.25)]
 
 
 def _ln_operands(C, M):
-    mu = torch.tensor([r[0] for r in LN_ROWS], dtype=F64)[torch.arange(M) % len(LN_ROWS)]
-    u = torch.tensor([r[1] for r in LN_ROWS], dtype=F64)[torch.arange(M) % len(LN_ROWS)]
+    """Rows LN_ROWS then LN_OFFSET_ROWS, cycling.  Returns v (bf16), mean, rstd, v - mean (fp64), and per row the fp32 slack
+    of the statistics beyond exact sums -- relative on rstd, absolute on the mean -- which is zero for the closed-form
+    rows.  On the offset rows any order of summing C terms errs by at most (C - 1) u sum |terms|: a variance shifted by
+    the first channel v0 by C u E[(v - v0)^2] / (var + eps) relative, the mean by C u E|v - v0|."""
+    nr = len(LN_ROWS) + len(LN_OFFSET_ROWS)
+    fam = torch.arange(M) % nr
+    rows = LN_ROWS + LN_OFFSET_ROWS
+    mu = torch.tensor([r[0] for r in rows], dtype=F64)[fam]
+    u = torch.tensor([r[1] for r in rows], dtype=F64)[fam]
     sign = 1.0 - 2.0 * (torch.arange(C) % 2).to(F64)
-    v = mu[:, None] + u[:, None] * sign[None, :]
-    assert torch.equal(v.to(torch.bfloat16).double(), v)
-    rstd = 1.0 / torch.sqrt(u * u + 1e-6)
-    return v.to(torch.bfloat16).to(DEV), mu.to(DEV), rstd.to(DEV), (u[:, None] * sign[None, :]).to(DEV)
+    z = torch.randn(M, C, generator=torch.Generator().manual_seed(C + M), dtype=F64)
+    closed = fam < len(LN_ROWS)
+    v = torch.where(closed[:, None], mu[:, None] + u[:, None] * sign[None, :], mu[:, None] + u[:, None] * z)
+    v = v.to(torch.bfloat16).double()
+    assert torch.equal(v[closed], mu[closed, None] + u[closed, None] * sign[None, :])
+    mean = v.mean(1)
+    dev = v - mean[:, None]
+    var = (dev * dev).mean(1)
+    rstd = 1.0 / torch.sqrt(var + 1e-6)
+    assert torch.equal(mean[closed], mu[closed]) and torch.equal(var[closed], u[closed] ** 2)
+    sh = v - v[:, :1]
+    rel = torch.where(closed, 0.0, 0.5 * C * U24 * (sh * sh).mean(1) / (var + 1e-6))
+    mean_err = torch.where(closed, 0.0, C * U24 * sh.abs().mean(1))
+    return (v.to(torch.bfloat16).to(DEV), mean.to(DEV), rstd.to(DEV), dev.to(DEV),
+            (rel.to(DEV)[:, None], mean_err.to(DEV)[:, None]))
 
 
 def test_layernorm_statistics_readout():
     """acx_gp_row_stats and acx_layernorm_rows on rows with closed-form statistics: rstd = 1 / sqrt(u^2 + 1e-6) to fp32
-    accuracy, -mean rstd likewise, and LN(v) within one bf16 rounding of its fp64 value."""
+    accuracy, -mean rstd likewise, and LN(v) within one bf16 rounding of its fp64 value; on the full-mantissa offset rows
+    the same plus the rounding of the (shifted) sums."""
     for C in (96, 192, 384):
         M = 128 * 3 + 5
-        v, mu, rstd, dev = _ln_operands(C, M)
+        v, mu, rstd, dev, (rel, mean_err) = _ln_operands(C, M)
+        rel, mean_err = rel[:, 0], mean_err[:, 0]
         stats = _row_stats(v).double()
-        assert ((stats[:, 0] - rstd).abs() <= 4 * U24 * rstd).all(), ((stats[:, 0] / rstd - 1).abs().max().item())
-        assert ((stats[:, 1] + mu * rstd).abs() <= 4 * U24 * (mu * rstd).abs() + 1e-30).all()
+        assert ((stats[:, 0] - rstd).abs() <= (4 * U24 + rel) * rstd).all(), ((stats[:, 0] / rstd - 1).abs().max().item())
+        assert ((stats[:, 1] + mu * rstd).abs() <= (4 * U24 + rel) * (mu * rstd).abs() + mean_err * rstd + 1e-30).all(), \
+            ((stats[:, 1] + mu * rstd).abs() - (4 * U24 + rel) * (mu * rstd).abs() - mean_err * rstd).max().item()
         g = torch.Generator().manual_seed(C)
         lw = (torch.rand(C, generator=g) * 0.4 + 0.8).to(DEV)
         lb = (torch.randn(C, generator=g) * 0.1).to(DEV)
@@ -230,6 +255,7 @@ def test_layernorm_statistics_readout():
         ref = dev * rstd[:, None] * lw.double() + lb.double()
         # out = v (rstd w) + (b - mean rstd w) in fp32: the two terms cancel for rows with a large common offset
         slack = (((v.double().abs() + mu.abs()[:, None]) * rstd[:, None] * lw.double()).abs() + lb.double().abs()) * 8 * U24
+        slack = slack + (rel[:, None] * dev.abs() + mean_err[:, None]) * rstd[:, None] * lw.double().abs()
         yd = y.double()
         assert ((yd - ref).abs() <= 0.5 * _ulp(yd) + slack).all(), ((yd - ref).abs() / _ulp(yd)).max().item()
 
@@ -242,7 +268,7 @@ def test_layernorm_readout_through_the_gelu(C):
     statistics and of the fold's cancellation, one bf16 rounding of the normalised operand (in-smem form), the GELU's E,
     and the output rounding."""
     M = 128 * 150 + 77
-    v, mu, rstd, dev = _ln_operands(C, M)
+    v, mu, rstd, dev, (rel, mean_err) = _ln_operands(C, M)
     w1 = torch.zeros(4 * C, C)
     for j in range(4 * C):
         w1[j, j % C] = SCALES[j // C]
@@ -267,6 +293,9 @@ def test_layernorm_readout_through_the_gelu(C):
     # folded: pre = rstd G + (-mean rstd) s + b1 in fp32, G = v_k s_j exact; the two terms cancel
     big = (mu.abs() + dev.abs().amax(1))[:, None] * rstd[:, None] * sc.abs()
     d_fold = big * 8 * U24
+    # offset rows: the rounding of the statistics' sums, the same in every form
+    d_stats = ((rel * dev.abs() + mean_err) * rstd[:, None]).repeat(1, 4) * sc.abs()
+    d_smem, d_fold = d_smem + d_stats, d_fold + d_stats
     lw, lb = ones, zc
     cases = [("mlp_fused_ln", read("ln", ln_w=lw, ln_b=lb), d_smem),
              ("mlp_fused_gp ln_w/ln_b", read("gp", ln_w=lw, ln_b=lb), d_smem),
